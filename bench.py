@@ -144,6 +144,40 @@ def touched_cell_bytes(rois_b4n, counts, grids, strides, C, finest=56.0):
     return total
 
 
+DUMP_FEAT_ROWS = 512
+
+
+def dump_outputs(path, out):
+    """Write what one TrainHotPath.step returned to `path`/<name>.npy as float32 (the integer outputs are counts, labels
+    and indices, all exact in float32), so that two builds can be compared output for output.  Entries past an image's
+    count are zeroed: a caller never reads them and they may hold what an earlier step left.  roi_feats (205 MB at
+    batch 8) is stored as a fixed, seeded sample of DUMP_FEAT_ROWS rows (25.7 MB), their indices in roi_feats_rows."""
+    import torch
+
+    rpn, rcnn = out["rpn"], out["rcnn"]
+    pc, rn, bn = (t.cpu().numpy() for t in (out["prop_count"], rpn.n_chosen, rcnn.n_chosen))
+
+    def upto(t, n):
+        a = t.cpu().numpy()
+        keep = np.arange(a.shape[-1])[None, :] < n[:, None]                     # [B, last axis]
+        return np.where(keep.reshape((a.shape[0],) + (1,) * (a.ndim - 2) + (a.shape[-1],)), a, 0)
+
+    arrays = {"props": upto(out["props"], pc), "scores": upto(out["scores"], pc), "prop_count": pc,
+              "rpn_count": rn, "rpn_label": upto(rpn.tar_label, rn), "rpn_param": upto(rpn.tar_param, rn),
+              "rpn_tar_cls": upto(out["rpn_tar_cls"], rn), "rpn_tar_reg": upto(out["rpn_tar_reg"], rn),
+              "roi_count": bn, "roi_box": upto(rcnn.tar_box, bn), "roi_label": upto(rcnn.tar_label, bn),
+              "roi_param": upto(rcnn.tar_param, bn)}
+    feats = out["roi_feats"]
+    ld = feats.shape[0] // len(bn)
+    rows = np.sort(np.random.default_rng(0).choice(feats.shape[0], min(DUMP_FEAT_ROWS, feats.shape[0]), replace=False))
+    sample = feats.index_select(0, torch.from_numpy(rows).to(feats.device)).cpu().numpy()
+    sample[rows % ld >= bn[rows // ld]] = 0
+    arrays["roi_feats"], arrays["roi_feats_rows"] = sample, rows
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def workload_config(world):
     """`config` of the JSON line: the workload only (identical for both arms; what the B200 arm does with it is `run_config`)."""
     return {"workload": WORKLOAD, "global_batch": IMGS_PER_GPU * world, "parallelism": "per-image partition, dp%d" % world,
@@ -353,6 +387,8 @@ def run_b200(args):
     barrier()
     sampler.window = (t_host0, time.perf_counter())
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)                            # out: the buffers every step writes
     # The timed region is a few milliseconds; where an NVML query takes longer than that (box-dependent) no sample can
     # fall inside it.  The identical load is therefore kept up, UNTIMED, for ~240 more steps while the sampler keeps
     # spinning; those samples are reported separately (clocks.samples_under_load) and only used when the region has none.
@@ -753,6 +789,8 @@ if __name__ == "__main__":
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-dropin", action="store_true", help="skip the reference-call-sequence measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy, float32")
     a = ap.parse_args()
     if a.impl == "reference":
         run_reference(a)
