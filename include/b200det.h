@@ -310,6 +310,14 @@ B2D_API int b2d_rcnn_detect(float* out_box, float* out_score, int64_t* out_label
                     int reg_classes, const float* means_host, const float* stds_host, const float* img_hw,
                     float min_score, float nms_thr_f, int max_per_img, int strict, int cap, int B, int* overflow,
                     void* workspace, size_t ws_bytes, void* stream);
+/* b2d_rcnn_detect plus the packed detection records of dist.pack_detections: records fp32
+ * [B][max_per_img][6] = (x1, y1, x2, y2, score, float(label)), rows past out_count[b] zero --
+ * the payload of dist.gather_detections, written by the gather kernel itself. */
+B2D_API int b2d_rcnn_detect_records(float* out_box, float* out_score, int64_t* out_label, int* out_count, float* records,
+                            const float* props, long long ld, const int* counts, long long n, const float* cls_out,
+                            const float* reg_out, int C, int reg_classes, const float* means_host, const float* stds_host,
+                            const float* img_hw, float min_score, float nms_thr_f, int max_per_img, int strict, int cap,
+                            int B, int* overflow, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- K5/K6: FPN level-mapped RoIAlign (BasicRoIExtractor, lib/region.py:243-306 +
  * torchvision RoIAlign aligned=False).  rois [4, R] column-major, roi_img int32[R]
@@ -374,6 +382,16 @@ B2D_API int b2d_refine_bboxes(float* out, int* out_count, const float* props, lo
                       long long n, const int64_t* label, const float* reg_out, int C, const int64_t* is_gt,
                       const float* means_host, const float* stds_host, int clamp, const float* img_hw, int B,
                       void* stream);
+/* Test-time form (CascadeRCNN.forward_test, lib/detectors/cascade_rcnn.py:186-190): the label of
+ * row i is argmax(cls_out[b][i][0..num_classes)) -- the first maximal index, background
+ * included, as torch.argmax -- computed in the kernel; no GT columns, nothing dropped
+ * (out_count = counts).  cls_out [B][ld][num_classes] raw logits; reg_out [B][ld][4*reg_classes]
+ * (reg_classes = num_classes, or 1 when class-agnostic); always clamped to img_hw[b].
+ * Rows at or past counts[b] are neither read nor written. */
+B2D_API int b2d_refine_bboxes_argmax(float* out, int* out_count, const float* props, long long ld, const int* counts,
+                             long long n, const float* cls_out, int num_classes, const float* reg_out,
+                             int reg_classes, const float* means_host, const float* stds_host, const float* img_hw,
+                             int B, void* stream);
 
 /* ---- a18 / K9: ATSS target assignment (FCOSHead.single_image_targets_atss,
  * lib/heads/fcos_head.py:283-368 with topk_by_center :106-116 read as integer division).

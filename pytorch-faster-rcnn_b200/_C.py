@@ -76,6 +76,8 @@ _SIGS = {
     "b2d_fcos_targets": [_P, _P, _P, _P, _P, c_int, _P, _P, _P, _P, c_int, _P],
     "b2d_rcnn_detect": [_P, _P, _P, _P, _P, c_ll, _P, c_ll, _P, _P, c_int, c_int, _P, _P, _P, c_float, c_float, c_int,
                         c_int, c_int, c_int, _P, _P, c_size_t, _P],
+    "b2d_rcnn_detect_records": [_P, _P, _P, _P, _P, _P, c_ll, _P, c_ll, _P, _P, c_int, c_int, _P, _P, _P, c_float, c_float,
+                                c_int, c_int, c_int, c_int, _P, _P, c_size_t, _P],
     "b2d_gather_head_outputs": [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, _P],
     "b2d_roi_align_fwd_batched": [_P, _P, _P, c_ll, _P, c_int, _P, _P],
     "b2d_label_census": [_P, _P, c_int, _P, c_ll, _P, c_ll, c_int, _P],
@@ -94,6 +96,7 @@ _SIGS = {
     "b2d_roi_levels": [_P, _P, c_ll, c_ll, c_float, c_int, _P],
     "b2d_nchw_to_nhwc": [_P, _P, c_int, c_int, c_int, c_int, _P],
     "b2d_refine_bboxes": [_P, _P, _P, c_ll, _P, c_ll, _P, _P, c_int, _P, _P, _P, c_int, _P, c_int, _P],
+    "b2d_refine_bboxes_argmax": [_P, _P, _P, c_ll, _P, c_ll, _P, c_int, _P, c_int, _P, _P, _P, c_int, _P],
     "b2d_atss_assign": [_P, _P, _P, _P, _P, c_int, _P, _P, _P, c_int, c_int, _P, c_size_t, _P],
     "b2d_fcos_decode": [_P, _P, _P, _P, _P, _P, _P, _P, c_int, c_float, c_float, c_float, _P, c_int, _P],
     "b2d_roi_pool_fwd": [_P, _P, _P, c_int, c_int, c_int, c_int, _P, c_ll, _P, c_ll, c_float, c_int, c_int, _P],

@@ -14,13 +14,18 @@
 
 namespace b2d {
 
-// ------------------------------------------------------------------ a17
+// ------------------------------------------------------------------ a17 (+ its test-time form, arg-max labels)
 struct RefineArgs {
     const float* props; long long ld; const int* counts; long long n;
     const int64_t* label; const float* reg; int C; const int64_t* is_gt;
+    const float* cls; int NC;                   // kArgmax: raw logits [B][ld][NC], label = first maximal index
     float ms[8]; int clamp; const float* img_hw;
 };
 
+// kArgmax == false: labels from p.label (the training stages' sampled labels), GT columns dropped.
+// kArgmax == true: CascadeRCNN.forward_test's `argmax(cls_out)` (lib/detectors/cascade_rcnn.py:186-190) computed
+// in place -- the first maximal index like torch.argmax, background included; nothing is dropped.
+template <bool kArgmax>
 __global__ void __launch_bounds__(256) k_refine(RefineArgs p, float* __restrict__ out, int* __restrict__ out_count) {
     __shared__ int s_warp[8], s_base;
     const int b = blockIdx.x;
@@ -35,11 +40,23 @@ __global__ void __launch_bounds__(256) k_refine(RefineArgs p, float* __restrict_
     __syncthreads();
     for (int i0 = 0; i0 < n; i0 += blockDim.x) {
         const int i = i0 + threadIdx.x;
-        const bool keep = i < n && !(gtf && gtf[i] != 0);
+        const bool keep = i < n && !(!kArgmax && gtf && gtf[i] != 0);
         Box r{0, 0, 0, 0};
         if (keep) {
             const Box base{pr[i], pr[p.ld + i], pr[2 * p.ld + i], pr[3 * p.ld + i]};
-            const int c = (p.C > 1 && lab) ? (int)lab[i] : 0;               // reg_out.view(-1, 4, C)[i, :, label]
+            int c = 0;                                                      // reg_out.view(-1, 4, C)[i, :, label]
+            if (kArgmax) {
+                if (p.C > 1) {
+                    const float* x = p.cls + ((long long)b * p.ld + i) * p.NC;
+                    float best = x[0];
+                    for (int k = 1; k < p.NC; ++k) {
+                        const float v = x[k];
+                        if (v > best) { best = v; c = k; }
+                    }
+                }
+            } else if (p.C > 1 && lab) {
+                c = (int)lab[i];
+            }
             const float* q = reg + (long long)i * 4 * p.C + c;
             r = decode_box(base, q[0], q[p.C], q[2 * p.C], q[3 * p.C], p.ms, p.clamp != 0, img_h, img_w);
         }
@@ -323,11 +340,29 @@ int b2d_refine_bboxes(float* out, int* out_count, const float* props, long long 
     B2D_REQUIRE(C >= 1 && (C == 1 || label), "refine_bboxes: per-class deltas need labels");
     B2D_REQUIRE(!clamp || img_hw, "refine_bboxes: clamp needs img_hw");
     RefineArgs a;
+    memset(&a, 0, sizeof(a));
     a.props = props; a.ld = ld; a.counts = counts; a.n = n; a.label = label; a.reg = reg_out; a.C = C; a.is_gt = is_gt;
     for (int i = 0; i < 4; ++i) { a.ms[i] = means_host ? means_host[i] : 0.0f; a.ms[4 + i] = stds_host ? stds_host[i] : 1.0f; }
     a.clamp = clamp; a.img_hw = img_hw;
-    k_refine<<<B, 256, 0, (cudaStream_t)stream>>>(a, out, out_count);
+    k_refine<false><<<B, 256, 0, (cudaStream_t)stream>>>(a, out, out_count);
     return check_launch("refine_bboxes");
+}
+
+int b2d_refine_bboxes_argmax(float* out, int* out_count, const float* props, long long ld, const int* counts, long long n,
+                             const float* cls_out, int num_classes, const float* reg_out, int reg_classes,
+                             const float* means_host, const float* stds_host, const float* img_hw, int B, void* stream) {
+    B2D_REQUIRE(out && out_count && props && cls_out && reg_out && img_hw && B >= 1 && ld >= 1 && n >= 0 && n <= ld,
+                "refine_bboxes_argmax: bad args");
+    B2D_REQUIRE(num_classes >= 1 && (reg_classes == num_classes || reg_classes == 1),
+                "refine_bboxes_argmax: need reg_classes in {1, num_classes}");
+    RefineArgs a;
+    memset(&a, 0, sizeof(a));
+    a.props = props; a.ld = ld; a.counts = counts; a.n = n; a.reg = reg_out; a.C = reg_classes;
+    a.cls = cls_out; a.NC = num_classes;
+    for (int i = 0; i < 4; ++i) { a.ms[i] = means_host ? means_host[i] : 0.0f; a.ms[4 + i] = stds_host ? stds_host[i] : 1.0f; }
+    a.clamp = 1; a.img_hw = img_hw;
+    k_refine<true><<<B, 256, 0, (cudaStream_t)stream>>>(a, out, out_count);
+    return check_launch("refine_bboxes_argmax");
 }
 
 size_t b2d_atss_workspace_bytes(const b2d_pyramid* pyr_host, int B) {

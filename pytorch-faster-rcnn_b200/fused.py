@@ -632,3 +632,101 @@ class CascadeHotPath(object):
                     _C.ptr(self.roi_img), None, self.B * self.m, self.B, ctypes.byref(self.bwd_cfg), _C.ptr(self.bwd_ws),
                     self.bwd_ws.numel(), _C.stream())
         return self.grads
+
+
+class InferHotPath(object):
+    """CascadeRCNN.forward_test (SURVEY 3.2, lib/detectors/cascade_rcnn.py:157-200) minus the backbone, neck and head
+    layers, batched: RPN proposals at the test configuration (K3 + K4) -> per stage FPN RoIAlign of the current boxes (K5)
+    -> [the caller's stage head] -> between stages BBoxHead.refine_bboxes with the arg-max labels
+    (b2d_refine_bboxes_argmax) -> after the last stage BBoxHead.predict_bboxes_single_image on that stage's input boxes
+    (b2d_rcnn_detect: softmax, per-class decode + clamp, class-offset NMS, top max_per_img).  num_stages = 1 is
+    faster_rcnn_r50_fpn, 3 the cascade.  Everything is allocated here; step() reads nothing back to the host, so a step
+    (head modules included) can be captured in one CUDA graph after a first eager call."""
+
+    def __init__(self, B, grids, device, strides=(4, 8, 16, 32, 64), feat_channels=256, num_classes=21, num_stages=1,
+                 rpn_test=None, rcnn_test=None,
+                 stage_stds=((0.1, 0.1, 0.2, 0.2), (0.05, 0.05, 0.1, 0.1), (0.033, 0.033, 0.067, 0.067)),
+                 reg_class_agnostic=False, layout=1):
+        rpn_test = rpn_test or dict(pre_nms=1000, post_nms=1000, max_num=1000, nms_iou=0.7, min_bbox_size=0)
+        rcnn_test = rcnn_test or dict(min_score=0.05, nms_iou=0.5, max_per_img=100, nms_type='official')
+        if not 1 <= num_stages <= len(stage_stds):
+            raise ValueError("num_stages must be in 1..%d (one stds tuple per stage)" % len(stage_stds))
+        z4 = (0.0, 0.0, 0.0, 0.0)
+        self.B, self.device, self.S = B, device, int(num_stages)
+        self.NC, self.reg_c = int(num_classes), 1 if reg_class_agnostic else int(num_classes)
+        self.pyr = AnchorPyramid(strides, grids)
+        self.proposals = RpnProposals(self.pyr, B, rpn_test, z4, (1.0, 1.0, 1.0, 1.0), device)
+        self.P = P = self.proposals.P
+        shapes = [(feat_channels, g[0], g[1]) for g in grids[:4]]
+        self.roi_align = [BatchedRoIAlign(B, P, shapes, list(strides[:4]), device, layout=layout) for _ in range(self.S)]
+        self.stds = [_C.host_f4(sd, [1, 1, 1, 1]) for sd in stage_stds[:self.S]]
+        self.zero4 = _C.host_f4(z4, [0, 0, 0, 0])
+        self.boxes = [torch.zeros((B, 4, P), dtype=torch.float32, device=device) for _ in range(self.S - 1)]
+        self.counts = [torch.zeros(B, dtype=torch.int32, device=device) for _ in range(self.S - 1)]
+        get = (lambda k, d=None: rcnn_test.get(k, d)) if hasattr(rcnn_test, "get") else (lambda k, d=None: getattr(rcnn_test, k, d))
+        mode = get('nms_type', 'official')
+        self.min_score, self.nms_thr = float(np.float32(get('min_score'))), _C.floor_f32(float(get('nms_iou')))
+        self.strict = int(mode == 'strict')
+        self.cap = max(1, min(16384, P * ((self.NC - 1) if not self.strict else 1)))
+        mpi = get('max_per_img')
+        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap))
+        self.det_box = torch.zeros((B, 4, M), dtype=torch.float32, device=device)
+        self.det_score = torch.zeros((B, M), dtype=torch.float32, device=device)
+        self.det_label = torch.zeros((B, M), dtype=torch.int64, device=device)
+        self.det_count = torch.zeros(B, dtype=torch.int32, device=device)
+        self.overflow = torch.zeros(1, dtype=torch.int32, device=device)
+        self.det_ws = torch.empty(_C.lib().b2d_rcnn_detect_workspace_bytes(self.cap, B), dtype=torch.uint8, device=device)
+
+    def step(self, cls_outs, reg_outs, feats, img_hw, heads, records=None, mark=None):
+        """cls_outs / reg_outs: the RPN head maps per level ([B,A,H,W], [B,4A,H,W]); feats: the first four FPN maps
+        (channels_last for layout 1); img_hw fp32 [B,2]; heads[s](roi_feats [B*P,C,7,7]) -> (cls_out [B*P, num_classes]
+        logits, reg_out [B*P, 4*num_classes] or [B*P, 4]); records: optional fp32 [B, max_per_img, 6] that receives the
+        packed detections of dist.pack_detections (the payload of dist.gather_detections); mark(name): optional
+        callable run after each phase (e.g. to record a CUDA event).  Returns the detections (boxes [B,4,M], scores
+        [B,M], labels int64 [B,M], count int32 [B]) and per stage the input boxes, counts and RoI features."""
+        if records is not None and (tuple(records.shape) != (self.B, self.M, 6) or records.dtype != torch.float32
+                                    or not records.is_contiguous()):
+            raise _C.B200DetError("InferHotPath.step: records must be contiguous fp32 [%d, %d, 6]" % (self.B, self.M))
+        props, _, count = self.proposals(cls_outs, reg_outs, img_hw)
+        if mark is not None:
+            mark("proposals")
+        boxes, stages = props, []
+        for s in range(self.S):
+            roi_feats = self.roi_align[s](feats, boxes, count)
+            if mark is not None:
+                mark("roi_align%d" % s)
+            cls_out, reg_out = heads[s](roi_feats)
+            cls_out, reg_out = _C.f32c(cls_out), _C.f32c(reg_out)
+            if tuple(cls_out.shape) != (self.B * self.P, self.NC) or tuple(reg_out.shape) != (self.B * self.P, 4 * self.reg_c):
+                raise _C.B200DetError("InferHotPath.step: stage %d head returned %s / %s, expected [%d, %d] / [%d, %d]"
+                                      % (s, tuple(cls_out.shape), tuple(reg_out.shape), self.B * self.P, self.NC,
+                                         self.B * self.P, 4 * self.reg_c))
+            if mark is not None:
+                mark("head%d" % s)
+            stages.append(dict(boxes=boxes, count=count, roi_feats=roi_feats, cls_out=cls_out, reg_out=reg_out))
+            if s + 1 < self.S:
+                _C.call("b2d_refine_bboxes_argmax", _C.ptr(self.boxes[s]), _C.ptr(self.counts[s]), _C.ptr(boxes), self.P,
+                        _C.ptr(count), self.P, _C.ptr(cls_out), self.NC, _C.ptr(reg_out), self.reg_c, self.zero4,
+                        self.stds[s], _C.ptr(img_hw), self.B, _C.stream())
+                boxes, count = self.boxes[s], self.counts[s]
+                if mark is not None:
+                    mark("refine%d" % s)
+        last = stages[-1]
+        args = [_C.ptr(self.det_box), _C.ptr(self.det_score), _C.ptr(self.det_label), _C.ptr(self.det_count)]
+        if records is not None:
+            args.append(_C.ptr(records))
+        args += [_C.ptr(boxes), self.P, _C.ptr(count), self.P, _C.ptr(last["cls_out"]), _C.ptr(last["reg_out"]), self.NC,
+                 self.reg_c, self.zero4, self.stds[-1], _C.ptr(img_hw), self.min_score, self.nms_thr, self.M, self.strict,
+                 self.cap, self.B, _C.ptr(self.overflow), _C.ptr(self.det_ws), self.det_ws.numel(), _C.stream()]
+        _C.call("b2d_rcnn_detect_records" if records is not None else "b2d_rcnn_detect", *args)
+        if mark is not None:
+            mark("detect")
+        return dict(boxes=self.det_box, scores=self.det_score, labels=self.det_label, count=self.det_count,
+                    records=records, stages=stages)
+
+    def check(self):
+        """Synchronise and raise if the last step had an image with more than 16384 (box, class) candidates (its
+        candidates past the cap were dropped in enumeration order)."""
+        torch.cuda.synchronize(self.device)
+        if int(self.overflow[0]):
+            raise _C.B200DetError("rcnn_detect: more than 16384 (box, class) candidates; raise min_score")
