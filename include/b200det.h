@@ -319,6 +319,38 @@ B2D_API int b2d_rcnn_detect_records(float* out_box, float* out_score, int64_t* o
                             const float* img_hw, float min_score, float nms_thr_f, int max_per_img, int strict, int cap,
                             int B, int* overflow, void* workspace, size_t ws_bytes, void* stream);
 
+/* ---- dense-head test-time detections: utils.multiclass_nms (lib/utils.py:224-269) for B images at once, as
+ * AnchorHead.predict_single_image (lib/heads/anchor_head.py:207-258, RetinaNet) and FCOSHead.predict_single_image
+ * (lib/heads/fcos_head.py:570-631) call it after their selection.  Rows: boxes [B][4][ld] already decoded
+ * (class-agnostic), counts int32[B], rows int32[B][ld] = the flat anchor / point index of each row.  The C class values
+ * of a row with flat index f in level l (lv.offset[l] <= f < lv.offset[l + 1]) are
+ * lv.base[l][b * lv.img_stride[l] + c * lv.class_stride[l] + (f - lv.offset[l])] -- e.g. RetinaNet's logit maps
+ * cls_l.view(B, C, -1) in place, or FCOS's score [B][C][total] as one level.  transform: 0 the values are scores, 1
+ * sigmoid, 2 softmax over the C values.  min_score is tested on that score; the candidate's score is score *
+ * score_factor[b][f] (score_factor [B][factor_ld] or NULL).  chan_mask_host: 2 x u64 bitmap of nms_channel; strict:
+ * only the first maximal channel of a row, if it is an NMS channel.  Candidates are ordered row-major, channel minor;
+ * the NMS offset is channel * max(candidate boxes); label_add is added to the written labels only (1 for a sigmoid head's
+ * 1-based labels).  Outputs and records as b2d_rcnn_detect(_records); workspace b2d_rcnn_detect_workspace_bytes(cap, B);
+ * cap <= 16384 candidates per image, *overflow = 1 if an image had more.  events_host: NULL, or two cudaEvent_t (either
+ * may be NULL) recorded after the candidate stage and after the NMS. */
+typedef struct b2d_dense_levels {
+    int num_levels, _pad;
+    long long offset[B2D_MAX_LEVELS];       /* first flat index of the level (offset[0] == 0, ascending) */
+    const float* base[B2D_MAX_LEVELS];      /* DEVICE pointer of the level's class values (image 0, class 0, index 0) */
+    long long img_stride[B2D_MAX_LEVELS], class_stride[B2D_MAX_LEVELS];
+} b2d_dense_levels;
+B2D_API int b2d_dense_detect(float* out_box, float* out_score, int64_t* out_label, int* out_count, const float* boxes,
+                     long long ld, const int* counts, const int* rows, const b2d_dense_levels* lv_host, int C, int transform,
+                     const float* score_factor, long long factor_ld, const unsigned long long* chan_mask_host,
+                     float min_score, int label_add, float nms_thr_f, int max_per_img, int strict, int cap, int B,
+                     int* overflow, void* workspace, size_t ws_bytes, void* const* events_host, void* stream);
+B2D_API int b2d_dense_detect_records(float* out_box, float* out_score, int64_t* out_label, int* out_count, float* records,
+                             const float* boxes, long long ld, const int* counts, const int* rows,
+                             const b2d_dense_levels* lv_host, int C, int transform, const float* score_factor,
+                             long long factor_ld, const unsigned long long* chan_mask_host, float min_score, int label_add,
+                             float nms_thr_f, int max_per_img, int strict, int cap, int B, int* overflow, void* workspace,
+                             size_t ws_bytes, void* const* events_host, void* stream);
+
 /* ---- K5/K6: FPN level-mapped RoIAlign (BasicRoIExtractor, lib/region.py:243-306 +
  * torchvision RoIAlign aligned=False).  rois [4, R] column-major, roi_img int32[R]
  * (NULL => image 0).  feat_ptrs_host[l] -> level l features, fp32 NCHW [B,C,H,W]
@@ -413,6 +445,17 @@ B2D_API int b2d_fcos_decode(float* boxes, float* key, float* score, float* ctr_s
                     const void* const* reg_ptrs_host, const void* const* ctr_ptrs_host, const b2d_pyramid* pyr_host,
                     int cls_channels, float reg_mean, float reg_std, float min_size, const float* img_hw, int B,
                     void* stream);
+/* FCOS per-level selection (lib/heads/fcos_head.py:602-613), batched and without host reads: on key [B][total] of
+ * b2d_fcos_decode (-inf = failed the size test), levels of level_sizes_host[l] points in order.  Per (image, level): more
+ * than pre_nms valid points -> the top pre_nms by key, descending, ties to the lowest index (b2d_topk); otherwise all
+ * valid points in ascending index order; levels concatenated.  idx int32 [B][P], P = sum_l min(pre_nms, n_l)
+ * (pre_nms <= 0: n_l), receives flat point indices (-1 past count[b]); count int32[B].  sel_boxes (optional, with
+ * boxes [B][4][total]): [B][4][P] the boxes of the selected points (zero past count[b]).  The workspace query returns
+ * 0 for an unsupported configuration (a level top-k over 16384). */
+B2D_API size_t b2d_dense_select_workspace_bytes(const int* level_sizes_host, int num_levels, int B, int pre_nms);
+B2D_API int b2d_dense_select(int* idx, int* count, float* sel_boxes, const float* key, const float* boxes,
+                     const int* level_sizes_host, int num_levels, int B, int pre_nms, void* workspace, size_t ws_bytes,
+                     void* stream);
 
 #ifdef __cplusplus
 }

@@ -50,6 +50,13 @@ class RoiCfg(ctypes.Structure):
                 ("W", c_int * MAX_LEVELS), ("spatial_scale", c_float * MAX_LEVELS)]
 
 
+class DenseLevels(ctypes.Structure):
+    """b2d_dense_levels: where the class values of a dense head's rows live (per level: first flat index, base pointer,
+    image stride, class stride)."""
+    _fields_ = [("num_levels", c_int), ("_pad", c_int), ("offset", c_ll * MAX_LEVELS), ("base", c_void_p * MAX_LEVELS),
+                ("img_stride", c_ll * MAX_LEVELS), ("class_stride", c_ll * MAX_LEVELS)]
+
+
 class B200DetError(RuntimeError):
     pass
 
@@ -78,6 +85,11 @@ _SIGS = {
                         c_int, c_int, c_int, _P, _P, c_size_t, _P],
     "b2d_rcnn_detect_records": [_P, _P, _P, _P, _P, _P, c_ll, _P, c_ll, _P, _P, c_int, c_int, _P, _P, _P, c_float, c_float,
                                 c_int, c_int, c_int, c_int, _P, _P, c_size_t, _P],
+    "b2d_dense_detect": [_P, _P, _P, _P, _P, c_ll, _P, _P, _P, c_int, c_int, _P, c_ll, _P, c_float, c_int, c_float, c_int,
+                         c_int, c_int, c_int, _P, _P, c_size_t, _P, _P],
+    "b2d_dense_detect_records": [_P, _P, _P, _P, _P, _P, c_ll, _P, _P, _P, c_int, c_int, _P, c_ll, _P, c_float, c_int, c_float,
+                                 c_int, c_int, c_int, c_int, _P, _P, c_size_t, _P, _P],
+    "b2d_dense_select": [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, _P, c_size_t, _P],
     "b2d_gather_head_outputs": [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, _P],
     "b2d_roi_align_fwd_batched": [_P, _P, _P, c_ll, _P, c_int, _P, _P],
     "b2d_label_census": [_P, _P, c_int, _P, c_ll, _P, c_ll, c_int, _P],
@@ -124,6 +136,7 @@ _SIZE_FNS = {
     "b2d_roi_align_bwd_workspace_bytes": [c_ll, c_int, _P],
     "b2d_atss_workspace_bytes": [_P, c_int],
     "b2d_rcnn_detect_workspace_bytes": [c_int, c_int],
+    "b2d_dense_select_workspace_bytes": [_P, c_int, c_int, c_int],
     "b2d_anchor_loss_workspace_bytes": [_P, c_int],
     "b2d_multiclass_nms_workspace_bytes": [c_int],
     "b2d_sampled_ce_workspace_bytes": [],

@@ -8,6 +8,7 @@
 //        strict min-size test, selection key max_c sigmoid(cls) [* sigmoid(ctr)]
 // All of it is small, latency-bound work; the point of the kernels is to replace the
 // reference's Python double loops (GT x level, ~40 launches each) by 2-3 launches per batch.
+#include <algorithm>
 #include <cstring>
 
 #include "common.cuh"
@@ -326,6 +327,83 @@ __global__ void __launch_bounds__(256) k_fcos_decode(FcosArgs p, float* __restri
     key[(long long)b * p.total + c] = ok ? best : -INFINITY;
 }
 
+// ------------------------------------------------------------------ a19: batched per-level selection
+// FCOSHead.predict_single_image's per-level filter + top-k (lib/heads/fcos_head.py:602-613) for a batch, on the key of
+// k_fcos_decode.  Grid (level, image): the CTA counts the valid points (key > -inf) of the earlier levels to find where
+// its level starts in the concatenation, then writes either the level's b2d_topk result (more than pre_nms valid
+// points) or all its valid points in ascending index order.
+constexpr int kDsThreads = 512;
+constexpr int kDsSortCap = 16384;             // largest segment b2d_topk sorts at any pitch (one CTA)
+
+struct DsArgs {
+    const float* key; long long total; int L, pre; long long P;
+    long long off[kMaxLevels]; int n[kMaxLevels];
+    const int* topk[kMaxLevels];              // [B][pre] in-level indices, for levels with n > pre; else NULL
+    const float* boxes; float* sel_boxes;     // [B][4][total] -> [B][4][P] (optional)
+    int* idx; int* count;
+};
+
+__device__ __forceinline__ int ds_block_sum(int v, int* s_red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int t = 0;
+#pragma unroll
+    for (int w = 0; w < kDsThreads / 32; ++w) t += s_red[w];
+    __syncthreads();
+    return t;
+}
+
+__global__ void __launch_bounds__(kDsThreads) k_dense_select(DsArgs p) {
+    __shared__ int s_red[kDsThreads / 32];
+    const int l = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float* key = p.key + (long long)b * p.total;
+    auto valid_in = [&](int q) {
+        int c = 0;
+        for (int i = tid; i < p.n[q]; i += kDsThreads) c += key[p.off[q] + i] > -INFINITY;
+        return ds_block_sum(c, s_red);
+    };
+    auto take = [&](int v) { return (p.pre > 0 && v > p.pre) ? p.pre : v; };
+    int base = 0;
+    for (int q = 0; q < l; ++q) base += take(valid_in(q));
+    const int v = valid_in(l), kl = take(v);
+    int* out = p.idx + (long long)b * p.P;
+    float* sb = p.sel_boxes ? p.sel_boxes + (long long)b * 4 * p.P : nullptr;
+    const float* bx = p.boxes ? p.boxes + (long long)b * 4 * p.total : nullptr;
+    auto put = [&](int pos, long long f) {
+        out[pos] = (int)f;
+        if (sb) { sb[pos] = bx[f]; sb[p.P + pos] = bx[p.total + f]; sb[2 * p.P + pos] = bx[2 * p.total + f]; sb[3 * p.P + pos] = bx[3 * p.total + f]; }
+    };
+    if (kl < v) {                                                   // top pre_nms by key (region.topk_desc order)
+        const int* t = p.topk[l] + (long long)b * p.pre;
+        for (int j = tid; j < kl; j += kDsThreads) put(base + j, p.off[l] + t[j]);
+    } else {                                                        // every valid point, ascending index
+        int run = base;
+        for (int i0 = 0; i0 < p.n[l]; i0 += kDsThreads) {
+            const int i = i0 + tid;
+            const bool ok = i < p.n[l] && key[p.off[l] + i] > -INFINITY;
+            const unsigned bal = __ballot_sync(0xffffffffu, ok);
+            if (lane == 0) s_red[warp] = __popc(bal);
+            __syncthreads();
+            int before = 0, total = 0;
+#pragma unroll
+            for (int w = 0; w < kDsThreads / 32; ++w) { const int c = s_red[w]; before += w < warp ? c : 0; total += c; }
+            if (ok) put(run + before + __popc(bal & ((1u << lane) - 1u)), p.off[l] + i);
+            run += total;
+            __syncthreads();
+        }
+    }
+    if (l == p.L - 1) {                                             // the last level knows the image's count
+        const int cnt = base + kl;
+        if (tid == 0) p.count[b] = cnt;
+        for (long long j = cnt + tid; j < p.P; j += kDsThreads) {
+            out[j] = -1;
+            if (sb) { sb[j] = 0.0f; sb[p.P + j] = 0.0f; sb[2 * p.P + j] = 0.0f; sb[3 * p.P + j] = 0.0f; }
+        }
+    }
+}
+
 }  // namespace b2d
 
 using namespace b2d;
@@ -429,6 +507,85 @@ int b2d_fcos_decode(float* boxes, float* key, float* score, float* ctr_score, co
     dim3 g(cdiv(a.total, 256), B);
     k_fcos_decode<<<g, 256, 0, (cudaStream_t)stream>>>(a, boxes, key, score, ctr_score);
     return check_launch("fcos_decode");
+}
+
+static size_t ds_al(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// Workspace plan of b2d_dense_select: per level with n > pre_nms a top-k output [B][pre] + counts [B]; one packed key
+// buffer [B][n] for the largest such level over kDsSortCap (b2d_topk wants dense segments there); the largest b2d_topk
+// workspace.  false: unsupported.
+static bool ds_plan(const int* n_host, int L, int B, int pre, size_t* bytes, size_t* topk_at, size_t* packed_at,
+                    size_t* ws_at, size_t* ws_len) {
+    if (!n_host || L < 1 || L > kMaxLevels || B < 1) return false;
+    size_t off = 0, topk_ws = 0;
+    long long packed = 0;
+    for (int l = 0; l < L; ++l) {
+        if (n_host[l] < 0) return false;
+        if (topk_at) topk_at[l] = (size_t)-1;
+        if (pre > 0 && n_host[l] > pre) {
+            if (pre > kDsSortCap) return false;
+            const size_t t = b2d_topk_workspace_bytes(n_host[l], B, pre);
+            if (t == 0) return false;
+            topk_ws = std::max(topk_ws, t);
+            if (n_host[l] > kDsSortCap) packed = std::max(packed, (long long)n_host[l]);
+            if (topk_at) topk_at[l] = off;
+            off += ds_al((size_t)B * pre * 4) + ds_al((size_t)B * 4);
+        }
+    }
+    if (packed_at) *packed_at = off;
+    off += ds_al((size_t)B * packed * 4);
+    if (ws_at) *ws_at = off;
+    if (ws_len) *ws_len = topk_ws;
+    *bytes = off + topk_ws + 256;
+    return true;
+}
+
+size_t b2d_dense_select_workspace_bytes(const int* level_sizes_host, int num_levels, int B, int pre_nms) {
+    size_t bytes = 0;
+    return ds_plan(level_sizes_host, num_levels, B, pre_nms, &bytes, nullptr, nullptr, nullptr, nullptr) ? bytes : 0;
+}
+
+int b2d_dense_select(int* idx, int* count, float* sel_boxes, const float* key, const float* boxes,
+                     const int* level_sizes_host, int num_levels, int B, int pre_nms, void* workspace, size_t ws_bytes,
+                     void* stream) {
+    B2D_REQUIRE(idx && count && key && level_sizes_host && (!sel_boxes || boxes), "dense_select: null pointer");
+    size_t bytes = 0, topk_at[kMaxLevels], packed_at = 0, ws_at = 0, ws_len = 0;
+    B2D_REQUIRE(ds_plan(level_sizes_host, num_levels, B, pre_nms, &bytes, topk_at, &packed_at, &ws_at, &ws_len),
+                "dense_select: unsupported configuration (1..8 levels, a level top-k <= 16384)");
+    B2D_REQUIRE(workspace && ws_bytes >= bytes, "dense_select: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    char* w = (char*)workspace;
+    DsArgs a;
+    memset(&a, 0, sizeof(a));
+    a.key = key; a.L = num_levels; a.pre = pre_nms; a.boxes = boxes; a.sel_boxes = sel_boxes; a.idx = idx; a.count = count;
+    long long off = 0, P = 0;
+    for (int l = 0; l < num_levels; ++l) {
+        const int n = level_sizes_host[l];
+        a.off[l] = off; a.n[l] = n;
+        P += (pre_nms > 0 && n > pre_nms) ? pre_nms : n;
+        off += n;
+    }
+    a.total = off; a.P = P;
+    for (int l = 0; l < num_levels; ++l) {
+        if (topk_at[l] == (size_t)-1) continue;
+        const int n = a.n[l];
+        int* tk = (int*)(w + topk_at[l]);
+        int* tc = (int*)(w + topk_at[l] + ds_al((size_t)B * pre_nms * 4));
+        const float* v = key + a.off[l];
+        long long ld = a.total;
+        if (n > kDsSortCap) {                                       // dense [B][n] copy of the level's keys
+            float* pk = (float*)(w + packed_at);
+            if (cudaMemcpy2DAsync(pk, (size_t)n * 4, v, (size_t)a.total * 4, (size_t)n * 4, B, cudaMemcpyDeviceToDevice, st) !=
+                cudaSuccess)
+                return check_launch("dense_select(pack)");
+            v = pk; ld = n;
+        }
+        const int rc = b2d_topk(tk, tc, v, ld, nullptr, n, B, pre_nms, w + ws_at, ws_len, st);
+        if (rc != B2D_OK) return rc;
+        a.topk[l] = tk;
+    }
+    k_dense_select<<<dim3(num_levels, B), kDsThreads, 0, st>>>(a);
+    return check_launch("dense_select");
 }
 
 }  // extern "C"

@@ -730,3 +730,164 @@ class InferHotPath(object):
         torch.cuda.synchronize(self.device)
         if int(self.overflow[0]):
             raise _C.B200DetError("rcnn_detect: more than 16384 (box, class) candidates; raise min_score")
+
+
+class DenseInferHotPath(object):
+    """The test path of the one-stage detectors after the head convolutions, batched: RetinaNet
+    (AnchorHead.predict_single_image, lib/heads/anchor_head.py:207-258; BASELINE config 4) and FCOS / ATSS
+    (FCOSHead.predict_single_image, lib/heads/fcos_head.py:570-631; config 5).
+      head='retina': per-level top pre_nms on the best class score, decode, clamp, size filter (RpnProposals with
+                     score_mode 2 / 3 and do_nms off) -> b2d_dense_detect on the logit maps read in place;
+      head='fcos':   b2d_fcos_decode -> b2d_dense_select (per-level filter + top pre_nms) -> b2d_dense_detect on the
+                     sigmoid scores with the centerness as score factor.
+    b2d_dense_detect is utils.multiclass_nms for all images at once: candidate test, ordered compaction, class-offset NMS,
+    the first max_per_img survivors, and optionally the packed records of dist.pack_detections.
+    num_classes counts the background as the reference heads do: a sigmoid head (RetinaNet with use_sigmoid, FCOS) has
+    num_classes - 1 class channels and 1-based labels, a softmax head num_classes channels with channel 0 the background.
+    Everything is allocated here; step() reads nothing back to the host, so a step can be captured in one CUDA graph after
+    a first eager call.  More than 16384 (box, class) candidates in an image set a device flag that check() raises."""
+
+    def __init__(self, B, grids, device, head="retina", num_classes=21, test_cfg=None, strides=(8, 16, 32, 64, 128),
+                 use_sigmoid=True, anchor_scales=tuple(4 * 2 ** (i / 3) for i in range(3)), anchor_ratios=(0.5, 1.0, 2.0),
+                 center_lt=False, target_means=(0.0, 0.0, 0.0, 0.0), target_stds=(1.0, 1.0, 1.0, 1.0), reg_mean=0.0,
+                 reg_std=300.0, use_centerness=True, scale_factor=1.0):
+        if head not in ("retina", "fcos"):
+            raise _C.B200DetError("DenseInferHotPath: head must be 'retina' or 'fcos', got %r" % (head,))
+        test_cfg = test_cfg or dict(pre_nms=1000, min_bbox_size=0, min_score=0.05, nms_iou=0.5, max_per_img=100,
+                                    nms_type="strict")
+        get = (lambda k, d=None: test_cfg.get(k, d)) if hasattr(test_cfg, "get") else (lambda k, d=None: getattr(test_cfg, k, d))
+        mode = get("nms_type", "official")
+        if mode not in ("official", "strict"):
+            raise _C.B200DetError("DenseInferHotPath: nms_type must be 'official' or 'strict'")
+        self.B, self.device, self.head = int(B), device, head
+        self.grids = [tuple(int(v) for v in g) for g in grids]
+        self.L = len(self.grids)
+        sigmoid = head == "fcos" or bool(use_sigmoid)
+        self.C = C = int(num_classes) - 1 if sigmoid else int(num_classes)
+        if not 1 <= C <= 128:
+            raise _C.B200DetError("DenseInferHotPath: 1..128 class channels supported, got %d" % C)
+        self.pre = int(get("pre_nms", 0) or 0)
+        min_bbox = float(get("min_bbox_size", 0) or 0)
+        self.min_score = float(np.float32(get("min_score", -1)))
+        self.nms_thr = _C.floor_f32(float(get("nms_iou")))
+        self.strict = int(mode == "strict")
+        chans = list(range(0, C)) if sigmoid else list(range(1, C))
+        mask = [0, 0]
+        for c in chans:
+            mask[c >> 6] |= 1 << (c & 63)
+        self.chan = (_C.c_ull * 2)(*mask)
+        self.label_add = 1 if sigmoid else 0
+        self.lv = _C.DenseLevels()
+        if head == "retina":
+            self.transform = 1 if sigmoid else 2
+            self.pyr = AnchorPyramid(strides, self.grids, tuple(anchor_scales), tuple(anchor_ratios), center_lt)
+            self.A = self.pyr.num_anchors
+            sel_cfg = dict(pre_nms=self.pre, post_nms=0, max_num=0, nms_iou=0.5, min_bbox_size=min_bbox)
+            self.select = RpnProposals(self.pyr, B, sel_cfg, target_means, target_stds, device,
+                                       score_mode=2 if sigmoid else 3, cls_channels=C, do_nms=False, scale_factor=scale_factor)
+            self.P = self.select.P
+            self.lv.num_levels = self.L
+            for l, n in enumerate(self.pyr.level_sizes):              # cls_l.view(B, C, -1): [B][C][A*H*W]
+                self.lv.offset[l], self.lv.img_stride[l], self.lv.class_stride[l] = int(self.pyr.c.lv[l].offset), C * n, n
+        else:
+            from . import heads
+            self.transform, self.centerness = 0, bool(use_centerness)
+            self.pyr_c = heads._point_pyramid(self.grids, strides, 8)
+            self.total = T = int(self.pyr_c.total)
+            sizes = [h * w for h, w in self.grids]
+            self.sizes = (_C.c_int * _C.MAX_LEVELS)(*sizes)
+            self.P = sum(min(self.pre, n) if self.pre > 0 else n for n in sizes)
+            self.reg_mean, self.reg_std = float(reg_mean), float(reg_std)
+            self.min_size = float(np.float32(scale_factor * min_bbox))
+            self.boxes = torch.zeros((B, 4, T), dtype=torch.float32, device=device)
+            self.key = torch.zeros((B, T), dtype=torch.float32, device=device)
+            self.score = torch.zeros((B, C, T), dtype=torch.float32, device=device)
+            self.ctrs = torch.zeros((B, T), dtype=torch.float32, device=device) if self.centerness else None
+            self.sel_idx = torch.zeros((B, self.P), dtype=torch.int32, device=device)
+            self.sel_count = torch.zeros(B, dtype=torch.int32, device=device)
+            self.sel_boxes = torch.zeros((B, 4, self.P), dtype=torch.float32, device=device)
+            nb = _C.lib().b2d_dense_select_workspace_bytes(self.sizes, self.L, B, self.pre)
+            if nb == 0:
+                raise _C.B200DetError("DenseInferHotPath: unsupported selection (1..8 levels, a level top-k <= 16384)")
+            self.sel_ws = torch.empty(nb, dtype=torch.uint8, device=device)
+            self.lv.num_levels = 1                                    # score [B][C][total] as one level
+            self.lv.offset[0], self.lv.img_stride[0], self.lv.class_stride[0] = 0, C * T, T
+            self.lv.base[0] = self.score.data_ptr()
+        self.cap = max(1, min(16384, self.P * (len(chans) if not self.strict else 1)))
+        mpi = get("max_per_img")
+        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap))
+        self.det_box = torch.zeros((B, 4, M), dtype=torch.float32, device=device)
+        self.det_score = torch.zeros((B, M), dtype=torch.float32, device=device)
+        self.det_label = torch.zeros((B, M), dtype=torch.int64, device=device)
+        self.det_count = torch.zeros(B, dtype=torch.int32, device=device)
+        self.overflow = torch.zeros(1, dtype=torch.int32, device=device)
+        self.det_ws = torch.empty(_C.lib().b2d_rcnn_detect_workspace_bytes(self.cap, B), dtype=torch.uint8, device=device)
+
+    def _check_maps(self, what, maps, per_cell):
+        if maps is None or len(maps) != self.L:
+            raise _C.B200DetError("DenseInferHotPath.step: %s needs %d levels" % (what, self.L))
+        for (h, w), t in zip(self.grids, maps):
+            if (tuple(t.shape) != (self.B, per_cell, h, w) or t.dtype != torch.float32 or not t.is_contiguous()
+                    or not t.is_cuda):
+                raise _C.B200DetError("DenseInferHotPath.step: %s level of shape %s (%s), expected contiguous fp32 CUDA "
+                                      "[%d, %d, %d, %d]" % (what, tuple(t.shape), t.dtype, self.B, per_cell, h, w))
+
+    def step(self, cls_outs, reg_outs, img_hw, ctr_outs=None, records=None, mark=None, detect_events=None):
+        """cls_outs / reg_outs (/ ctr_outs for FCOS with centerness): the head maps per level, contiguous fp32 --
+        RetinaNet [B, A*C, H, W] / [B, 4A, H, W], FCOS [B, C, H, W] / [B, 4, H, W] / [B, 1, H, W]; img_hw fp32 [B, 2];
+        records: optional fp32 [B, max_per_img, 6] that receives the packed detections of dist.pack_detections;
+        mark(name): optional callable run after each phase; detect_events: optional two torch.cuda.Event (already
+        recorded once) that the detection call records after its candidate stage and after its NMS.  Returns the
+        detections (boxes [B,4,M], scores [B,M], labels int64 [B,M], count int32 [B]) and the selected rows."""
+        B = self.B
+        if tuple(img_hw.shape) != (B, 2) or img_hw.dtype != torch.float32 or not img_hw.is_contiguous():
+            raise _C.B200DetError("DenseInferHotPath.step: img_hw must be contiguous fp32 [%d, 2]" % B)
+        if records is not None and (tuple(records.shape) != (B, self.M, 6) or records.dtype != torch.float32
+                                    or not records.is_contiguous()):
+            raise _C.B200DetError("DenseInferHotPath.step: records must be contiguous fp32 [%d, %d, 6]" % (B, self.M))
+        if self.head == "retina":
+            self._check_maps("cls_outs", cls_outs, self.A * self.C)
+            self._check_maps("reg_outs", reg_outs, 4 * self.A)
+            boxes, count, rows = self.select(cls_outs, reg_outs, img_hw)[0], self.select.count, self.select.prov
+            for l, t in enumerate(cls_outs):
+                self.lv.base[l] = t.data_ptr()
+            factor = None
+            if mark is not None:
+                mark("selection")
+        else:
+            self._check_maps("cls_outs", cls_outs, self.C)
+            self._check_maps("reg_outs", reg_outs, 4)
+            if self.centerness:
+                self._check_maps("ctr_outs", ctr_outs, 1)
+            _C.call("b2d_fcos_decode", _C.ptr(self.boxes), _C.ptr(self.key), _C.ptr(self.score), _C.ptr(self.ctrs),
+                    _ptrs(cls_outs), _ptrs(reg_outs), _ptrs(ctr_outs) if self.centerness else None, ctypes.byref(self.pyr_c),
+                    self.C, self.reg_mean, self.reg_std, self.min_size, _C.ptr(img_hw), B, _C.stream())
+            if mark is not None:
+                mark("decode")
+            _C.call("b2d_dense_select", _C.ptr(self.sel_idx), _C.ptr(self.sel_count), _C.ptr(self.sel_boxes), _C.ptr(self.key),
+                    _C.ptr(self.boxes), self.sizes, self.L, B, self.pre, _C.ptr(self.sel_ws), self.sel_ws.numel(), _C.stream())
+            boxes, count, rows, factor = self.sel_boxes, self.sel_count, self.sel_idx, self.ctrs
+            if mark is not None:
+                mark("selection")
+        ev = None
+        if detect_events is not None:
+            ev = (_C.c_void_p * 2)(*[e.cuda_event for e in detect_events])
+        args = [_C.ptr(self.det_box), _C.ptr(self.det_score), _C.ptr(self.det_label), _C.ptr(self.det_count)]
+        if records is not None:
+            args.append(_C.ptr(records))
+        args += [_C.ptr(boxes), self.P, _C.ptr(count), _C.ptr(rows), ctypes.byref(self.lv), self.C, self.transform,
+                 _C.ptr(factor), self.total if factor is not None else 0, self.chan, self.min_score, self.label_add,
+                 self.nms_thr, self.M, self.strict, self.cap, B, _C.ptr(self.overflow), _C.ptr(self.det_ws),
+                 self.det_ws.numel(), ev, _C.stream()]
+        _C.call("b2d_dense_detect_records" if records is not None else "b2d_dense_detect", *args)
+        if mark is not None:
+            mark("detect")
+        return dict(boxes=self.det_box, scores=self.det_score, labels=self.det_label, count=self.det_count,
+                    records=records, sel_boxes=boxes, sel_count=count, sel_rows=rows)
+
+    def check(self):
+        """Synchronise and raise if the last step had an image with more than 16384 (box, class) candidates (its
+        candidates past the cap were dropped in enumeration order)."""
+        torch.cuda.synchronize(self.device)
+        if int(self.overflow[0]):
+            raise _C.B200DetError("dense_detect: more than 16384 (box, class) candidates in an image; raise min_score")
