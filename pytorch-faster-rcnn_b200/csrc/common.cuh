@@ -80,6 +80,9 @@ static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b)
 
 // ---- monotone float <-> uint key (larger float => larger key; total order) ----
 __host__ __device__ __forceinline__ uint32_t f2key(float f) {
+    // -0.0 and +0.0 compare equal (torch.topk / sort treat them as one value and order the tie by index): one key for
+    // both, else a -0.0 logit would rank below a +0.0 one of a higher index
+    f = f + 0.0f;
 #ifdef __CUDA_ARCH__
     uint32_t u = __float_as_uint(f);
 #else

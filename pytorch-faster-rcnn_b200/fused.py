@@ -651,6 +651,10 @@ class InferHotPath(object):
         rcnn_test = rcnn_test or dict(min_score=0.05, nms_iou=0.5, max_per_img=100, nms_type='official')
         if not 1 <= num_stages <= len(stage_stds):
             raise ValueError("num_stages must be in 1..%d (one stds tuple per stage)" % len(stage_stds))
+        if not 2 <= int(num_classes) <= 128:
+            # b2d_rcnn_detect holds a row's classes in one warp; without this check the first step would only fail at
+            # the detection call, after the proposals, RoIAlign and the caller's head (or in the middle of a graph capture)
+            raise _C.B200DetError("InferHotPath: 2..128 classes (background included) supported, got %d" % int(num_classes))
         z4 = (0.0, 0.0, 0.0, 0.0)
         self.B, self.device, self.S = B, device, int(num_stages)
         self.NC, self.reg_c = int(num_classes), 1 if reg_class_agnostic else int(num_classes)
