@@ -34,12 +34,6 @@ static void load_knobs() {
     k.nms_sweep = geti("B2D_NMS_SWEEP", 1);
     k.sweep_t = geti("B2D_SWEEP_T", 0);
     k.sweep_g = geti("B2D_SWEEP_G", 0);
-    k.roi_tma = geti("B2D_ROI_TMA", 0);
-    k.roi_pf = geti("B2D_ROI_PF", 0);
-    k.roi_order = geti("B2D_ROI_ORDER", 0);
-    k.roi_x2 = geti("B2D_ROI_X2", 1);
-    k.roi_bulk_store = geti("B2D_ROI_BULK_STORE", 1);
-    k.roi_tma_dev = geti("B2D_ROI_TMA_DEV", 0);
     k.roi_bwd_tile = geti("B2D_ROI_BWD_TILE", 2);
     k.assign_old = getenv("B2D_ASSIGN_OLD") != nullptr;
     k.sample_threads = geti("B2D_SAMPLE_THREADS", 1024);

@@ -30,12 +30,6 @@ struct Knobs {
     int nms_p1_chains;     // B2D_NMS_P1_CHAINS
     int nms_sweep;         // B2D_NMS_SWEEP      0 disables the x-sweep mask kernel
     int sweep_t, sweep_g;  // B2D_SWEEP_T / _G   launch shape of k_nms_sweep
-    int roi_tma;           // B2D_ROI_TMA        1: TMA-ring RoIAlign, 2: tensor-map window RoIAlign
-    int roi_pf;            // B2D_ROI_PF         L2 prefetch distance of k_roi_align_win
-    int roi_order;         // B2D_ROI_ORDER
-    int roi_x2;            // B2D_ROI_X2         0: scalar adds in k_roi_align_win
-    int roi_bulk_store;    // B2D_ROI_BULK_STORE 0: result tile through LDS + STG instead of one bulk async store
-    int roi_tma_dev;       // B2D_ROI_TMA_DEV
     int roi_bwd_tile;      // B2D_ROI_BWD_TILE   2: patch form (default), 1: tile-gather form, 0: generic backward kernel
     int assign_old;        // B2D_ASSIGN_OLD     1: round-1a assignment kernels in pyramid mode
     int debug_sync;        // B2D_DEBUG_SYNC     synchronise after every launch (localise a faulting kernel)

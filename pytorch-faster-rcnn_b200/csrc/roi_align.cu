@@ -12,7 +12,7 @@
 //                     128-channel tile), lanes across channels; the distinct tap cells of a
 //                     bin are loaded once as coalesced 128-bit channel quads, all loads of a
 //                     bin in flight together; the [C,7,7] result is staged in shared memory
-//                     in its HBM layout and leaves as contiguous 128-bit stores.
+//                     in its HBM layout and leaves as one bulk async store.
 //   k_roi_align_nhwc  NHWC, any fixed sampling ratio: per-sample tap descriptors in smem.
 //   k_roi_align_any   generic fallback (NCHW input, adaptive sampling, odd shapes):
 //                     one thread per output element, pw fastest.
@@ -139,9 +139,6 @@ __global__ void __launch_bounds__(256) k_roi_align_nhwc(RoiArgs a, float* __rest
 }
 
 
-template <typename FT>
-__device__ __forceinline__ float4 ld4b(const char* p) { return ld4(reinterpret_cast<const FT*>(p)); }
-
 // ---- window kernel (2x2 samples per bin: every reference config) --------------------------------
 // Design notes from the ncu captures of round 1 (profiles/):
 //  * ptxas, left to its default occupancy target, sinks every tap load next to its use (2 loads
@@ -165,60 +162,38 @@ struct __align__(16) BinTab {
     int pat, _p0, _p1, _p2;
 };
 
-// V consecutive channels of one cell as fp32 (V = 4: one 128-bit load of fp32 / 64-bit of bf16)
-template <int V> struct VecF { float f[V]; };
-
-template <typename FT, int V>
-__device__ __forceinline__ VecF<V> ldv(const char* p) {
-    VecF<V> o;
-    if constexpr (sizeof(FT) == 4 && V == 4) {
-        const float4 t = __ldg(reinterpret_cast<const float4*>(p));
-        o.f[0] = t.x; o.f[1] = t.y; o.f[2] = t.z; o.f[3] = t.w;
-    } else if constexpr (sizeof(FT) == 4 && V == 2) {
-        const float2 t = __ldg(reinterpret_cast<const float2*>(p));
-        o.f[0] = t.x; o.f[1] = t.y;
-    } else if constexpr (sizeof(FT) == 2 && V == 4) {
-        const float4 t = ld4(reinterpret_cast<const __nv_bfloat16*>(p));
-        o.f[0] = t.x; o.f[1] = t.y; o.f[2] = t.z; o.f[3] = t.w;
-    } else {
-        const unsigned u = __ldg(reinterpret_cast<const unsigned*>(p));
-        const float2 t = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
-        o.f[0] = t.x; o.f[1] = t.y;
-    }
-    return o;
-}
-
-template <typename FT, int V, int PY, int PX>
-__device__ __forceinline__ VecF<V> bin_eval(const char* fb, const BinTab* t) {
+// bf16 features (4 channels per lane, one 64-bit load per cell, converted to fp32): scalar additions
+template <int PY, int PX>
+__device__ __forceinline__ float4 bin_eval(const char* fb, const BinTab* t) {
     const int4 ry = *reinterpret_cast<const int4*>(t->ry);
     const int4 cx = *reinterpret_cast<const int4*>(t->cx);
     const int ryv[4] = {ry.x, ry.y, ry.z, ry.w}, cxv[4] = {cx.x, cx.y, cx.z, cx.w};
-    VecF<V> v[4][4];
+    float4 v[4][4];
 #pragma unroll
     for (int r = 0; r < PY + 2; ++r) {
         const char* rp = fb + ryv[r];
 #pragma unroll
-        for (int c = 0; c < PX + 2; ++c) v[r][c] = ldv<FT, V>(rp + cxv[c]);
+        for (int c = 0; c < PX + 2; ++c) v[r][c] = ld4(reinterpret_cast<const __nv_bfloat16*>(rp + cxv[c]));
     }
-    VecF<V> acc;
-#pragma unroll
-    for (int e = 0; e < V; ++e) acc.f[e] = 0.0f;
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int iy = 0; iy < 2; ++iy) {
 #pragma unroll
         for (int ix = 0; ix < 2; ++ix) {
             const int r0 = iy ? PY : 0, c0 = ix ? PX : 0;
             const float4 w = *reinterpret_cast<const float4*>(&t->w[(iy * 2 + ix) * 4]);
-#pragma unroll
-            for (int e = 0; e < V; ++e)      // torchvision's order: ((w1 v1 + w2 v2) + w3 v3) + w4 v4, summed over samples
-                acc.f[e] += ((w.x * v[r0][c0].f[e] + w.y * v[r0][c0 + 1].f[e]) + w.z * v[r0 + 1][c0].f[e]) +
-                            w.w * v[r0 + 1][c0 + 1].f[e];
+            const float4 &v1 = v[r0][c0], &v2 = v[r0][c0 + 1], &v3 = v[r0 + 1][c0], &v4 = v[r0 + 1][c0 + 1];
+            // torchvision's order: ((w1 v1 + w2 v2) + w3 v3) + w4 v4, summed over samples
+            acc.x += ((w.x * v1.x + w.y * v2.x) + w.z * v3.x) + w.w * v4.x;
+            acc.y += ((w.x * v1.y + w.y * v2.y) + w.z * v3.y) + w.w * v4.y;
+            acc.z += ((w.x * v1.z + w.y * v2.z) + w.z * v3.z) + w.w * v4.z;
+            acc.w += ((w.x * v1.w + w.y * v2.w) + w.z * v3.w) + w.w * v4.w;
         }
     }
     return acc;
 }
 
-// Packed-add variant (fp32 features, 4 channels per lane): the same products and sums in the same order, with the
+// fp32 features (4 channels per lane, one 128-bit load per cell): the same products and sums in the same order, with the
 // additions two channels per instruction (add.rn.f32x2 -> FADD2).  The products stay scalar FMULs on purpose:
 // ptxas (CUDA 12.9) contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 even with -fmad=false, which would change
 // the rounding; a scalar product feeding a packed add is left alone (checked in SASS).
@@ -233,7 +208,7 @@ __device__ __forceinline__ unsigned long long pack2(float lo, float hi) {
     return r;
 }
 template <int PY, int PX>
-__device__ __forceinline__ VecF<4> bin_eval_x2(const char* fb, const BinTab* t) {
+__device__ __forceinline__ float4 bin_eval_x2(const char* fb, const BinTab* t) {
     const int4 ry = *reinterpret_cast<const int4*>(t->ry);
     const int4 cx = *reinterpret_cast<const int4*>(t->cx);
     const int ryv[4] = {ry.x, ry.y, ry.z, ry.w}, cxv[4] = {cx.x, cx.y, cx.z, cx.w};
@@ -258,9 +233,9 @@ __device__ __forceinline__ VecF<4> bin_eval_x2(const char* fb, const BinTab* t) 
                                       pack2(w.z * v3.z, w.z * v3.w)), pack2(w.w * v4.z, w.w * v4.w)));
         }
     }
-    VecF<4> acc;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(acc.f[0]), "=f"(acc.f[1]) : "l"(a01));
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(acc.f[2]), "=f"(acc.f[3]) : "l"(a23));
+    float4 acc;
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(acc.x), "=f"(acc.y) : "l"(a01));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(acc.z), "=f"(acc.w) : "l"(a23));
     return acc;
 }
 
@@ -268,20 +243,14 @@ __device__ __forceinline__ void sts_f32(unsigned addr, float v) {
     asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
 }
 
-// NT threads per CTA, CT channels per CTA (grid.y = C / CT tiles), MINB = min resident CTAs/SM
+// NT threads per CTA, CT channels per CTA (grid.y = C / CT tiles), 4 channels per lane, MINB = min resident CTAs/SM
 // (the register bound that keeps the window loads batched, see the notes above).
-template <typename FT, int NT, int CT, int MINB, int V, int X2 = 0>
+template <typename FT, int NT, int CT, int MINB>
 __global__ void __launch_bounds__(NT, MINB) k_roi_align_win(RoiArgs a, float* __restrict__ out) {
-    static_assert(!X2 || (sizeof(FT) == 4 && V == 4), "packed path: fp32 features, 4 channels per lane");
     using Tab = BinTab;
     extern __shared__ __align__(16) float s_tile[];                      // [CT][bins] (+ bin table behind it)
-    long long r = a.tiles > 0 ? blockIdx.x / a.tiles : blockIdx.x;
-    const int tile = a.tiles > 0 ? blockIdx.x % a.tiles : blockIdx.y;
-    if (a.sel_m > 1) {                                  // heterogeneous split: this kernel takes the RoIs with r % m != 0
-        const long long q = r / (a.sel_m - 1);
-        r = q * a.sel_m + 1 + (r - q * (a.sel_m - 1));
-        if (r >= a.R) return;
-    }
+    const long long r = blockIdx.x;
+    const int tile = blockIdx.y;
     const b2d_roi_cfg& c = a.cfg;
     float x1, y1, x2, y2;
     int img;
@@ -293,45 +262,6 @@ __global__ void __launch_bounds__(NT, MINB) k_roi_align_win(RoiArgs a, float* __
     const int bins = c.PH * c.PW;
     Tab* s_tab = reinterpret_cast<Tab*>(s_tile + CT * bins);
     const RoiGeom g = roi_geom(x1, y1, x2, y2, c.spatial_scale[lvl], c.PH, c.PW, 2, c.aligned);
-    // L2 prefetch for the RoI that runs `pf_dist` CTAs later: one bulk prefetch per feature row of
-    // its tap rectangle (rows are contiguous in NHWC).  Costs no registers, and turns the DRAM
-    // round trips of that CTA's gathers into L2 hits.
-    if (a.pf_dist > 0 && threadIdx.x >= 64 && threadIdx.x < 128) {
-        const long long r2 = r + a.pf_dist;
-        float px1, py1, px2, py2;
-        int img2;
-        if (r2 < a.R && roi_fetch(a, r2, img2, px1, py1, px2, py2)) {
-            const int lvl2 = a.levels ? a.levels[r2]
-                                      : (c.num_levels > 1 ? roi_level(px1, py1, px2, py2, c.finest_scale, c.num_levels) : 0);
-            const int H2 = c.H[lvl2], W2 = c.W[lvl2];
-            const RoiGeom g2 = roi_geom(px1, py1, px2, py2, c.spatial_scale[lvl2], c.PH, c.PW, 2, c.aligned);
-            const AxisTap ya = axis_tap(g2.sy, g2.bh, 0, 0, 2, H2), yb = axis_tap(g2.sy, g2.bh, c.PH - 1, 1, 2, H2);
-            const AxisTap xa = axis_tap(g2.sx, g2.bw, 0, 0, 2, W2), xb = axis_tap(g2.sx, g2.bw, c.PW - 1, 1, 2, W2);
-            const int ylo = min(ya.lo, yb.lo), yhi = max(ya.hi, yb.hi);
-            const int xlo = min(xa.lo, xb.lo), xhi = max(xa.hi, xb.hi);
-            const FT* f2 = reinterpret_cast<const FT*>(a.feat[lvl2]) + (long long)img2 * H2 * W2 * C;
-            const unsigned bytes = (unsigned)(xhi - xlo + 1) * C * (unsigned)sizeof(FT);
-            for (int y = ylo + (int)threadIdx.x - 64; y <= yhi; y += 64) {
-                const FT* ptr = f2 + ((long long)y * W2 + xlo) * C;
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(ptr), "r"(bytes) : "memory");
-            }
-        }
-    }
-    if (a.pf_dist == -1) {
-        // dev knob B2D_ROI_PF=-1: own tap rectangle, this CTA's channel slice only -- every DRAM request of the CTA is in
-        // flight before the first bin is evaluated.  Measured r2: 150.0 vs 152.0 us (cold L2): the per-bin waits are not
-        // DRAM latency; prefetching the next bin's window from inside the bin loop (CCTL.E.PF2 x 2 per lane): 156 us.
-        const AxisTap ya = axis_tap(g.sy, g.bh, 0, 0, 2, H), yb = axis_tap(g.sy, g.bh, c.PH - 1, 1, 2, H);
-        const AxisTap xa = axis_tap(g.sx, g.bw, 0, 0, 2, W), xb = axis_tap(g.sx, g.bw, c.PW - 1, 1, 2, W);
-        const int ylo = min(ya.lo, yb.lo), yhi = max(ya.hi, yb.hi), xlo = min(xa.lo, xb.lo), xhi = max(xa.hi, xb.hi);
-        const int wc = xhi - xlo + 1, lines = CT * (int)sizeof(FT) / 128, n = (yhi - ylo + 1) * wc * lines;
-        const char* f0 = reinterpret_cast<const char*>(reinterpret_cast<const FT*>(a.feat[lvl]) + (long long)img * H * W * C + tile * CT);
-        for (int i = threadIdx.x; i < n; i += NT) {
-            const int cell = i / lines, ln = i - cell * lines, yy = cell / wc, xx = cell - yy * wc;
-            const char* ptr = f0 + ((long long)(ylo + yy) * W + (xlo + xx)) * C * (int)sizeof(FT) + ln * 128;
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(ptr));
-        }
-    }
     if ((int)threadIdx.x < bins) {
         const int bin = threadIdx.x, ph = bin / c.PW, pw = bin - ph * c.PW;
         const AxisTap ty0 = axis_tap(g.sy, g.bh, ph, 0, 2, H), ty1 = axis_tap(g.sy, g.bh, ph, 1, 2, H);
@@ -366,12 +296,12 @@ __global__ void __launch_bounds__(NT, MINB) k_roi_align_win(RoiArgs a, float* __
     }
     __syncthreads();
     const FT* feat = reinterpret_cast<const FT*>(a.feat[lvl]) + (long long)img * H * W * C;
-    constexpr int LG = CT / V, NG = NT / LG;               // lanes per bin group, bin groups
+    constexpr int LG = CT / 4, NG = NT / LG;               // lanes per bin group, bin groups
     const int cq = threadIdx.x % LG, grp = threadIdx.x / LG;
     float* o = out + r * (long long)C * bins;
     {
         const int c0 = tile * CT;
-        const int ch = c0 + cq * V;
+        const int ch = c0 + cq * 4;
         if (ch < C) {
             const char* fb = reinterpret_cast<const char*>(feat + ch);
             // The lanes of a warp are 4 * bins floats apart in the [channel][bin] tile, i.e. on 8 banks only; lane
@@ -382,15 +312,15 @@ __global__ void __launch_bounds__(NT, MINB) k_roi_align_win(RoiArgs a, float* __
             const int rot = (cq >> 3) & 3;
             const bool r1 = rot & 1, r2 = rot & 2;
             const int4* s_rot = reinterpret_cast<const int4*>(s_tab + bins) + rot;
-            const unsigned st_base = (unsigned)__cvta_generic_to_shared(s_tile + (cq * V) * bins);
+            const unsigned st_base = (unsigned)__cvta_generic_to_shared(s_tile + (cq * 4) * bins);
             for (int bin = grp; bin < bins; bin += NG) {
                 const Tab* t = s_tab + bin;
-                VecF<V> acc;
+                float4 acc;
                 const int pat = t->pat, py = pat / 3, px = pat - py * 3;   // uniform over the warps of a bin
 #define B2D_BIN(PY_, PX_)                                                  \
     do {                                                                   \
-        if constexpr (X2) acc = bin_eval_x2<PY_, PX_>(fb, t);              \
-        else acc = bin_eval<FT, V, PY_, PX_>(fb, t);                       \
+        if constexpr (sizeof(FT) == 4) acc = bin_eval_x2<PY_, PX_>(fb, t); \
+        else acc = bin_eval<PY_, PX_>(fb, t);                              \
     } while (0)
                 if (py == 0) {
                     if (px == 0) B2D_BIN(0, 0);
@@ -406,43 +336,31 @@ __global__ void __launch_bounds__(NT, MINB) k_roi_align_win(RoiArgs a, float* __
                     else B2D_BIN(2, 2);
                 }
 #undef B2D_BIN
-                // x / 4 == x * 0.25 exactly; rotated stores, see st_rot above
-                if constexpr (V == 4) {
-                    const float f0 = acc.f[0] * 0.25f, f1 = acc.f[1] * 0.25f, f2 = acc.f[2] * 0.25f, f3 = acc.f[3] * 0.25f;
-                    const float g0 = r1 ? f1 : f0, g1 = r1 ? f2 : f1, g2 = r1 ? f3 : f2, g3 = r1 ? f0 : f3;
-                    const int4 ro = *s_rot;
-                    const unsigned sb = st_base + bin * 4;
-                    sts_f32(sb + ro.x, r2 ? g2 : g0);       // f[(s + rot) % 4] at step s
-                    sts_f32(sb + ro.y, r2 ? g3 : g1);
-                    sts_f32(sb + ro.z, r2 ? g0 : g2);
-                    sts_f32(sb + ro.w, r2 ? g1 : g3);
-                } else {
-                    float* st = s_tile + (cq * V) * bins + bin;
-#pragma unroll
-                    for (int e = 0; e < V; ++e) st[e * bins] = acc.f[e] * 0.25f;
-                }
+                // x / 4 == x * 0.25 exactly; rotated stores, see the rotation note above
+                const float f0 = acc.x * 0.25f, f1 = acc.y * 0.25f, f2 = acc.z * 0.25f, f3 = acc.w * 0.25f;
+                const float g0 = r1 ? f1 : f0, g1 = r1 ? f2 : f1, g2 = r1 ? f3 : f2, g3 = r1 ? f0 : f3;
+                const int4 ro = *s_rot;
+                const unsigned sb = st_base + bin * 4;
+                sts_f32(sb + ro.x, r2 ? g2 : g0);       // f[(s + rot) % 4] at step s
+                sts_f32(sb + ro.y, r2 ? g3 : g1);
+                sts_f32(sb + ro.z, r2 ? g0 : g2);
+                sts_f32(sb + ro.w, r2 ? g1 : g3);
             }
         }
+        // the [ctile][bins] tile is contiguous in shared memory and in HBM: ONE bulk async store (TMA engine) instead
+        // of an LDS.128 + STG.128 per 16 bytes through the LSU pipe, which this kernel keeps 64 % busy (ncu r1j).
+        // C % 4 == 0 (checked by the launcher) makes its size and its offset in the output multiples of 16 bytes.
         const int ctile = min(CT, C - c0);
-        const int total = ctile * bins;                    // multiple of 4 (checked by the launcher)
-        if (a.bulk_store) {
-            // the [ctile][bins] tile is contiguous in shared memory and in HBM: ONE bulk async store (TMA engine) instead
-            // of an LDS.128 + STG.128 per 16 bytes through the LSU pipe, which this kernel keeps 64 % busy (ncu r1j)
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                const unsigned src = (unsigned)__cvta_generic_to_shared(s_tile);
-                float* dstp = o + (long long)c0 * bins;
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dstp), "r"(src), "r"((unsigned)(total * 4)) : "memory");
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            }
-            return;
-        }
+        const int total = ctile * bins;
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncthreads();
-        float4* dst = reinterpret_cast<float4*>(o + (long long)c0 * bins);
-        const float4* src = reinterpret_cast<const float4*>(s_tile);
-        for (int q = threadIdx.x; q < total / 4; q += NT) dst[q] = src[q];
+        if (threadIdx.x == 0) {
+            const unsigned src = (unsigned)__cvta_generic_to_shared(s_tile);
+            float* dstp = o + (long long)c0 * bins;
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dstp), "r"(src), "r"((unsigned)(total * 4)) : "memory");
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+        }
     }
 }
 
@@ -546,63 +464,21 @@ static int roi_align_launch(float* out, const void* const* feat_ptrs_host, const
                       bins * c.sampling_ratio * c.sampling_ratio <= kMaxSamples && (c.C % 4) == 0 &&
                       bins * (kCTile + 4) * 4 <= 200 * 1024;
     // 2x2 samples per bin (every reference config): window kernel, 128 channels per 128-thread CTA
-    const bool win = fast && c.sampling_ratio == 2 && bins <= 64 && (((long long)c.C * bins) % 4) == 0 &&
-                     ((128ll * bins) % 4) == 0;
+    const bool win = fast && c.sampling_ratio == 2 && bins <= 64;
     if (win) {
-        // TMA-ring kernel (roi_align_tma.cu): opt-in with B2D_ROI_TMA=1.  Bit-identical, but measured slower than
-        // the L1-path kernel below on config 2 (380 vs 159 us, round 1: issue-bound consumers, see DESIGN.md).
-        const int use_tma = knobs().roi_tma;
-        cudaStream_t side = nullptr;
-        cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-        bool hetero = false;
-        if (use_tma == 2) {                               // tensor-map band kernel (roi_align_tband.cu)
-            const int nimg = batched_ld > 0 ? (int)(R / batched_ld) : (1 << 20);     // image-index bound of the 4-D tensor map
-            const int rc = roi_align_tband_try(a, out, nimg, st);
-            if (rc != 1) return rc;
-        } else if (use_tma == 3 && c.layout == 1 && R >= 64 && roi_hetero_streams(&side, &ev_fork, &ev_join)) {
-            // heterogeneous: one persistent tensor-map CTA per SM (97 KB of shared memory, 24 K registers) takes every m-th
-            // RoI; the window kernel below takes the others and finds room for 4 CTAs beside it (smem-bound in-flight
-            // bytes + register-bound in-flight bytes on the same SM)
-            const int m = knobs().roi_tma_dev >= 2 ? knobs().roi_tma_dev : 4;
-            const int nimg = batched_ld > 0 ? (int)(R / batched_ld) : (1 << 20);
-            int sms = 148, dev = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            RoiArgs t = a;
-            t.sel_m = m;
-            cudaEventRecord(ev_fork, st);
-            cudaStreamWaitEvent(side, ev_fork, 0);
-            const int rc = roi_align_tband_try(t, out, nimg, side, sms);
-            if (rc == B2D_OK) { a.sel_m = m; hetero = true; }
-            else if (rc != 1) return rc;
-            cudaEventRecord(ev_join, side);
-        } else if (use_tma == 1) {
-            const int rc = roi_align_tma_try(a, out, st);
-            if (rc != 1) return rc;
-        }
-        a.pf_dist = knobs().roi_pf;
-        // bulk store of the result tile: needs 16-byte multiples (tile bytes and its offset in the output)
-        a.bulk_store = knobs().roi_bulk_store && ((128ll * bins * 4) % 16 == 0) && (((long long)c.C * bins * 4) % 16 == 0) ? 1 : 0;   // dev knob (L2 prefetch: measured slower, r1)
         int rc5 = 0;
         auto launch5 = [&](auto kern, int nt, int ct) {
             const size_t smem5 = (size_t)ct * bins * 4 + (size_t)bins * sizeof(BinTab) + 64;
             if ((rc5 = set_dyn_smem(kern, smem5, "k_roi_align_win")) != 0) return;
-            const int tiles = cdiv(c.C, ct);
-            a.tiles = (knobs().roi_order == 1 && R * tiles < (1ll << 31)) ? tiles : 0;
-            const long long Rw = a.sel_m > 1 ? R - (R + a.sel_m - 1) / a.sel_m : R;       // RoIs of this kernel
-            dim3 grid(a.tiles ? (unsigned)(Rw * tiles) : (unsigned)Rw, a.tiles ? 1u : (unsigned)tiles);
-            if (Rw > 0) kern<<<grid, nt, smem5, st>>>(a, out);
+            kern<<<dim3((unsigned)R, (unsigned)cdiv(c.C, ct)), nt, smem5, st>>>(a, out);
         };
         // 128 threads x 4 channels = 128 channels per CTA, 6 CTAs/SM: fastest of the measured
         // (threads, channels/CTA, CTAs/SM, channels/thread) points -- (256,256,2,4) 200 us,
         // (256,256,3,4) 169, (128,128,4,4) 169, (128,128,6,4) 159, (128,128,7,4) 186 (spills),
         // (256,128,5,2) 175, (128,64,8,2) 186, (128,64,10,2) 173 (config 2, 4096 RoIs)
-        // B2D_ROI_X2=0 (dev knob): scalar adds (157 vs 151 us, config 2)
-        if (c.layout == 1 && knobs().roi_x2 != 0) launch5(k_roi_align_win<float, 128, 128, 6, 4, 1>, 128, 128);
-        else if (c.layout == 1) launch5(k_roi_align_win<float, 128, 128, 6, 4>, 128, 128);
-        else launch5(k_roi_align_win<__nv_bfloat16, 128, 128, 6, 4>, 128, 128);
+        if (c.layout == 1) launch5(k_roi_align_win<float, 128, 128, 6>, 128, 128);
+        else launch5(k_roi_align_win<__nv_bfloat16, 128, 128, 6>, 128, 128);
         if (rc5) return rc5;
-        if (hetero) cudaStreamWaitEvent(st, ev_join, 0);
     } else if (fast) {
         const size_t smem = (size_t)bins * (kCTile + 4) * 4;
         if (c.layout == 1) {

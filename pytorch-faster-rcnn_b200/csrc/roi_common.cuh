@@ -1,6 +1,7 @@
 // roi_common.cuh -- RoI argument block, RoI fetch, FPN level map and the bilinear sample geometry
-// shared by the RoIAlign kernels (roi_align.cu, roi_align_tma.cu).  torchvision RoIAlign
-// semantics (pre_calc_for_bilinear_interpolate); lib/region.py:243-306.
+// shared by the RoIAlign forward (roi_align.cu), its backward (roi_bwd_common.cuh) and the sparse
+// feature fetch (roi_fetch.cu).  torchvision RoIAlign semantics (pre_calc_for_bilinear_interpolate);
+// lib/region.py:243-306.
 #pragma once
 #include "common.cuh"
 
@@ -14,10 +15,6 @@ struct RoiArgs {
     long long R;
     long long batched_ld;          // > 0: rois are image-major [B][4][ld], counts per image
     const int* counts;
-    int tiles;                     // window kernel: > 0 = 1-D grid, channel tiles of a RoI adjacent (bid = r * tiles + tile)
-    int pf_dist;                   // window kernel: L2-prefetch the RoI pf_dist CTAs ahead (0 = off)
-    int bulk_store;                // window kernel: result tile leaves as one cp.async.bulk store
-    int sel_m;                     // > 1: heterogeneous split -- the tensor-map kernel takes the RoIs r % sel_m == 0, the window kernel the others
 };
 
 // slot r -> (image, coordinates); false if the slot is past the image's count
@@ -75,14 +72,5 @@ __device__ __forceinline__ RoiGeom roi_geom(float x1, float y1, float x2, float 
     g.gx = sr > 0 ? sr : (int)ceilf(rw / (float)PW);
     return g;
 }
-
-// TMA-ring kernel (roi_align_tma.cu): returns B2D_OK if it handled the launch, 1 if the config is
-// not eligible (the caller then uses the L1-path kernels of roi_align.cu).
-struct RoiArgs;
-int roi_align_tma_try(const RoiArgs& a, float* out, cudaStream_t st);
-// tensor-map TMA band kernel (roi_align_tband.cu): same contract; B = images in the feature tensors (upper bound)
-int roi_align_tband_try(const RoiArgs& a, float* out, int B, cudaStream_t st, int persistent_ctas = 0);
-// side stream + fork / join events for the heterogeneous launch (created once per device); false if unavailable
-bool roi_hetero_streams(cudaStream_t* side, cudaEvent_t* fork, cudaEvent_t* join);
 
 }  // namespace b2d

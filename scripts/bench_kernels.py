@@ -30,39 +30,7 @@ def main():
     out = hp.step(cls, reg, feats, gt, gcount, gl, img_hw)
     torch.cuda.synchronize()
     bt = out["rcnn"]
-    which = sys.argv[1:] or ["roi"]
-    if "roi" in which:
-        ref = None
-        # VARIANTS: comma list of <order><x2>[:pf], e.g. "00,10,01,11" -> B2D_ROI_ORDER, B2D_ROI_X2 dev knobs
-        for v in os.environ.get("VARIANTS", "00,10,01,11").split(","):
-            if ":" in v:
-                v, pf = v.split(":"); os.environ["B2D_ROI_PF"] = pf
-            os.environ["B2D_ROI_ORDER"] = v[0]; os.environ["B2D_ROI_X2"] = v[1] if len(v) > 1 else "0"
-            hp.roi_align.out.zero_()
-            us = timeit(lambda: hp.roi_align(feats, bt.tar_box, bt.n_chosen))
-            o = hp.roi_align.out.clone()
-            if ref is None: ref = o
-            print("roi_align variant %s pf=%s: %.1f us  bitexact_vs_first=%s" % (v, os.environ.get("B2D_ROI_PF"), us, bool(torch.equal(o, ref))))
-    if "tma" in which:
-        ref = None
-        rb = bt.tar_box.cpu().numpy(); nb = bt.n_chosen.cpu().numpy()
-        wide = 0; tot = 0
-        for b in range(B):
-            r = rb[b][:, :nb[b]]
-            s_ = np.sqrt((r[2] - r[0] + 1) * (r[3] - r[1] + 1))
-            lv = np.clip(np.floor(np.log2(s_ / 56 + 1e-6)), 0, 3)
-            wc = (r[2] - r[0]) / (4 * 2 ** lv)
-            wide += int((wc > 29).sum()); tot += r.shape[1]
-        print("RoIs wider than 29 cells: %d of %d" % (wide, tot), flush=True)
-        for v in ("0", "1", "1:-7"):
-            if ":" in v:
-                v, d = v.split(":"); os.environ["B2D_ROI_TMA_DEV"] = d
-            os.environ["B2D_ROI_TMA"] = v
-            hp.roi_align.out.zero_()
-            us = timeit(lambda: hp.roi_align(feats, bt.tar_box, bt.n_chosen))
-            o = hp.roi_align.out.clone()
-            if ref is None: ref = o
-            print("roi_align B2D_ROI_TMA=%s: %.1f us  bitexact_vs_first=%s" % (v, us, bool(torch.equal(o, ref))), flush=True)
+    which = sys.argv[1:] or ["stages"]
     if "roil2" in which:
         # same RoIs, but every image reads the features of image 0 -> after warm-up all taps are L2 hits
         import ctypes
@@ -72,13 +40,9 @@ def main():
         R = rois.shape[1]
         outb = torch.empty((R, 256, 7, 7), device=dev)
         cfg = hp.roi_align.cfg
-        for v in os.environ.get("VARIANTS", "4,5").split(","):
-            if ":" in v:
-                v, pf = v.split(":"); os.environ["B2D_ROI_PF"] = pf
-            os.environ["B2D_ROI_VARIANT"] = v
-            fn = lambda: _C.call("b2d_roi_align_fwd", _C.ptr(outb), fused._ptrs(feats), _C.ptr(rois), R, None, None, R,
-                                 ctypes.byref(cfg), _C.stream())
-            print("L2-resident roi_align variant %s: %.1f us for %d rois" % (v, timeit(fn), R))
+        fn = lambda: _C.call("b2d_roi_align_fwd", _C.ptr(outb), fused._ptrs(feats), _C.ptr(rois), R, None, None, R,
+                             ctypes.byref(cfg), _C.stream())
+        print("L2-resident roi_align: %.1f us for %d rois" % (timeit(fn), R))
     if "stages" in which:
         print("proposals %.1f us" % timeit(lambda: hp.proposals(cls, reg, img_hw)))
         print("rpn_targets %.1f us" % timeit(lambda: hp.rpn_targets(gt, gcount, None, img_hw=img_hw)))

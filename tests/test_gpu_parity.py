@@ -447,9 +447,9 @@ def test_roi_align_bf16_nhwc_close():
     np.testing.assert_allclose(N(out), ref, rtol=1e-5, atol=1e-6)      # same bf16-rounded inputs, fp32 math
 
 
-def _ring_case(seed, C, K, B=2):
-    """RoIs that exercise every branch of the TMA-ring kernel (csrc/roi_align_tma.cu): level-mapped sizes,
-    RoIs wider than the ring holds (generic in-kernel path), sub-cell RoIs, RoIs on / beyond the borders."""
+def _edge_roi_case(seed, C, K, B=2):
+    """Level-mapped RoIs plus the edge cases of the RoIAlign kernels: RoIs far wider than a level's window (sample
+    spacing above two cells), sub-cell RoIs, RoIs on / beyond the image borders."""
     rng = np.random.default_rng(seed)
     grids = [(48, 80), (24, 40), (12, 20), (6, 10)]                       # 192 x 320 image, strides 4..32
     feats = [rng.standard_normal((B, C) + gsz).astype(np.float32) for gsz in grids]
@@ -463,39 +463,25 @@ def _ring_case(seed, C, K, B=2):
     return grids, feats, rois, img
 
 
-@pytest.mark.parametrize("mode", ["1", "2", "3"])
-@pytest.mark.parametrize("C,K", [(256, 700), (128, 333)])
-def test_roi_align_tma_ring_bit_exact_vs_oracle(C, K, mode, setknob):
-    """The two opt-in TMA forms of K5 -- 1: bulk-copy row ring (roi_align_tma.cu), 2: tensor-map band kernel
-    (roi_align_tband.cu, cp.async.bulk.tensor.4d / UTMALDG; RoIs wider than 16 cells take its in-kernel window path),
-    3: heterogeneous launch (a persistent band CTA per SM takes every m-th RoI beside the window kernel)."""
-    setknob(B2D_ROI_TMA=mode)                                             # opt-in kernels
-    grids, feats, rois, img = _ring_case(11, C, K)
+@pytest.mark.parametrize("dtype,C,K,seed", [("fp32", 256, 700, 11), ("fp32", 128, 333, 11), ("bf16", 256, 500, 12)])
+def test_roi_align_window_edge_rois_vs_oracle(dtype, C, K, seed):
+    """K5's window kernel (k_roi_align_win) on NHWC features at one and two full 128-channel tiles, fp32 (packed adds)
+    and bf16 (scalar adds), on the edge-case RoIs: bit-identical to the oracle on the same (bf16-rounded) inputs."""
+    grids, feats, rois, img = _edge_roi_case(seed, C, K)
     fs = [T(f).contiguous(memory_format=torch.channels_last) for f in feats]
+    if dtype == "bf16":
+        fs = [f.to(torch.bfloat16) for f in fs]
+        feats = [N(f.float()) for f in fs]                                  # the bf16-rounded values, NCHW
     out = N(bregion.roi_align_levels(fs, T(rois), T(img), [1 / 4, 1 / 8, 1 / 16, 1 / 32]))
     for b in range(feats[0].shape[0]):
         m = img == b
         ref = oracle.roi_extract([f[b] for f in feats], np.ascontiguousarray(rois[:, m]))
-        assert np.array_equal(bits(out[m]), bits(ref)), "ring kernel must be bit-identical to the oracle"
-    # single level, one image, aligned=True (bin sizes may be ~0 / negative -> generic path), 5x3 bins
+        assert np.array_equal(bits(out[m]), bits(ref)), "window kernel must be bit-identical to the oracle"
+    # single level, one image, aligned=True (bin sizes may be ~0 / negative), 5x3 bins
     r1 = np.ascontiguousarray(rois[:, img == 0])
     o1 = N(bregion.roi_align_levels([fs[1][:1]], T(r1), None, [1 / 8], out_size=(5, 3), aligned=True))
     ref1 = oracle.roi_align(feats[1][0], r1, 1 / 8, (5, 3), 2, True)
     assert np.array_equal(bits(o1), bits(ref1))
-
-
-def test_roi_align_tma_ring_bf16_and_l1_path_agree(setknob):
-    grids, feats, rois, img = _ring_case(12, 256, 500)
-    fs = [T(f).to(torch.bfloat16).contiguous(memory_format=torch.channels_last) for f in feats]
-    setknob(B2D_ROI_TMA=1)
-    out = N(bregion.roi_align_levels(fs, T(rois), T(img), [1 / 4, 1 / 8, 1 / 16, 1 / 32]))
-    setknob(B2D_ROI_TMA=0)                                                # L1-path kernel (k_roi_align_win)
-    out_l1 = N(bregion.roi_align_levels(fs, T(rois), T(img), [1 / 4, 1 / 8, 1 / 16, 1 / 32]))
-    assert np.array_equal(bits(out), bits(out_l1))
-    for b in range(2):
-        m = img == b
-        ref = oracle.roi_extract([N(f[b].float()) for f in fs], np.ascontiguousarray(rois[:, m]))
-        assert np.array_equal(bits(out[m]), bits(ref))
 
 
 @pytest.mark.parametrize("form", ["2", "1"])
@@ -506,7 +492,7 @@ def test_roi_align_backward_tile_kernel_vs_oracle_and_generic(C, K, form, setkno
     inside a cell differs from torchvision's), against the generic torchvision-ordered kernel, and run-to-run
     bit-identical; RoIs incl. borders / outside / sub-cell / wider than the map."""
     setknob(B2D_ROI_BWD_TILE=form)
-    grids, feats, rois, img = _ring_case(13, C, K)
+    grids, feats, rois, img = _edge_roi_case(13, C, K)
     fs = [T(f).contiguous(memory_format=torch.channels_last).requires_grad_(True) for f in feats]
     rng = np.random.default_rng(5)
     go = rng.standard_normal((K, C, 7, 7)).astype(np.float32)
@@ -628,7 +614,7 @@ def test_roi_align_backward_full_size_properties(setknob):
 def test_roi_align_reference_layout_takes_fast_kernels():
     """fp32 NCHW features (the reference's FPN output layout, lib/necks.py) are transposed once and go through the same
     K5 / K6 kernels as channels_last inputs: identical forward bits, identical gradients (returned for the NCHW input)."""
-    grids, feats, rois, img = _ring_case(14, 64, 200)
+    grids, feats, rois, img = _edge_roi_case(14, 64, 200)
     scales = [1 / 4, 1 / 8, 1 / 16, 1 / 32]
     go = np.random.default_rng(2).standard_normal((200, 64, 7, 7)).astype(np.float32)
     outs, grads = [], []
@@ -918,7 +904,7 @@ def test_mark_and_fetch_touched_cells_cover_every_tap(setknob):
     exactly the marked cells are copied from pinned channels_last host maps; RoIAlign on a NaN-poisoned device pyramid
     that received only those cells is bit-identical to RoIAlign on the whole pyramid."""
     import ctypes
-    grids, feats, rois, img = _ring_case(21, 64, 600)
+    grids, feats, rois, img = _edge_roi_case(21, 64, 600)
     B, strides = feats[0].shape[0], [4, 8, 16, 32]
     order = np.argsort(img, kind="stable")
     rois, img = rois[:, order], img[order]
