@@ -144,6 +144,15 @@ B2D_API int b2d_roi_targets_fused(int64_t* labels, float* max_iou, long long out
 B2D_API int b2d_gather_head_outputs(float* tar_cls, float* tar_reg, const void* const* cls_ptrs_host,
                             const void* const* reg_ptrs_host, const b2d_pyramid* pyr_host, int cls_channels,
                             const int* chosen, const int* n_chosen, int max_num, int B, void* stream);
+/* its adjoint (the backward of the torch index in lib/anchor.py:49-56): grad_tar_cls [B][C][max_num] and grad_tar_reg
+ * [B][4][max_num] -> dense head-map gradients dcls_ptrs_host[l] -> [B, A*C, H, W], dreg_ptrs_host[l] -> [B, 4A, H, W]
+ * (the element of channel c at level index li is at (b * C + c) * A*H*W + li, as the gather reads it).  Every element is
+ * written once, in one launch: the upstream value at a sampled anchor, zero elsewhere; no memset, no atomics,
+ * deterministic.  Precondition: chosen[b][0 .. n_chosen[b]) is ascending and duplicate-free (what b2d_sample_labels and
+ * b2d_roi_targets_fused emit); rows at or past n_chosen[b] are not read. */
+B2D_API int b2d_scatter_head_grads(void* const* dcls_ptrs_host, void* const* dreg_ptrs_host, const float* grad_tar_cls,
+                                   const float* grad_tar_reg, const b2d_pyramid* pyr_host, int cls_channels,
+                                   const int* chosen, const int* n_chosen, int max_num, int B, void* stream);
 
 /* ---- K3: fused RPN proposal selection, all images and levels per launch
  * (RPNHead.predict_single_image, lib/heads/rpn_head.py:68-120; AnchorHead
@@ -375,6 +384,13 @@ B2D_API size_t b2d_roi_align_bwd_workspace_bytes(long long R, int B, const b2d_r
 B2D_API int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois,
                       long long roi_ld, const int* roi_img, const int* levels, long long R, int B,
                       const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes, void* stream);
+/* backward of b2d_roi_align_fwd_batched: rois [B][4][ld] with counts int32[B], grad_out [B*ld, C, PH, PW] as the forward
+ * wrote out.  Slots at or past counts[b] contribute nothing: neither their grad_out rows nor their boxes are read.  Same
+ * kernels, same results as b2d_roi_align_bwd on the compacted RoI list (image-major, roi_img = image). */
+B2D_API size_t b2d_roi_align_bwd_batched_workspace_bytes(long long ld, int B, const b2d_roi_cfg* cfg_host);
+B2D_API int b2d_roi_align_bwd_batched(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois,
+                                      long long ld, const int* counts, int B, const b2d_roi_cfg* cfg_host, void* workspace,
+                                      size_t ws_bytes, void* stream);
 /* fp32 NCHW [B,C,H,W] -> NHWC [B,H,W,C]: reference-layout FPN features (lib/necks.py:69-90)
  * to the channels-last layout the vectorised RoIAlign kernels read. */
 B2D_API int b2d_nchw_to_nhwc(float* dst, const float* src, int B, int C, int H, int W, void* stream);

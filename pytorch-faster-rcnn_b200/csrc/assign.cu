@@ -812,6 +812,73 @@ __global__ void __launch_bounds__(128) k_gather_head(GatherArgs p, b2d_pyramid p
         tar_reg[((long long)b * 4 + c) * p.max_num + t] = live ? p.reg[l][((long long)b * 4 + c) * n + li] : 0.0f;
 }
 
+// ---- adjoint of k_gather_head: the dense head-map gradients from the gradients at the sampled anchors ----------
+// A thread owns kScatterRun consecutive elements of one plane (image b, level l, channel: cls_ch class planes, then 4
+// regression planes) and writes each of them exactly once: the upstream value where the anchor was sampled, zero
+// elsewhere -- no memset, no atomics.  Precondition (DESIGN §8, every sampler of this library): chosen[b][0 .. n_chosen[b])
+// is ascending and free of duplicates; its first sample at or after the run is found by binary search.
+constexpr int kScatterRun = 16;
+
+struct ScatterArgs {
+    float* cls[kMaxLevels]; float* reg[kMaxLevels];
+    const float* g_cls; const float* g_reg;
+    const int* chosen; const int* n_chosen; int max_num, cls_ch;
+    long long run_off[kMaxLevels + 1];     // first run of each level within an image
+};
+
+__global__ void __launch_bounds__(256) k_scatter_head(ScatterArgs p, b2d_pyramid pyr) {
+    const int b = blockIdx.y;
+    long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= p.run_off[pyr.num_levels]) return;
+    int l = 0;
+    for (int q = 1; q < pyr.num_levels; ++q) if (t >= p.run_off[q]) l = q;
+    t -= p.run_off[l];
+    const long long n = (long long)pyr.lv[l].A * pyr.lv[l].H * pyr.lv[l].W;
+    const long long runs = (n + kScatterRun - 1) / kScatterRun;
+    const int plane = (int)(t / runs);
+    const long long li0 = (t - plane * runs) * kScatterRun;
+    const int len = (int)min((long long)kScatterRun, n - li0);
+    float* dst;
+    const float* g;
+    if (plane < p.cls_ch) {
+        dst = p.cls[l] + ((long long)b * p.cls_ch + plane) * n + li0;
+        g = p.g_cls + ((long long)b * p.cls_ch + plane) * p.max_num;
+    } else {
+        dst = p.reg[l] + ((long long)b * 4 + plane - p.cls_ch) * n + li0;
+        g = p.g_reg + ((long long)b * 4 + plane - p.cls_ch) * p.max_num;
+    }
+    const int* ch = p.chosen + (long long)b * p.max_num;
+    const int cnt = min(p.n_chosen[b], p.max_num);
+    const long long base = pyr.lv[l].offset + li0;          // flat anchor index of the run's first element
+    int lo = 0, hi = cnt;                                   // first sample >= base
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if ((long long)__ldg(ch + mid) < base) lo = mid + 1; else hi = mid;
+    }
+    int j = lo;
+    int nxt = j < cnt ? (int)min((long long)__ldg(ch + j) - base, (long long)kScatterRun) : kScatterRun;
+    float v[kScatterRun];
+#pragma unroll
+    for (int e = 0; e < kScatterRun; ++e) {
+        float x = 0.0f;
+        if (e == nxt) {
+            x = __ldg(g + j);
+            ++j;
+            nxt = j < cnt ? (int)min((long long)__ldg(ch + j) - base, (long long)kScatterRun) : kScatterRun;
+        }
+        v[e] = x;
+    }
+    if (len == kScatterRun && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+#pragma unroll
+        for (int e = 0; e < kScatterRun; e += 4)
+            *reinterpret_cast<float4*>(dst + e) = make_float4(v[e], v[e + 1], v[e + 2], v[e + 3]);
+    } else {
+#pragma unroll
+        for (int e = 0; e < kScatterRun; ++e)
+            if (e < len) dst[e] = v[e];
+    }
+}
+
 // ---- bbox_target of one image in ONE launch (lib/bbox.py:6-82) -----------------------------------
 // assignment (assign_small_body) -> device-RNG sampler (the specification of k_sample,
 // oracle/sampler_spec.py: identical `chosen`) -> gather + encode (k_encode_targets), one CTA per
@@ -941,6 +1008,32 @@ int b2d_gather_head_outputs(float* tar_cls, float* tar_reg, const void* const* c
     dim3 grid(cdiv(max_num, 128), B);
     k_gather_head<<<grid, 128, 0, (cudaStream_t)stream>>>(p, *pyr_host, tar_cls, tar_reg);
     return check_launch("gather_head_outputs");
+}
+
+int b2d_scatter_head_grads(void* const* dcls_ptrs_host, void* const* dreg_ptrs_host, const float* grad_tar_cls,
+                           const float* grad_tar_reg, const b2d_pyramid* pyr_host, int cls_channels, const int* chosen,
+                           const int* n_chosen, int max_num, int B, void* stream) {
+    B2D_REQUIRE(dcls_ptrs_host && dreg_ptrs_host && grad_tar_cls && grad_tar_reg && pyr_host && chosen && n_chosen,
+                "scatter_head_grads: null pointer");
+    B2D_REQUIRE(B >= 1 && max_num >= 1 && cls_channels >= 1 && pyr_host->num_levels >= 1 &&
+                pyr_host->num_levels <= kMaxLevels, "scatter_head_grads: bad sizes");
+    ScatterArgs p;
+    memset(&p, 0, sizeof(p));
+    long long run = 0;
+    for (int l = 0; l < pyr_host->num_levels; ++l) {
+        B2D_REQUIRE(dcls_ptrs_host[l] && dreg_ptrs_host[l], "scatter_head_grads: null level pointer");
+        p.cls[l] = (float*)dcls_ptrs_host[l]; p.reg[l] = (float*)dreg_ptrs_host[l];
+        const b2d_level& v = pyr_host->lv[l];
+        p.run_off[l] = run;
+        run += (long long)(cls_channels + 4) * cdiv((long long)v.A * v.H * v.W, kScatterRun);
+    }
+    p.run_off[pyr_host->num_levels] = run;
+    p.g_cls = grad_tar_cls; p.g_reg = grad_tar_reg;
+    p.chosen = chosen; p.n_chosen = n_chosen; p.max_num = max_num; p.cls_ch = cls_channels;
+    if (run == 0) return B2D_OK;
+    dim3 grid((unsigned)cdiv(run, 256), (unsigned)B);
+    k_scatter_head<<<grid, 256, 0, (cudaStream_t)stream>>>(p, *pyr_host);
+    return check_launch("scatter_head_grads");
 }
 
 int b2d_encode_targets(float* tar_box, float* tar_gt, float* tar_param, int64_t* tar_label, int64_t* tar_is_gt,

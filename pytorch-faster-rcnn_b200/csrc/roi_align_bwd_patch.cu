@@ -56,6 +56,15 @@ struct PatchArgs {
     int tile_off[kMaxLevels + 1], tiles_x[kMaxLevels];
 };
 
+// scratch budget: 512 patch cells per RoI on average (config 2: 177; RoIs spread over a level's octave: ~520), at least
+// 16 K cells, at most 6 M cells
+__host__ __device__ __forceinline__ long long patch_budget_cells(long long R) {
+    long long n = R * 512;
+    if (n < 16384) n = 16384;
+    if (n > 6000000) n = 6000000;
+    return n;
+}
+
 __device__ __forceinline__ long long patch_area(const BwdMeta& m) {
     return (m.y1 >= m.y0 && m.x1 >= m.x0) ? (long long)(m.y1 - m.y0 + 1) * (m.x1 - m.x0 + 1) : 0;
 }
@@ -90,10 +99,11 @@ __global__ void __launch_bounds__(1024) k_bwd_bucket_scan(const BwdMeta* __restr
         if (threadIdx.x == 0) bcount[blockIdx.x] = (int)s_base;
         return;
     }
+    int live = 0;                                       // records of RoIs (batched form: slots below their image's count)
     for (long long r0 = 0; r0 < R; r0 += 1024) {
         const long long r = r0 + threadIdx.x;
         long long a = 0;
-        if (r < R) a = patch_area(meta[r]);
+        if (r < R) { const BwdMeta m = meta[r]; a = patch_area(m); live += m.img >= 0; }
         long long inc = a;
         for (int d = 1; d < 32; d <<= 1) {
             const long long t = __shfl_up_sync(0xffffffffu, inc, d);
@@ -108,9 +118,16 @@ __global__ void __launch_bounds__(1024) k_bwd_bucket_scan(const BwdMeta* __restr
         if (threadIdx.x == 0) { long long t = 0; for (int w = 0; w < 32; ++w) t += s_w[w]; s_base += t; }
         __syncthreads();
     }
+    // the budget of the RoIs actually present, so that the batched entry (empty slots included in R) takes the patch or
+    // the tile form exactly when the unbatched call on the compacted list does
+    live = (int)__reduce_add_sync(0xffffffffu, (unsigned)live);
+    if (lane == 0) s_w[warp] = live;
+    __syncthreads();
     if (threadIdx.x == 0) {
+        long long n = 0;
+        for (int w = 0; w < 32; ++w) n += s_w[w];
         poff[R] = s_base;
-        flags[0] = s_base > cap_cells ? 1 : 0;
+        flags[0] = s_base > min(cap_cells, patch_budget_cells(n)) ? 1 : 0;
     }
 }
 
@@ -430,15 +447,6 @@ long long bitmap_words(const b2d_roi_cfg& c, int B, long long* word0) {
 
 }  // namespace
 
-// scratch budget: 512 patch cells per RoI on average (config 2: 177; RoIs spread over a level's octave: ~520), at least
-// 16 K cells, at most 6 M cells
-static long long patch_budget_cells(long long R) {
-    long long n = R * 512;
-    if (n < 16384) n = 16384;
-    if (n > 6000000) n = 6000000;
-    return n;
-}
-
 size_t roi_align_bwd_patch_workspace(long long R, int B, const b2d_roi_cfg& c) {
     const size_t r = (size_t)(R > 0 ? R : 1);
     const size_t words = (size_t)bitmap_words(c, B, nullptr);
@@ -448,7 +456,8 @@ size_t roi_align_bwd_patch_workspace(long long R, int B, const b2d_roi_cfg& c) {
 
 // returns 1 if the configuration is not eligible (the caller then uses the tile / generic kernels)
 int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                            const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg& c, void* workspace,
+                            const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace,
                             cudaStream_t st) {
     if (c.layout != 1 || c.sampling_ratio != 2 || c.PH > kMaxTerms || c.PW > kMaxTerms || c.PH * c.PW > kMaxBinsT) return 1;
     if (c.C % kPCg != 0 || R < 1) return 1;
@@ -470,6 +479,7 @@ int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_
     MetaArgs ma;
     memset(&ma, 0, sizeof(ma));
     ma.cfg = c; ma.rois = rois; ma.roi_ld = roi_ld; ma.roi_img = roi_img; ma.levels = levels; ma.R = R;
+    ma.batched_ld = batched_ld; ma.counts = counts;
     a.cap_cells = patch_budget_cells(R);
     if (cudaMemsetAsync(anyb, 0, 2 * align256((size_t)words * 4 + 16), st) != cudaSuccess) return check_launch("roi_align_bwd(patch memset)");
     int run = 0;

@@ -229,7 +229,8 @@ size_t roi_align_bwd_tile_workspace(long long R, int B, int L) {
 
 // returns 1 if the configuration is not eligible (the caller then uses the generic kernel)
 int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                           const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg& c, void* workspace,
+                           const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace,
                            cudaStream_t st) {
     if (c.layout != 1 || c.sampling_ratio != 2 || 2 * c.PH > kMaxS || 2 * c.PW > kMaxS || c.PH * c.PW > kMaxBinsT) return 1;
     if (c.C % kCg != 0 || R < 1) return 1;
@@ -242,6 +243,7 @@ int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_o
     MetaArgs ma;
     memset(&ma, 0, sizeof(ma));
     ma.cfg = c; ma.rois = rois; ma.roi_ld = roi_ld; ma.roi_img = roi_img; ma.levels = levels; ma.R = R;
+    ma.batched_ld = batched_ld; ma.counts = counts;
     k_bwd_meta<<<cdiv(R, 256), 256, 0, st>>>(ma, meta);
     k_bwd_bucket<<<B * c.num_levels, 256, 0, st>>>(meta, R, c.num_levels, bucket, bcount);
     return roi_align_bwd_tile_launch(grad_feat_ptrs_host, grad_out, R, B, c, meta, bucket, bcount, nullptr, st);

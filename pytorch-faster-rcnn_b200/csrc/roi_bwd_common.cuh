@@ -17,13 +17,30 @@ struct __align__(16) BwdMeta {
 struct MetaArgs {
     b2d_roi_cfg cfg;
     const float* rois; long long roi_ld; const int* roi_img; const int* levels; long long R;
+    long long batched_ld;          // > 0: rois are image-major [B][4][ld], slot r = (r / ld, r % ld), counts per image
+    const int* counts;
 };
 
+// The record of slot r.  A batched slot at or past its image's count gets img = -1 and an empty tap box: no bucket lists
+// it and it has no patch, so neither its box nor its grad_out row is ever read.
 __device__ __forceinline__ BwdMeta bwd_meta_of(const MetaArgs& a, long long r) {
     const b2d_roi_cfg& c = a.cfg;
-    const float x1 = a.rois[r], y1 = a.rois[a.roi_ld + r], x2 = a.rois[2 * a.roi_ld + r], y2 = a.rois[3 * a.roi_ld + r];
     BwdMeta m;
-    m.img = a.roi_img ? a.roi_img[r] : 0;
+    const float* p = a.rois + r;
+    if (a.batched_ld > 0) {
+        const int img = (int)(r / a.batched_ld);
+        if (r - (long long)img * a.batched_ld >= a.counts[img]) {
+            m.img = -1; m.lvl = 0; m.y0 = m.x0 = 0; m.y1 = m.x1 = -1;
+            m.sx = m.sy = m.bw = m.bh = 0.0f; m._p0 = m._p1 = 0;
+            return m;
+        }
+        p += (long long)img * 3 * a.batched_ld;
+        m.img = img;
+    } else {
+        m.img = a.roi_img ? a.roi_img[r] : 0;
+    }
+    const long long ld = a.batched_ld > 0 ? a.batched_ld : a.roi_ld;
+    const float x1 = p[0], y1 = p[ld], x2 = p[2 * ld], y2 = p[3 * ld];
     m.lvl = a.levels ? a.levels[r] : (c.num_levels > 1 ? roi_level(x1, y1, x2, y2, c.finest_scale, c.num_levels) : 0);
     const int H = c.H[m.lvl], W = c.W[m.lvl];
     const RoiGeom g = roi_geom(x1, y1, x2, y2, c.spatial_scale[m.lvl], c.PH, c.PW, 2, c.aligned);

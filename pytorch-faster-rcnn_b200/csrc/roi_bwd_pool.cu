@@ -13,7 +13,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "common.cuh"
+#include "roi_common.cuh"
 
 namespace b2d {
 
@@ -22,10 +22,12 @@ size_t roi_align_bwd_tile_workspace(long long R, int B, int L);
 // patch form (roi_align_bwd_patch.cu): its workspace begins with the tile form's tables, so either can use it
 size_t roi_align_bwd_patch_workspace(long long R, int B, const b2d_roi_cfg& c);
 int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                            const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg& c, void* workspace,
+                            const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace,
                             cudaStream_t st);
 int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                           const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg& c, void* workspace,
+                           const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace,
                            cudaStream_t st);
 
 struct AxisTapB { int lo, hi; float l, h; int valid; };
@@ -51,9 +53,26 @@ struct BwdArgs {
     void* grad[kMaxLevels];
     const float* gout; const float* rois; long long roi_ld;
     const int* roi_img; const int* levels; long long R; int B;
+    long long bld;                          // > 0: rois image-major [B][4][bld] (roi_ld == bld); levels -1 = empty slot
     int tile_off[kMaxLevels + 1];           // CTA-tile prefix per level (per image)
     int tiles_x[kMaxLevels];
 };
+
+// x1 of slot r; coordinate k at [k * roi_ld]
+__device__ __forceinline__ const float* bwd_roi_ptr(const BwdArgs& a, long long r) {
+    return a.rois + r + (a.bld > 0 ? (r / a.bld) * 3 * a.bld : 0);
+}
+
+// level of every slot of an image-major [B][4][ld] RoI list, -1 for the slots at or past counts[b] (their boxes unread)
+__global__ void __launch_bounds__(256) k_bwd_levels_batched(int* __restrict__ lv, const float* __restrict__ rois, long long ld,
+                                                            const int* __restrict__ counts, long long R, float finest, int L) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= R) return;
+    const int img = (int)(r / ld);
+    if (r - (long long)img * ld >= counts[img]) { lv[r] = -1; return; }
+    const float* p = rois + r + (long long)img * 3 * ld;
+    lv[r] = roi_level(p[0], p[ld], p[2 * ld], p[3 * ld], finest, L);
+}
 
 __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
     __shared__ int s_list[kSub];
@@ -88,10 +107,11 @@ __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
         while (r0 < a.R && s_n < kSub) {
             const long long r = r0 + threadIdx.x;
             bool hit = false;
-            if (r < a.R && (a.roi_img ? a.roi_img[r] : 0) == img && a.levels[r] == lvl) {
+            if (r < a.R && a.levels[r] == lvl && (a.bld > 0 ? (int)(r / a.bld) : (a.roi_img ? a.roi_img[r] : 0)) == img) {
+                const float* rp = bwd_roi_ptr(a, r);
                 const float off = c.aligned ? 0.5f : 0.0f;
-                const float sx = a.rois[r] * scale - off, sy = a.rois[a.roi_ld + r] * scale - off;
-                const float ex = a.rois[2 * a.roi_ld + r] * scale - off, ey = a.rois[3 * a.roi_ld + r] * scale - off;
+                const float sx = rp[0] * scale - off, sy = rp[a.roi_ld] * scale - off;
+                const float ex = rp[2 * a.roi_ld] * scale - off, ey = rp[3 * a.roi_ld] * scale - off;
                 // conservative extent of the taps: samples lie in [s, max(e, s+1)], taps reach one cell
                 // further, and everything beyond the map is clamped onto the last row / column
                 float ylo = floorf(fminf(sy, ey)) - 1.0f, yhi = ceilf(fmaxf(ey, sy + 1.0f)) + 1.0f;
@@ -125,10 +145,10 @@ __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
         // ---- axis taps of the batch
         for (int q = threadIdx.x; q < nb * (ny + nx); q += blockDim.x) {
             const int e = q / (ny + nx), k = q - e * (ny + nx);
-            const long long r = s_list[e];
+            const float* rp = bwd_roi_ptr(a, s_list[e]);
             const float off = c.aligned ? 0.5f : 0.0f;
-            const float sx = a.rois[r] * scale - off, sy = a.rois[a.roi_ld + r] * scale - off;
-            const float ex = a.rois[2 * a.roi_ld + r] * scale - off, ey = a.rois[3 * a.roi_ld + r] * scale - off;
+            const float sx = rp[0] * scale - off, sy = rp[a.roi_ld] * scale - off;
+            const float ex = rp[2 * a.roi_ld] * scale - off, ey = rp[3 * a.roi_ld] * scale - off;
             float rw = ex - sx, rh = ey - sy;
             if (!c.aligned) { rw = fmaxf(rw, 1.0f); rh = fmaxf(rh, 1.0f); }
             const float bh = rh / (float)c.PH, bw = rw / (float)c.PW;
@@ -288,9 +308,11 @@ size_t b2d_roi_align_bwd_workspace_bytes(long long R, int B, const b2d_roi_cfg* 
     return bwd_levels_bytes(R) + n;                                                   // level ids in front
 }
 
-int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                      const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg* cfg_host,
-                      void* workspace, size_t ws_bytes, void* stream) {
+// the two entry points below: an explicit RoI list with roi_img / levels, or (batched_ld > 0) the image-major
+// [B][4][batched_ld] slots of b2d_roi_align_fwd_batched with per-image counts
+static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
+                              const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+                              const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes, void* stream) {
     B2D_REQUIRE(grad_feat_ptrs_host && grad_out && rois && cfg_host && R >= 0 && B >= 1, "roi_align_bwd: bad args");
     const b2d_roi_cfg& c = *cfg_host;
     B2D_REQUIRE(c.num_levels >= 1 && c.num_levels <= B2D_MAX_LEVELS, "roi_align_bwd: bad cfg");
@@ -302,19 +324,22 @@ int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, c
     {   // NHWC fp32 gradients with 2x2 samples: patch form (B2D_ROI_BWD_TILE=2, default), tile-gather form (=1);
         // B2D_ROI_BWD_TILE=0 forces the generic, torchvision-bit-identical kernel below
         if (knobs().roi_bwd_tile >= 2) {                  // patch form ("sorted scatter", roi_align_bwd_patch.cu): default
-            const int rc = roi_align_bwd_patch_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, R, B, c,
-                                                   (char*)workspace + bwd_levels_bytes(R), st);
+            const int rc = roi_align_bwd_patch_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, batched_ld, counts,
+                                                   R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
             if (rc != 1) return rc;
         }
         if (knobs().roi_bwd_tile != 0) {
-            const int rc = roi_align_bwd_tile_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, R, B, c,
-                                                  (char*)workspace + bwd_levels_bytes(R), st);
+            const int rc = roi_align_bwd_tile_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, batched_ld, counts,
+                                                  R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
             if (rc != 1) return rc;
         }
     }
     int* lv = (int*)workspace;
-    if (levels) cudaMemcpyAsync(lv, levels, sizeof(int) * R, cudaMemcpyDeviceToDevice, st);
-    else if (R > 0) {
+    if (batched_ld > 0) {
+        if (R > 0) k_bwd_levels_batched<<<cdiv(R, 256), 256, 0, st>>>(lv, rois, batched_ld, counts, R, c.finest_scale, c.num_levels);
+    } else if (levels) {
+        cudaMemcpyAsync(lv, levels, sizeof(int) * R, cudaMemcpyDeviceToDevice, st);
+    } else if (R > 0) {
         int rc = b2d_roi_levels(lv, rois, roi_ld, R, c.finest_scale, c.num_levels, stream);
         if (rc != B2D_OK) return rc;
     }
@@ -329,10 +354,30 @@ int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, c
         run += a.tiles_x[l] * cdiv(c.H[l], kTileH);
     }
     a.tile_off[c.num_levels] = run;
-    a.gout = grad_out; a.rois = rois; a.roi_ld = roi_ld; a.roi_img = roi_img; a.levels = lv; a.R = R; a.B = B;
+    a.gout = grad_out; a.rois = rois; a.roi_ld = batched_ld > 0 ? batched_ld : roi_ld; a.roi_img = roi_img; a.levels = lv;
+    a.R = R; a.B = B; a.bld = batched_ld;
     dim3 grid((unsigned)(run * B), cdiv(c.C, kChPerCta));
     k_roi_align_bwd<<<grid, 256, 0, st>>>(a);
     return check_launch("roi_align_bwd");
+}
+
+int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
+                      const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg* cfg_host,
+                      void* workspace, size_t ws_bytes, void* stream) {
+    return roi_align_bwd_impl(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, 0, nullptr, R, B, cfg_host,
+                              workspace, ws_bytes, stream);
+}
+
+size_t b2d_roi_align_bwd_batched_workspace_bytes(long long ld, int B, const b2d_roi_cfg* cfg_host) {
+    return b2d_roi_align_bwd_workspace_bytes(ld * (B > 0 ? B : 1), B, cfg_host);
+}
+
+int b2d_roi_align_bwd_batched(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long ld,
+                              const int* counts, int B, const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes,
+                              void* stream) {
+    B2D_REQUIRE(counts && ld >= 1 && B >= 1, "roi_align_bwd_batched: bad args");
+    return roi_align_bwd_impl(grad_feat_ptrs_host, grad_out, rois, ld, nullptr, nullptr, ld, counts, (long long)B * ld, B,
+                              cfg_host, workspace, ws_bytes, stream);
 }
 
 int b2d_roi_pool_fwd(float* out, int* argmax, const float* feat, int B, int C, int H, int W, const float* rois,

@@ -431,6 +431,68 @@ class TrainHotPath(object):
                     rpn=self.rpn_targets, rpn_tar_cls=self.tar_cls, rpn_tar_reg=self.tar_reg, rcnn=self.roi_targets,
                     roi_feats=self.roi_align.out)
 
+    # ------------------------------------------------------------------ backward
+    def _bwd_buffers(self):
+        """Gradient maps and K6 workspace, allocated by the first backward() (call it once eagerly before capturing it)."""
+        if not hasattr(self, "_bwd"):
+            dev, B, cfg = self.device, self.B, self.roi_align.cfg
+            A = self.pyr.num_anchors
+            mf = torch.channels_last if cfg.layout == 1 else torch.contiguous_format
+            nb = _C.lib().b2d_roi_align_bwd_batched_workspace_bytes(self.roi_align.ld, B, ctypes.byref(cfg))
+            self._bwd = dict(
+                dcls=[torch.empty((B, A, H, W), dtype=torch.float32, device=dev) for H, W in self.pyr.grids],
+                dreg=[torch.empty((B, 4 * A, H, W), dtype=torch.float32, device=dev) for H, W in self.pyr.grids],
+                dfeat=[torch.empty((B, cfg.C, cfg.H[l], cfg.W[l]), dtype=torch.float32, device=dev, memory_format=mf)
+                       for l in range(cfg.num_levels)],
+                ws=torch.empty(nb, dtype=torch.uint8, device=dev),
+                stream=torch.cuda.Stream(device=dev))
+        return self._bwd
+
+    def backward(self, grad_rpn_cls, grad_rpn_reg, grad_roi_feats):
+        """Backward of the current step: the upstream gradients of its differentiable outputs -- rpn_tar_cls [B,1,m],
+        rpn_tar_reg [B,4,m] (m = RPN samples per image; columns at or past rpn.n_chosen[b] are not read) and roi_feats
+        [B*ld, C, 7, 7] (rows of slots at or past rcnn.n_chosen[b] are not read) -- to the gradients of its inputs:
+        (dcls_maps, dreg_maps, dfeat_maps), per level [B,A,H,W] / [B,4A,H,W] for the RPN head maps (zero away from the
+        sampled anchors: the adjoint of the gather in lib/anchor.py:49-56) and [B,C,H,W] for the first four FPN maps in
+        the layout the step read (channels_last for layout 1, NCHW for layout 0).  The head-map scatter
+        (b2d_scatter_head_grads) runs on a side stream beside the RoIAlign backward (b2d_roi_align_bwd_batched, K6);
+        both are joined before return.  The results live in buffers owned by the path, valid until the next backward();
+        after the first call nothing is allocated and nothing waits for the host, so step() + backward() can be
+        captured in one CUDA graph."""
+        cfg = self.roi_align.cfg
+        if cfg.layout not in (0, 1):
+            raise _C.B200DetError("TrainHotPath.backward: fp32 features (layout 0 or 1) only; bf16 features (layout %d) "
+                                  "have no RoIAlign backward" % cfg.layout)
+        B, rt, bt = self.B, self.rpn_targets, self.roi_targets
+        g_cls, g_reg, g_feat = _C.f32c(grad_rpn_cls), _C.f32c(grad_rpn_reg), _C.f32c(grad_roi_feats)
+        _C.require_cuda(g_cls, g_reg, g_feat)
+        for name, g, want in (("grad_rpn_cls", g_cls, self.tar_cls.shape), ("grad_rpn_reg", g_reg, self.tar_reg.shape),
+                              ("grad_roi_feats", g_feat, self.roi_align.out.shape)):
+            if g.shape != want:
+                raise _C.B200DetError("TrainHotPath.backward: %s has shape %s, expected %s"
+                                      % (name, tuple(g.shape), tuple(want)))
+        st = self._bwd_buffers()
+        cur, side = torch.cuda.current_stream(), st["stream"]
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            _C.call("b2d_scatter_head_grads", _ptrs(st["dcls"]), _ptrs(st["dreg"]), _C.ptr(g_cls), _C.ptr(g_reg),
+                    ctypes.byref(self.pyr.c), 1, _C.ptr(rt.chosen), _C.ptr(rt.n_chosen), rt.max_num, B, _C.stream())
+        _C.call("b2d_roi_align_bwd_batched", _ptrs(st["dfeat"]), _C.ptr(g_feat), _C.ptr(bt.tar_box), self.roi_align.ld,
+                _C.ptr(bt.n_chosen), B, ctypes.byref(cfg), _C.ptr(st["ws"]), st["ws"].numel(), _C.stream())
+        cur.wait_stream(side)
+        return st["dcls"], st["dreg"], st["dfeat"]
+
+    def step_autograd(self, cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw):
+        """step() as an autograd node (TrainStepFn): the same dict, with rpn_tar_cls, rpn_tar_reg and roi_feats
+        connected to cls_outs, reg_outs and feats, so that losses computed on them in PyTorch backpropagate into the
+        RPN head and the FPN through backward().  The outputs alias the path's buffers: run loss.backward() before the
+        next step."""
+        box = []
+        tc, tr, rf = TrainStepFn.apply(self, (gt, gt_count, gt_label, img_hw), box, *cls_outs, *reg_outs, *feats)
+        out = dict(box[0])
+        out.update(rpn_tar_cls=tc, rpn_tar_reg=tr, roi_feats=rf)
+        return out
+
     # ------------------------------------------------------------------ host-buffer entry
     def step_from_host(self, h_cls, h_reg, h_feats, h_gt, h_gt_label, gt_count, img_hw, h_out=None,
                        with_roi_feats=False, sparse=None):
@@ -564,6 +626,36 @@ class TrainHotPath(object):
         return self._read_back(out, h_out)
 
 
+class TrainStepFn(torch.autograd.Function):
+    """TrainHotPath.step as an autograd function: apply(path, (gt, gt_count, gt_label, img_hw), box, *cls_outs,
+    *reg_outs, *feats) -> (rpn_tar_cls, rpn_tar_reg, roi_feats); the step's whole output dict is appended to `box`.
+    The backward is TrainHotPath.backward; inputs that do not require grad (and FPN maps past the four RoIAlign
+    reads) get None."""
+
+    @staticmethod
+    def forward(ctx, path, args, box, *maps):
+        L = path.pyr.c.num_levels
+        out = path.step(list(maps[:L]), list(maps[L:2 * L]), list(maps[2 * L:]), *args)
+        box.append(out)
+        path._autograd_steps = getattr(path, "_autograd_steps", 0) + 1
+        ctx.path, ctx.step_id = path, path._autograd_steps
+        return out["rpn_tar_cls"].detach(), out["rpn_tar_reg"].detach(), out["roi_feats"].detach()
+
+    @staticmethod
+    def backward(ctx, g_cls, g_reg, g_feat):
+        path = ctx.path
+        if path._autograd_steps != ctx.step_id:
+            raise _C.B200DetError("TrainStepFn.backward: the path has run another step since; its outputs and sample "
+                                  "lists belong to that step (call loss.backward() before the next step)")
+        g_cls = torch.zeros_like(path.tar_cls) if g_cls is None else g_cls
+        g_reg = torch.zeros_like(path.tar_reg) if g_reg is None else g_reg
+        g_feat = torch.zeros_like(path.roi_align.out) if g_feat is None else g_feat
+        dcls, dreg, dfeat = path.backward(g_cls, g_reg, g_feat)
+        grads = list(dcls) + list(dreg) + list(dfeat)
+        grads += [None] * (len(ctx.needs_input_grad) - 3 - len(grads))
+        return (None, None, None) + tuple(g if need else None for g, need in zip(grads, ctx.needs_input_grad[3:]))
+
+
 class CascadeHotPath(object):
     """The stage loop of CascadeRCNN.forward_train (lib/detectors/cascade_rcnn.py:119-153; BASELINE config 3) minus
     the head convolutions and losses, batched: per stage bbox_target on the current boxes (b2d_roi_targets_fused,
@@ -592,13 +684,11 @@ class CascadeHotPath(object):
         self.step_cell = torch.zeros(1, dtype=torch.int64, device=device)        # one step counter for all stages
         for st in self.stages:
             st[0].step_cell, st[0].auto_bump = self.step_cell, False
-        self.roi_img = torch.arange(B, dtype=torch.int32, device=device).repeat_interleave(self.m).contiguous()
-        self.rois_flat = [torch.zeros((4, B * self.m), dtype=torch.float32, device=device) for _ in self.stages]
         mf = torch.channels_last if layout != 0 else torch.contiguous_format
         self.grads = [[torch.zeros((B,) + shp, dtype=torch.float32, device=device).contiguous(memory_format=mf) for shp in shapes]
                       for _ in self.stages]
         self.bwd_cfg = self.stages[0][1].cfg
-        nb = _C.lib().b2d_roi_align_bwd_workspace_bytes(B * self.m, B, ctypes.byref(self.bwd_cfg))
+        nb = _C.lib().b2d_roi_align_bwd_batched_workspace_bytes(self.m, B, ctypes.byref(self.bwd_cfg))
         self.bwd_ws = torch.empty(nb, dtype=torch.uint8, device=device)
         self.zero4 = _C.host_f4(z4, [0, 0, 0, 0])
         self.launches = len(self.stages) * (1 + 1 + 1) + 1
@@ -621,16 +711,12 @@ class CascadeHotPath(object):
         return outs
 
     def backward(self, grad_feats):
-        """grad_feats[s] [B*max_num, C, 7, 7] (zero rows for unused slots) -> per-stage feature gradients (K6);
+        """grad_feats[s] [B*max_num, C, 7, 7] (rows of unused slots are not read) -> per-stage feature gradients (K6);
         the caller (autograd in the reference) adds the stages."""
         for s, (tg, ra, _, _, _) in enumerate(self.stages):
-            self.rois_flat[s].copy_(tg.tar_box.permute(1, 0, 2).reshape(4, -1))
-            arr = (_C.c_void_p * _C.MAX_LEVELS)()
-            for i, g in enumerate(self.grads[s]):
-                arr[i] = g.data_ptr()
-            _C.call("b2d_roi_align_bwd", arr, _C.ptr(grad_feats[s]), _C.ptr(self.rois_flat[s]), self.B * self.m,
-                    _C.ptr(self.roi_img), None, self.B * self.m, self.B, ctypes.byref(self.bwd_cfg), _C.ptr(self.bwd_ws),
-                    self.bwd_ws.numel(), _C.stream())
+            _C.call("b2d_roi_align_bwd_batched", _ptrs(self.grads[s]), _C.ptr(grad_feats[s]), _C.ptr(tg.tar_box), self.m,
+                    _C.ptr(tg.n_chosen), self.B, ctypes.byref(self.bwd_cfg), _C.ptr(self.bwd_ws), self.bwd_ws.numel(),
+                    _C.stream())
         return self.grads
 
 
