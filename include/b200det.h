@@ -391,6 +391,15 @@ B2D_API size_t b2d_roi_align_bwd_batched_workspace_bytes(long long ld, int B, co
 B2D_API int b2d_roi_align_bwd_batched(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois,
                                       long long ld, const int* counts, int B, const b2d_roi_cfg* cfg_host, void* workspace,
                                       size_t ws_bytes, void* stream);
+/* backward of several b2d_roi_align_fwd_batched calls on one pyramid (the stages of a cascade): S = 1..4 sets, set s with
+ * rois_host[s] [B][4][ld_host[s]], counts_host[s] int32[B] and grad_out_host[s] [B*ld_host[s], C, PH, PW] (all DEVICE
+ * pointers, the arrays themselves on the host).  grad_feat receives the sum over the sets, every cell written once: the
+ * same kernels and bits as b2d_roi_align_bwd on the compacted RoI lists concatenated set-major.  Slots at or past
+ * counts_host[s][b] are not read.  b2d_roi_align_bwd_batched is the S = 1 case. */
+B2D_API size_t b2d_roi_align_bwd_multi_workspace_bytes(int S, const long long* ld_host, int B, const b2d_roi_cfg* cfg_host);
+B2D_API int b2d_roi_align_bwd_multi(void* const* grad_feat_ptrs_host, int S, const float* const* grad_out_host,
+                                    const float* const* rois_host, const long long* ld_host, const int* const* counts_host,
+                                    int B, const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes, void* stream);
 /* fp32 NCHW [B,C,H,W] -> NHWC [B,H,W,C]: reference-layout FPN features (lib/necks.py:69-90)
  * to the channels-last layout the vectorised RoIAlign kernels read. */
 B2D_API int b2d_nchw_to_nhwc(float* dst, const float* src, int B, int C, int H, int W, void* stream);

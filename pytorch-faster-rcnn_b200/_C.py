@@ -107,6 +107,7 @@ _SIGS = {
     "b2d_roi_align_fwd": [_P, _P, _P, c_ll, _P, _P, c_ll, _P, _P],
     "b2d_roi_align_bwd": [_P, _P, _P, c_ll, _P, _P, c_ll, c_int, _P, _P, c_size_t, _P],
     "b2d_roi_align_bwd_batched": [_P, _P, _P, c_ll, _P, c_int, _P, _P, c_size_t, _P],
+    "b2d_roi_align_bwd_multi": [_P, c_int, _P, _P, _P, _P, c_int, _P, _P, c_size_t, _P],
     "b2d_roi_levels": [_P, _P, c_ll, c_ll, c_float, c_int, _P],
     "b2d_nchw_to_nhwc": [_P, _P, c_int, c_int, c_int, c_int, _P],
     "b2d_refine_bboxes": [_P, _P, _P, c_ll, _P, c_ll, _P, _P, c_int, _P, _P, _P, c_int, _P, c_int, _P],
@@ -137,6 +138,7 @@ _SIZE_FNS = {
     "b2d_nms_workspace_bytes": [c_ll, c_int],
     "b2d_roi_align_bwd_workspace_bytes": [c_ll, c_int, _P],
     "b2d_roi_align_bwd_batched_workspace_bytes": [c_ll, c_int, _P],
+    "b2d_roi_align_bwd_multi_workspace_bytes": [c_int, _P, c_int, _P],
     "b2d_atss_workspace_bytes": [_P, c_int],
     "b2d_rcnn_detect_workspace_bytes": [c_int, c_int],
     "b2d_dense_select_workspace_bytes": [_P, c_int, c_int, c_int],

@@ -28,7 +28,7 @@
 
 namespace b2d {
 
-int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const float* grad_out, long long R, int B, const b2d_roi_cfg& c,
+int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const RoiSets& q, long long R, int B, const b2d_roi_cfg& c,
                               const void* meta, const int* bucket, const int* bcount, const int* guard, cudaStream_t st);
 
 namespace {
@@ -48,7 +48,8 @@ struct PatchArgs {
     b2d_roi_cfg cfg;
     float* grad[kMaxLevels];
     long long word0[kMaxLevels + 1];   // first bitmap word of each level
-    const float* gout; const BwdMeta* meta; const long long* poff;
+    RoiSets q;                         // grad_out rows
+    const BwdMeta* meta; const long long* poff;
     unsigned* anyb; unsigned* multi;
     float* scratch; int* flags;        // flags[0] = fallback
     const int* bucket; const int* bcount;
@@ -210,7 +211,7 @@ __global__ void __launch_bounds__(kPT, 7) k_bwd_patch(PatchArgs a) {
         // load = 4 sectors; one thread per channel would touch 32 sectors per load and bound the kernel by L1 sector
         // requests), 16 loads in flight; the shared-memory address of e advances incrementally (e += 128: channel += 128 /
         // bins, bin += 128 % bins with one wrap)
-        const float* go = a.gout + ((long long)r * C + (long long)cg * kPCg) * bins + tid;
+        const float* go = gout_row(a.q, r, (long long)C * bins) + (long long)cg * kPCg * bins + tid;
         const int dch = kPT / bins, db = kPT % bins;
         const int step = db * kPPitch + dch, wrap = 1 - bins * kPPitch;
         int b = tid % bins, addr = b * kPPitch + tid / bins;
@@ -455,10 +456,8 @@ size_t roi_align_bwd_patch_workspace(long long R, int B, const b2d_roi_cfg& c) {
 }
 
 // returns 1 if the configuration is not eligible (the caller then uses the tile / generic kernels)
-int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                            const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
-                            const b2d_roi_cfg& c, void* workspace,
-                            cudaStream_t st) {
+int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const RoiSets& q, const int* levels, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace, cudaStream_t st) {
     if (c.layout != 1 || c.sampling_ratio != 2 || c.PH > kMaxTerms || c.PW > kMaxTerms || c.PH * c.PW > kMaxBinsT) return 1;
     if (c.C % kPCg != 0 || R < 1) return 1;
     for (int l = 0; l < c.num_levels; ++l)
@@ -478,8 +477,7 @@ int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_
     float* scratch = (float*)w;
     MetaArgs ma;
     memset(&ma, 0, sizeof(ma));
-    ma.cfg = c; ma.rois = rois; ma.roi_ld = roi_ld; ma.roi_img = roi_img; ma.levels = levels; ma.R = R;
-    ma.batched_ld = batched_ld; ma.counts = counts;
+    ma.cfg = c; ma.q = q; ma.levels = levels; ma.R = R;
     a.cap_cells = patch_budget_cells(R);
     if (cudaMemsetAsync(anyb, 0, 2 * align256((size_t)words * 4 + 16), st) != cudaSuccess) return check_launch("roi_align_bwd(patch memset)");
     int run = 0;
@@ -490,7 +488,7 @@ int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_
         run += a.tiles_x[l] * cdiv(c.H[l], kMT);
     }
     a.tile_off[c.num_levels] = run;
-    a.gout = grad_out; a.meta = meta; a.poff = poff; a.anyb = anyb; a.multi = multi; a.scratch = scratch; a.flags = flags;
+    a.q = q; a.meta = meta; a.poff = poff; a.anyb = anyb; a.multi = multi; a.scratch = scratch; a.flags = flags;
     a.bucket = bucket; a.bcount = bcount; a.R = R;
     k_bwd_meta_mark<<<cdiv(R * 32, 256), 256, 0, st>>>(ma, a, meta);
     k_bwd_bucket_scan<<<B * c.num_levels + 1, 1024, 0, st>>>(meta, R, c.num_levels, B * c.num_levels, bucket, bcount, a.cap_cells,
@@ -502,7 +500,7 @@ int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_
     int rc = check_launch("roi_align_bwd(patch)");
     if (rc != B2D_OK) return rc;
     // fallback for patches that do not fit (flag raised by k_bwd_scan): the tile kernel on the same tables
-    return roi_align_bwd_tile_launch(grad_feat_ptrs_host, grad_out, R, B, c, meta, bucket, bcount, flags, st);
+    return roi_align_bwd_tile_launch(grad_feat_ptrs_host, q, R, B, c, meta, bucket, bcount, flags, st);
 }
 
 }  // namespace b2d

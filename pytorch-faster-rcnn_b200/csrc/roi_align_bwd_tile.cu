@@ -33,7 +33,8 @@ constexpr int kPitch = kCg + 4;        // shared-memory pitch of a bin row (floa
 struct TileArgs {
     b2d_roi_cfg cfg;
     float* grad[kMaxLevels];
-    const float* gout; const BwdMeta* meta; const int* bucket; const int* bcount;
+    RoiSets q;                         // grad_out rows
+    const BwdMeta* meta; const int* bucket; const int* bcount;
     long long R;
     int tile_off[kMaxLevels + 1], tiles_x[kMaxLevels];
     unsigned n_tiles;                  // tiles x images (grid.x of the ordinary launch)
@@ -86,7 +87,7 @@ __global__ void __launch_bounds__(kBT, 1) k_roi_align_bwd_tile(TileArgs a) {
     const int* bl = a.bucket + (long long)(img * c.num_levels + lvl) * a.R;
     const int nb = a.bcount[img * c.num_levels + lvl];
     auto fetch = [&](int r) {                            // grad_out[r][cg * 64 .. + 64][bins] -> registers
-        const float* go = a.gout + ((long long)r * C + (long long)cg * kCg + sch) * bins + sb0;
+        const float* go = gout_row(a.q, r, (long long)C * bins) + ((long long)cg * kCg + sch) * bins + sb0;
 #pragma unroll
         for (int k = 0; k < kStage; ++k) sv[k] = (sb0 + 4 * k < bins) ? go[4 * k] : 0.0f;
     };
@@ -219,7 +220,7 @@ __global__ void __launch_bounds__(kBT, 1) k_roi_align_bwd_tile(TileArgs a) {
 
 }  // namespace
 
-int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const float* grad_out, long long R, int B, const b2d_roi_cfg& c,
+int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const RoiSets& q, long long R, int B, const b2d_roi_cfg& c,
                               const void* meta, const int* bucket, const int* bcount, const int* guard, cudaStream_t st);
 
 size_t roi_align_bwd_tile_workspace(long long R, int B, int L) {
@@ -228,10 +229,8 @@ size_t roi_align_bwd_tile_workspace(long long R, int B, int L) {
 }
 
 // returns 1 if the configuration is not eligible (the caller then uses the generic kernel)
-int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                           const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
-                            const b2d_roi_cfg& c, void* workspace,
-                           cudaStream_t st) {
+int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const RoiSets& q, const int* levels, long long R, int B,
+                           const b2d_roi_cfg& c, void* workspace, cudaStream_t st) {
     if (c.layout != 1 || c.sampling_ratio != 2 || 2 * c.PH > kMaxS || 2 * c.PW > kMaxS || c.PH * c.PW > kMaxBinsT) return 1;
     if (c.C % kCg != 0 || R < 1) return 1;
     for (int l = 0; l < c.num_levels; ++l)
@@ -242,15 +241,14 @@ int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_o
     int* bcount = (int*)w;
     MetaArgs ma;
     memset(&ma, 0, sizeof(ma));
-    ma.cfg = c; ma.rois = rois; ma.roi_ld = roi_ld; ma.roi_img = roi_img; ma.levels = levels; ma.R = R;
-    ma.batched_ld = batched_ld; ma.counts = counts;
+    ma.cfg = c; ma.q = q; ma.levels = levels; ma.R = R;
     k_bwd_meta<<<cdiv(R, 256), 256, 0, st>>>(ma, meta);
     k_bwd_bucket<<<B * c.num_levels, 256, 0, st>>>(meta, R, c.num_levels, bucket, bcount);
-    return roi_align_bwd_tile_launch(grad_feat_ptrs_host, grad_out, R, B, c, meta, bucket, bcount, nullptr, st);
+    return roi_align_bwd_tile_launch(grad_feat_ptrs_host, q, R, B, c, meta, bucket, bcount, nullptr, st);
 }
 
 // the tile kernel alone, on a meta / bucket table that already exists; guard: see TileArgs
-int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const float* grad_out, long long R, int B, const b2d_roi_cfg& c,
+int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const RoiSets& q, long long R, int B, const b2d_roi_cfg& c,
                               const void* meta, const int* bucket, const int* bcount, const int* guard, cudaStream_t st) {
     TileArgs a;
     memset(&a, 0, sizeof(a));
@@ -263,7 +261,7 @@ int roi_align_bwd_tile_launch(void* const* grad_feat_ptrs_host, const float* gra
         run += a.tiles_x[l] * cdiv(c.H[l], kT);
     }
     a.tile_off[c.num_levels] = run;
-    a.gout = grad_out; a.meta = (const BwdMeta*)meta; a.bucket = bucket; a.bcount = bcount; a.R = R; a.guard = guard;
+    a.q = q; a.meta = (const BwdMeta*)meta; a.bucket = bucket; a.bcount = bcount; a.R = R; a.guard = guard;
     a.n_tiles = (unsigned)(run * B);
     unsigned gx = a.n_tiles;
     if (guard) {                                         // persistent: one wave

@@ -14,11 +14,60 @@ struct __align__(16) BwdMeta {
     float bw, bh; int _p0, _p1;
 };
 
+constexpr int kMaxSets = 4;            // RoI sets of one b2d_roi_align_bwd_multi call
+
+// The RoI slots of one K6 call.  Batched entries: S sets, set s the image-major [B][4][ld[s]] list b2d_roi_align_fwd_batched
+// read for it, with counts[s][B]; slots are numbered set-major, r = base[s] + b * ld[s] + j, and the grad_out row of slot r
+// is row b * ld[s] + j of gout[s].  Bucket lists are ascending in r, so a cell adds its contributions set by set: the result
+// is that of the unbatched entry on the compacted lists concatenated set-major.  The unbatched entry is one set with
+// ld[0] = 0: slot r is column r of rois[0] (stride roi_ld), of image roi_img[r], with grad_out row r.
+struct RoiSets {
+    int S;
+    long long roi_ld;
+    const int* roi_img;
+    long long base[kMaxSets + 1];      // first slot of each set; base[S] = R
+    long long ld[kMaxSets];
+    const float* rois[kMaxSets];
+    const float* gout[kMaxSets];
+    const int* counts[kMaxSets];
+};
+
+__device__ __forceinline__ int set_of(const RoiSets& q, long long r) {
+    int s = 0;
+    while (s + 1 < q.S && r >= q.base[s + 1]) ++s;
+    return s;
+}
+
+// first float of the grad_out row of slot r (`row` = C * PH * PW floats per row)
+__device__ __forceinline__ const float* gout_row(const RoiSets& q, long long r, long long row) {
+    const int s = set_of(q, r);
+    return q.gout[s] + (r - q.base[s]) * row;
+}
+
+struct RoiSlot { const float* box; long long ld; int img; };      // box: x1, coordinate k at box[k * ld]
+
+// box and image of slot r; box = NULL for a batched slot at or past its image's count (its box is not read)
+__device__ __forceinline__ RoiSlot roi_slot(const RoiSets& q, long long r) {
+    RoiSlot o;
+    const int s = set_of(q, r);
+    const long long ld = q.ld[s];
+    if (ld == 0) {
+        o.box = q.rois[0] + r; o.ld = q.roi_ld; o.img = q.roi_img ? q.roi_img[r] : 0;
+        return o;
+    }
+    const long long k = r - q.base[s];
+    o.img = (int)(k / ld);
+    const long long j = k - (long long)o.img * ld;
+    o.box = j < q.counts[s][o.img] ? q.rois[s] + (long long)o.img * 4 * ld + j : nullptr;
+    o.ld = ld;
+    return o;
+}
+
 struct MetaArgs {
     b2d_roi_cfg cfg;
-    const float* rois; long long roi_ld; const int* roi_img; const int* levels; long long R;
-    long long batched_ld;          // > 0: rois are image-major [B][4][ld], slot r = (r / ld, r % ld), counts per image
-    const int* counts;
+    RoiSets q;
+    const int* levels;                 // unbatched entry only (NULL: the level map)
+    long long R;
 };
 
 // The record of slot r.  A batched slot at or past its image's count gets img = -1 and an empty tap box: no bucket lists
@@ -26,20 +75,15 @@ struct MetaArgs {
 __device__ __forceinline__ BwdMeta bwd_meta_of(const MetaArgs& a, long long r) {
     const b2d_roi_cfg& c = a.cfg;
     BwdMeta m;
-    const float* p = a.rois + r;
-    if (a.batched_ld > 0) {
-        const int img = (int)(r / a.batched_ld);
-        if (r - (long long)img * a.batched_ld >= a.counts[img]) {
-            m.img = -1; m.lvl = 0; m.y0 = m.x0 = 0; m.y1 = m.x1 = -1;
-            m.sx = m.sy = m.bw = m.bh = 0.0f; m._p0 = m._p1 = 0;
-            return m;
-        }
-        p += (long long)img * 3 * a.batched_ld;
-        m.img = img;
-    } else {
-        m.img = a.roi_img ? a.roi_img[r] : 0;
+    const RoiSlot sl = roi_slot(a.q, r);
+    if (!sl.box) {
+        m.img = -1; m.lvl = 0; m.y0 = m.x0 = 0; m.y1 = m.x1 = -1;
+        m.sx = m.sy = m.bw = m.bh = 0.0f; m._p0 = m._p1 = 0;
+        return m;
     }
-    const long long ld = a.batched_ld > 0 ? a.batched_ld : a.roi_ld;
+    m.img = sl.img;
+    const float* p = sl.box;
+    const long long ld = sl.ld;
     const float x1 = p[0], y1 = p[ld], x2 = p[2 * ld], y2 = p[3 * ld];
     m.lvl = a.levels ? a.levels[r] : (c.num_levels > 1 ? roi_level(x1, y1, x2, y2, c.finest_scale, c.num_levels) : 0);
     const int H = c.H[m.lvl], W = c.W[m.lvl];

@@ -13,7 +13,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "roi_common.cuh"
+#include "roi_bwd_common.cuh"
 
 namespace b2d {
 
@@ -21,14 +21,10 @@ namespace b2d {
 size_t roi_align_bwd_tile_workspace(long long R, int B, int L);
 // patch form (roi_align_bwd_patch.cu): its workspace begins with the tile form's tables, so either can use it
 size_t roi_align_bwd_patch_workspace(long long R, int B, const b2d_roi_cfg& c);
-int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                            const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
-                            const b2d_roi_cfg& c, void* workspace,
-                            cudaStream_t st);
-int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                           const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
-                            const b2d_roi_cfg& c, void* workspace,
-                           cudaStream_t st);
+int roi_align_bwd_patch_try(void* const* grad_feat_ptrs_host, const RoiSets& q, const int* levels, long long R, int B,
+                            const b2d_roi_cfg& c, void* workspace, cudaStream_t st);
+int roi_align_bwd_tile_try(void* const* grad_feat_ptrs_host, const RoiSets& q, const int* levels, long long R, int B,
+                           const b2d_roi_cfg& c, void* workspace, cudaStream_t st);
 
 struct AxisTapB { int lo, hi; float l, h; int valid; };
 
@@ -51,27 +47,19 @@ constexpr int kAxisMax = 16;                // PH*sr, PW*sr limit (7*2 = 14)
 struct BwdArgs {
     b2d_roi_cfg cfg;
     void* grad[kMaxLevels];
-    const float* gout; const float* rois; long long roi_ld;
-    const int* roi_img; const int* levels; long long R; int B;
-    long long bld;                          // > 0: rois image-major [B][4][bld] (roi_ld == bld); levels -1 = empty slot
+    RoiSets q;
+    const int* levels;                      // level of every slot, -1 = empty batched slot
+    long long R; int B;
     int tile_off[kMaxLevels + 1];           // CTA-tile prefix per level (per image)
     int tiles_x[kMaxLevels];
 };
 
-// x1 of slot r; coordinate k at [k * roi_ld]
-__device__ __forceinline__ const float* bwd_roi_ptr(const BwdArgs& a, long long r) {
-    return a.rois + r + (a.bld > 0 ? (r / a.bld) * 3 * a.bld : 0);
-}
-
-// level of every slot of an image-major [B][4][ld] RoI list, -1 for the slots at or past counts[b] (their boxes unread)
-__global__ void __launch_bounds__(256) k_bwd_levels_batched(int* __restrict__ lv, const float* __restrict__ rois, long long ld,
-                                                            const int* __restrict__ counts, long long R, float finest, int L) {
+// level of every slot of the batched entries, -1 for the slots at or past their image's count (their boxes unread)
+__global__ void __launch_bounds__(256) k_bwd_levels_batched(int* __restrict__ lv, RoiSets q, long long R, float finest, int L) {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= R) return;
-    const int img = (int)(r / ld);
-    if (r - (long long)img * ld >= counts[img]) { lv[r] = -1; return; }
-    const float* p = rois + r + (long long)img * 3 * ld;
-    lv[r] = roi_level(p[0], p[ld], p[2 * ld], p[3 * ld], finest, L);
+    const RoiSlot sl = roi_slot(q, r);
+    lv[r] = sl.box ? roi_level(sl.box[0], sl.box[sl.ld], sl.box[2 * sl.ld], sl.box[3 * sl.ld], finest, L) : -1;
 }
 
 __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
@@ -107,11 +95,11 @@ __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
         while (r0 < a.R && s_n < kSub) {
             const long long r = r0 + threadIdx.x;
             bool hit = false;
-            if (r < a.R && a.levels[r] == lvl && (a.bld > 0 ? (int)(r / a.bld) : (a.roi_img ? a.roi_img[r] : 0)) == img) {
-                const float* rp = bwd_roi_ptr(a, r);
+            const RoiSlot sl = r < a.R && a.levels[r] == lvl ? roi_slot(a.q, r) : RoiSlot{nullptr, 0, -1};
+            if (sl.img == img) {
                 const float off = c.aligned ? 0.5f : 0.0f;
-                const float sx = rp[0] * scale - off, sy = rp[a.roi_ld] * scale - off;
-                const float ex = rp[2 * a.roi_ld] * scale - off, ey = rp[3 * a.roi_ld] * scale - off;
+                const float sx = sl.box[0] * scale - off, sy = sl.box[sl.ld] * scale - off;
+                const float ex = sl.box[2 * sl.ld] * scale - off, ey = sl.box[3 * sl.ld] * scale - off;
                 // conservative extent of the taps: samples lie in [s, max(e, s+1)], taps reach one cell
                 // further, and everything beyond the map is clamped onto the last row / column
                 float ylo = floorf(fminf(sy, ey)) - 1.0f, yhi = ceilf(fmaxf(ey, sy + 1.0f)) + 1.0f;
@@ -145,10 +133,11 @@ __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
         // ---- axis taps of the batch
         for (int q = threadIdx.x; q < nb * (ny + nx); q += blockDim.x) {
             const int e = q / (ny + nx), k = q - e * (ny + nx);
-            const float* rp = bwd_roi_ptr(a, s_list[e]);
+            const RoiSlot sl = roi_slot(a.q, s_list[e]);
+            const float* rp = sl.box;
             const float off = c.aligned ? 0.5f : 0.0f;
-            const float sx = rp[0] * scale - off, sy = rp[a.roi_ld] * scale - off;
-            const float ex = rp[2 * a.roi_ld] * scale - off, ey = rp[3 * a.roi_ld] * scale - off;
+            const float sx = rp[0] * scale - off, sy = rp[sl.ld] * scale - off;
+            const float ex = rp[2 * sl.ld] * scale - off, ey = rp[3 * sl.ld] * scale - off;
             float rw = ex - sx, rh = ey - sy;
             if (!c.aligned) { rw = fmaxf(rw, 1.0f); rh = fmaxf(rh, 1.0f); }
             const float bh = rh / (float)c.PH, bw = rw / (float)c.PW;
@@ -159,7 +148,7 @@ __global__ void __launch_bounds__(256) k_roi_align_bwd(BwdArgs a) {
         // ---- ordered accumulation
         if (live) {
             for (int e = 0; e < nb; ++e) {
-                const float* go = a.gout + ((long long)s_list[e] * c.C + c0) * bins;
+                const float* go = gout_row(a.q, s_list[e], (long long)c.C * bins) + (long long)c0 * bins;
                 for (int ph = 0; ph < c.PH; ++ph) {
                     // does any y-sample of this bin row touch row y?
                     bool anyy = false;
@@ -308,12 +297,11 @@ size_t b2d_roi_align_bwd_workspace_bytes(long long R, int B, const b2d_roi_cfg* 
     return bwd_levels_bytes(R) + n;                                                   // level ids in front
 }
 
-// the two entry points below: an explicit RoI list with roi_img / levels, or (batched_ld > 0) the image-major
-// [B][4][batched_ld] slots of b2d_roi_align_fwd_batched with per-image counts
-static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
-                              const int* roi_img, const int* levels, long long batched_ld, const int* counts, long long R, int B,
+// the entry points below: an explicit RoI list with roi_img / levels, or the image-major [B][4][ld] slots of
+// b2d_roi_align_fwd_batched with per-image counts, one or several sets of them (RoiSets)
+static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const RoiSets& q, const int* levels, long long R, int B,
                               const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes, void* stream) {
-    B2D_REQUIRE(grad_feat_ptrs_host && grad_out && rois && cfg_host && R >= 0 && B >= 1, "roi_align_bwd: bad args");
+    B2D_REQUIRE(grad_feat_ptrs_host && cfg_host && R >= 0 && B >= 1, "roi_align_bwd: bad args");
     const b2d_roi_cfg& c = *cfg_host;
     B2D_REQUIRE(c.num_levels >= 1 && c.num_levels <= B2D_MAX_LEVELS, "roi_align_bwd: bad cfg");
     B2D_REQUIRE(c.layout == 0 || c.layout == 1, "roi_align_bwd: fp32 NCHW (0) or NHWC (1) gradients only");
@@ -324,23 +312,21 @@ static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const float* gra
     {   // NHWC fp32 gradients with 2x2 samples: patch form (B2D_ROI_BWD_TILE=2, default), tile-gather form (=1);
         // B2D_ROI_BWD_TILE=0 forces the generic, torchvision-bit-identical kernel below
         if (knobs().roi_bwd_tile >= 2) {                  // patch form ("sorted scatter", roi_align_bwd_patch.cu): default
-            const int rc = roi_align_bwd_patch_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, batched_ld, counts,
-                                                   R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
+            const int rc = roi_align_bwd_patch_try(grad_feat_ptrs_host, q, levels, R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
             if (rc != 1) return rc;
         }
         if (knobs().roi_bwd_tile != 0) {
-            const int rc = roi_align_bwd_tile_try(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, batched_ld, counts,
-                                                  R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
+            const int rc = roi_align_bwd_tile_try(grad_feat_ptrs_host, q, levels, R, B, c, (char*)workspace + bwd_levels_bytes(R), st);
             if (rc != 1) return rc;
         }
     }
     int* lv = (int*)workspace;
-    if (batched_ld > 0) {
-        if (R > 0) k_bwd_levels_batched<<<cdiv(R, 256), 256, 0, st>>>(lv, rois, batched_ld, counts, R, c.finest_scale, c.num_levels);
+    if (q.ld[0] > 0) {
+        if (R > 0) k_bwd_levels_batched<<<cdiv(R, 256), 256, 0, st>>>(lv, q, R, c.finest_scale, c.num_levels);
     } else if (levels) {
         cudaMemcpyAsync(lv, levels, sizeof(int) * R, cudaMemcpyDeviceToDevice, st);
     } else if (R > 0) {
-        int rc = b2d_roi_levels(lv, rois, roi_ld, R, c.finest_scale, c.num_levels, stream);
+        int rc = b2d_roi_levels(lv, q.rois[0], q.roi_ld, R, c.finest_scale, c.num_levels, stream);
         if (rc != B2D_OK) return rc;
     }
     BwdArgs a;
@@ -354,8 +340,7 @@ static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const float* gra
         run += a.tiles_x[l] * cdiv(c.H[l], kTileH);
     }
     a.tile_off[c.num_levels] = run;
-    a.gout = grad_out; a.rois = rois; a.roi_ld = batched_ld > 0 ? batched_ld : roi_ld; a.roi_img = roi_img; a.levels = lv;
-    a.R = R; a.B = B; a.bld = batched_ld;
+    a.q = q; a.levels = lv; a.R = R; a.B = B;
     dim3 grid((unsigned)(run * B), cdiv(c.C, kChPerCta));
     k_roi_align_bwd<<<grid, 256, 0, st>>>(a);
     return check_launch("roi_align_bwd");
@@ -364,20 +349,53 @@ static int roi_align_bwd_impl(void* const* grad_feat_ptrs_host, const float* gra
 int b2d_roi_align_bwd(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long roi_ld,
                       const int* roi_img, const int* levels, long long R, int B, const b2d_roi_cfg* cfg_host,
                       void* workspace, size_t ws_bytes, void* stream) {
-    return roi_align_bwd_impl(grad_feat_ptrs_host, grad_out, rois, roi_ld, roi_img, levels, 0, nullptr, R, B, cfg_host,
-                              workspace, ws_bytes, stream);
+    B2D_REQUIRE(grad_out && rois, "roi_align_bwd: bad args");
+    RoiSets q;
+    memset(&q, 0, sizeof(q));
+    q.S = 1; q.roi_ld = roi_ld; q.roi_img = roi_img; q.base[1] = R; q.rois[0] = rois; q.gout[0] = grad_out;
+    return roi_align_bwd_impl(grad_feat_ptrs_host, q, levels, R, B, cfg_host, workspace, ws_bytes, stream);
+}
+
+// slots of S batched sets (0 if the arguments are out of range: the entry then refuses them)
+static long long multi_slots(int S, const long long* ld_host, int B) {
+    if (S < 1 || S > kMaxSets || !ld_host || B < 1) return 0;
+    long long R = 0;
+    for (int s = 0; s < S; ++s) {
+        if (ld_host[s] < 1) return 0;
+        R += ld_host[s] * B;
+    }
+    return R;
+}
+
+size_t b2d_roi_align_bwd_multi_workspace_bytes(int S, const long long* ld_host, int B, const b2d_roi_cfg* cfg_host) {
+    return b2d_roi_align_bwd_workspace_bytes(multi_slots(S, ld_host, B), B, cfg_host);
+}
+
+int b2d_roi_align_bwd_multi(void* const* grad_feat_ptrs_host, int S, const float* const* grad_out_host,
+                            const float* const* rois_host, const long long* ld_host, const int* const* counts_host, int B,
+                            const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes, void* stream) {
+    const long long R = multi_slots(S, ld_host, B);
+    B2D_REQUIRE(R > 0 && grad_out_host && rois_host && counts_host, "roi_align_bwd_multi: bad args (1 <= S <= 4, ld >= 1, B >= 1)");
+    RoiSets q;
+    memset(&q, 0, sizeof(q));
+    q.S = S;
+    for (int s = 0; s < S; ++s) {
+        B2D_REQUIRE(grad_out_host[s] && rois_host[s] && counts_host[s], "roi_align_bwd_multi: NULL set pointer");
+        q.ld[s] = ld_host[s]; q.rois[s] = rois_host[s]; q.gout[s] = grad_out_host[s]; q.counts[s] = counts_host[s];
+        q.base[s + 1] = q.base[s] + ld_host[s] * B;
+    }
+    return roi_align_bwd_impl(grad_feat_ptrs_host, q, nullptr, R, B, cfg_host, workspace, ws_bytes, stream);
 }
 
 size_t b2d_roi_align_bwd_batched_workspace_bytes(long long ld, int B, const b2d_roi_cfg* cfg_host) {
-    return b2d_roi_align_bwd_workspace_bytes(ld * (B > 0 ? B : 1), B, cfg_host);
+    return b2d_roi_align_bwd_multi_workspace_bytes(1, &ld, B, cfg_host);
 }
 
 int b2d_roi_align_bwd_batched(void* const* grad_feat_ptrs_host, const float* grad_out, const float* rois, long long ld,
                               const int* counts, int B, const b2d_roi_cfg* cfg_host, void* workspace, size_t ws_bytes,
                               void* stream) {
-    B2D_REQUIRE(counts && ld >= 1 && B >= 1, "roi_align_bwd_batched: bad args");
-    return roi_align_bwd_impl(grad_feat_ptrs_host, grad_out, rois, ld, nullptr, nullptr, ld, counts, (long long)B * ld, B,
-                              cfg_host, workspace, ws_bytes, stream);
+    return b2d_roi_align_bwd_multi(grad_feat_ptrs_host, 1, &grad_out, &rois, &ld, &counts, B, cfg_host, workspace, ws_bytes,
+                                   stream);
 }
 
 int b2d_roi_pool_fwd(float* out, int* argmax, const float* feat, int B, int C, int H, int W, const float* rois,

@@ -720,6 +720,232 @@ class CascadeHotPath(object):
         return self.grads
 
 
+class CascadeTrainHotPath(object):
+    """CascadeRCNN.forward_train (lib/detectors/cascade_rcnn.py:106-153; BASELINE config 3) after the convolutions, batched:
+    RPN proposals (K3 + K4), RPN anchor targets and the head-output gather as in TrainHotPath, then per stage bbox_target
+    on the current boxes (GT prepended, thresholds .5/.6/.7) -> FPN RoIAlign of the sampled RoIs (K5) -> the caller's
+    stage head -> BBoxHead.refine_bboxes on the detached reg_out with the sampled labels (b2d_refine_bboxes, stage stds,
+    GT columns dropped, clamped to img_hw) -> the next stage's boxes.  num_stages = 1 .. 3.  backward() returns the RPN
+    head-map gradients and the FPN gradient summed over every stage, the latter from ONE RoIAlign backward call over all
+    the stages' RoIs (b2d_roi_align_bwd_multi).  Everything is allocated here or by the first backward(); after that
+    step() + backward() allocate nothing and never wait for the host, so they can be captured in one CUDA graph."""
+
+    def __init__(self, B, grids, device, strides=(4, 8, 16, 32, 64), gt_ld=64, feat_channels=256,
+                 rpn_proposal=None, rpn_assigner=None, rpn_sampler=None, rcnn_sampler=None,
+                 rpn_stds=(1.0, 1.0, 1.0, 1.0), allowed_border=0, num_stages=3, num_classes=21, reg_class_agnostic=False,
+                 thresholds=(0.5, 0.6, 0.7),
+                 stage_stds=((0.1, 0.1, 0.2, 0.2), (0.05, 0.05, 0.1, 0.1), (0.033, 0.033, 0.067, 0.067)),
+                 layout=1, seed=0):
+        if layout not in (0, 1):
+            raise _C.B200DetError("CascadeTrainHotPath: fp32 features (layout 0 or 1) only; bf16 features (layout %d) "
+                                  "have no RoIAlign backward" % layout)
+        S = int(num_stages)
+        if not 1 <= S <= 3 or len(thresholds) < S or len(stage_stds) < S:
+            raise _C.B200DetError("CascadeTrainHotPath: num_stages must be in 1..3 with one threshold and one stds tuple "
+                                  "per stage (got %d stages, %d thresholds, %d stds)" % (S, len(thresholds), len(stage_stds)))
+        z4 = (0.0, 0.0, 0.0, 0.0)
+        rpn_proposal = rpn_proposal or dict(pre_nms=2000, post_nms=2000, max_num=2000, nms_iou=0.7, min_bbox_size=0)
+        rpn_assigner = rpn_assigner or dict(pos_iou=0.7, neg_iou=0.3, min_pos_iou=0.3)
+        rpn_sampler = rpn_sampler or dict(max_num=256, pos_num=128)
+        rcnn_sampler = rcnn_sampler or dict(max_num=512, pos_num=128)
+        self.B, self.device, self.S = B, device, S
+        self.NC, self.reg_c = int(num_classes), 1 if reg_class_agnostic else int(num_classes)
+        self.m = m = int(rcnn_sampler["max_num"])
+        self.pyr = AnchorPyramid(strides, grids)
+        self.proposals = RpnProposals(self.pyr, B, rpn_proposal, z4, rpn_stds, device)
+        self.rpn_targets = BatchedTargets(B, self.pyr.total, gt_ld, rpn_assigner, rpn_sampler, z4, rpn_stds, device,
+                                          pyramid=self.pyr, border=allowed_border, seed=seed)
+        shapes = [(feat_channels, g[0], g[1]) for g in grids[:4]]
+        self.targets, self.roi_align = [], []
+        n = self.proposals.P
+        for s in range(S):
+            thr = thresholds[s]
+            self.targets.append(BatchedTargets(B, n, gt_ld, dict(pos_iou=thr, neg_iou=thr, min_pos_iou=thr), rcnn_sampler, z4,
+                                               stage_stds[s], device, prepend_gt=True, seed=seed + 1 + s))
+            self.roi_align.append(BatchedRoIAlign(B, m, shapes, list(strides[:4]), device, layout=layout))
+            n = m
+        # one device-side step counter for every sampler (graph-replay safe): starts at 1, advanced once per step after
+        # the last stage's sampler has read it.  Stage 0 therefore draws what TrainHotPath's RoI sampler draws.
+        self.step_cell = torch.ones(1, dtype=torch.int64, device=device)
+        for t in [self.rpn_targets] + self.targets:
+            t.step_cell, t.auto_bump = self.step_cell, False
+        self.refined = [torch.zeros((B, 4, m), dtype=torch.float32, device=device) for _ in range(S - 1)]
+        self.refined_count = [torch.zeros(B, dtype=torch.int32, device=device) for _ in range(S - 1)]
+        self.stds = [_C.host_f4(sd, [1, 1, 1, 1]) for sd in stage_stds[:S]]
+        self.zero4 = _C.host_f4(z4, [0, 0, 0, 0])
+        k = rpn_sampler["max_num"]
+        self.tar_cls = torch.zeros((B, 1, k), dtype=torch.float32, device=device)
+        self.tar_reg = torch.zeros((B, 4, k), dtype=torch.float32, device=device)
+        self.no_rois = torch.zeros(B, dtype=torch.int32, device=device)      # counts of the empty set (no stage gradient)
+
+    def reset_step(self):
+        """Restart the samplers' step counter (tests: the same random stream again)."""
+        self.step_cell.fill_(1)
+
+    def step(self, cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw, heads):
+        """cls_outs / reg_outs: the RPN head maps per level; feats: the first four FPN maps (channels_last for layout 1);
+        heads[s](roi_feats [B*m, C, 7, 7]) -> (cls_out [B*m, num_classes], reg_out [B*m, 4*num_classes] or [B*m, 4]).
+        Returns TrainHotPath.step's keys (rcnn / roi_feats: stage 0) and `stages`, per stage a dict of its targets
+        (BatchedTargets), roi_feats, cls_out, reg_out and the refined boxes [B,4,m] + counts [B] that feed the next stage
+        (None after the last stage)."""
+        return self._run(cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw, heads)
+
+    def _run(self, cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw, heads, wrap_rpn=None, wrap_roi=None):
+        if len(heads) < self.S:
+            raise _C.B200DetError("CascadeTrainHotPath.step: %d stage heads for %d stages" % (len(heads), self.S))
+        B, m = self.B, self.m
+        props, scores, count = self.proposals(cls_outs, reg_outs, img_hw)
+        rt = self.rpn_targets(gt, gt_count, None, img_hw=img_hw)
+        _C.call("b2d_gather_head_outputs", _C.ptr(self.tar_cls), _C.ptr(self.tar_reg), _ptrs(cls_outs), _ptrs(reg_outs),
+                ctypes.byref(self.pyr.c), 1, _C.ptr(rt.chosen), _C.ptr(rt.n_chosen), rt.max_num, B, _C.stream())
+        tc, tr = (self.tar_cls, self.tar_reg) if wrap_rpn is None else wrap_rpn()
+        boxes, bcount, stages = props, count, []
+        for s in range(self.S):
+            bt = self.targets[s](gt, gt_count, gt_label, boxes=boxes, box_count=bcount)
+            if s + 1 == self.S:
+                _C.call("b2d_counter_add", _C.ptr(self.step_cell), 1, _C.stream())   # every sampler has read it
+            rf = self.roi_align[s](feats, bt.tar_box, bt.n_chosen)
+            if wrap_roi is not None:
+                rf = wrap_roi(s)
+            cls_out, reg_out = heads[s](rf)
+            if tuple(cls_out.shape) != (B * m, self.NC) or tuple(reg_out.shape) != (B * m, 4 * self.reg_c):
+                raise _C.B200DetError("CascadeTrainHotPath.step: stage %d head returned %s / %s, expected [%d, %d] / [%d, %d]"
+                                      % (s, tuple(cls_out.shape), tuple(reg_out.shape), B * m, self.NC, B * m, 4 * self.reg_c))
+            st = dict(targets=bt, roi_feats=rf, cls_out=cls_out, reg_out=reg_out, boxes=None, count=None)
+            if s + 1 < self.S:
+                reg = _C.f32c(reg_out.detach())
+                _C.call("b2d_refine_bboxes", _C.ptr(self.refined[s]), _C.ptr(self.refined_count[s]), _C.ptr(bt.tar_box), m,
+                        _C.ptr(bt.n_chosen), m, _C.ptr(bt.tar_label if self.reg_c > 1 else None), _C.ptr(reg), self.reg_c,
+                        _C.ptr(bt.tar_is_gt), self.zero4, self.stds[s], 1, _C.ptr(img_hw), B, _C.stream())
+                boxes, bcount = self.refined[s], self.refined_count[s]
+                st.update(boxes=boxes, count=bcount)
+            stages.append(st)
+        return dict(props=props, scores=scores, prop_count=count, rpn=rt, rpn_tar_cls=tc, rpn_tar_reg=tr,
+                    rcnn=stages[0]["targets"], roi_feats=stages[0]["roi_feats"], stages=stages)
+
+    def _bwd_buffers(self):
+        """Gradient maps and K6 workspace, allocated by the first backward() (call it once eagerly before capturing it)."""
+        if not hasattr(self, "_bwd"):
+            dev, B, cfg = self.device, self.B, self.roi_align[0].cfg
+            A = self.pyr.num_anchors
+            mf = torch.channels_last if cfg.layout == 1 else torch.contiguous_format
+            lds = (_C.c_ll * self.S)(*([self.m] * self.S))
+            nb = _C.lib().b2d_roi_align_bwd_multi_workspace_bytes(self.S, lds, B, ctypes.byref(cfg))
+            self._bwd = dict(
+                dcls=[torch.empty((B, A, H, W), dtype=torch.float32, device=dev) for H, W in self.pyr.grids],
+                dreg=[torch.empty((B, 4 * A, H, W), dtype=torch.float32, device=dev) for H, W in self.pyr.grids],
+                dfeat=[torch.empty((B, cfg.C, cfg.H[l], cfg.W[l]), dtype=torch.float32, device=dev, memory_format=mf)
+                       for l in range(cfg.num_levels)],
+                ws=torch.empty(nb, dtype=torch.uint8, device=dev),
+                stream=torch.cuda.Stream(device=dev))
+        return self._bwd
+
+    def backward(self, grad_rpn_cls, grad_rpn_reg, grad_roi_feats):
+        """Backward of the current step: upstream gradients of rpn_tar_cls [B,1,k], rpn_tar_reg [B,4,k] (columns at or past
+        rpn.n_chosen[b] are not read) and, per stage, of its roi_feats [B*m, C, 7, 7] (rows at or past the stage's
+        n_chosen[b] are not read; None leaves the stage out) -> (dcls_maps, dreg_maps, dfeat_maps) as in
+        TrainHotPath.backward, dfeat the sum over the stages.  The head-map scatter runs on a side stream beside ONE
+        b2d_roi_align_bwd_multi call over every given stage.  The results live in buffers owned by the path, valid until
+        the next backward()."""
+        if len(grad_roi_feats) != self.S:
+            raise _C.B200DetError("CascadeTrainHotPath.backward: %d roi_feats gradients for %d stages"
+                                  % (len(grad_roi_feats), self.S))
+        B, rt = self.B, self.rpn_targets
+        g_cls, g_reg = _C.f32c(grad_rpn_cls), _C.f32c(grad_rpn_reg)
+        g_feats = [None if g is None else _C.f32c(g) for g in grad_roi_feats]
+        _C.require_cuda(g_cls, g_reg, *g_feats)
+        want = self.roi_align[0].out.shape
+        checks = [("grad_rpn_cls", g_cls, self.tar_cls.shape), ("grad_rpn_reg", g_reg, self.tar_reg.shape)]
+        checks += [("grad_roi_feats[%d]" % s, g, want) for s, g in enumerate(g_feats) if g is not None]
+        for name, g, shape in checks:
+            if g.shape != shape:
+                raise _C.B200DetError("CascadeTrainHotPath.backward: %s has shape %s, expected %s"
+                                      % (name, tuple(g.shape), tuple(shape)))
+        st = self._bwd_buffers()
+        sets = [(g, self.targets[s].tar_box, self.targets[s].n_chosen) for s, g in enumerate(g_feats) if g is not None]
+        if not sets:                                     # no stage: one empty set writes the zero gradient
+            sets = [(self.roi_align[0].out, self.targets[0].tar_box, self.no_rois)]
+        n = len(sets)
+        gouts = (_C.c_void_p * n)(*[g.data_ptr() for g, _, _ in sets])
+        rois = (_C.c_void_p * n)(*[r.data_ptr() for _, r, _ in sets])
+        counts = (_C.c_void_p * n)(*[c.data_ptr() for _, _, c in sets])
+        lds = (_C.c_ll * n)(*([self.m] * n))
+        cur, side = torch.cuda.current_stream(), st["stream"]
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            _C.call("b2d_scatter_head_grads", _ptrs(st["dcls"]), _ptrs(st["dreg"]), _C.ptr(g_cls), _C.ptr(g_reg),
+                    ctypes.byref(self.pyr.c), 1, _C.ptr(rt.chosen), _C.ptr(rt.n_chosen), rt.max_num, B, _C.stream())
+        _C.call("b2d_roi_align_bwd_multi", _ptrs(st["dfeat"]), n, gouts, rois, lds, counts, B,
+                ctypes.byref(self.roi_align[0].cfg), _C.ptr(st["ws"]), st["ws"].numel(), _C.stream())
+        cur.wait_stream(side)
+        return st["dcls"], st["dreg"], st["dfeat"]
+
+    def step_autograd(self, cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw, heads):
+        """step() with rpn_tar_cls, rpn_tar_reg and every stage's roi_feats as autograd outputs of cls_outs, reg_outs and
+        feats; the heads run on those outputs, so one loss built in PyTorch trains the heads, the RPN head and the FPN.
+        loss.backward() runs backward() once, with one RoIAlign backward call for all the stages (see CascadeStepFn).
+        The outputs alias the path's buffers: run loss.backward() before the next step."""
+        self._autograd_steps = getattr(self, "_autograd_steps", 0) + 1
+        self._pending = dict(rpn=None, roi=[None] * self.S)
+        token = CascadeStepFn.apply(self, *cls_outs, *reg_outs, *feats)
+        wrap_rpn = lambda: _CascadeOutFn.apply(self, "rpn", token, self.tar_cls, self.tar_reg)
+        wrap_roi = lambda s: _CascadeOutFn.apply(self, s, token, self.roi_align[s].out)
+        return self._run(cls_outs, reg_outs, feats, gt, gt_count, gt_label, img_hw, heads, wrap_rpn, wrap_roi)
+
+    def _check_step(self, step_id):
+        if self._autograd_steps != step_id:
+            raise _C.B200DetError("CascadeTrainHotPath: backward after another step; its outputs and sample lists belong "
+                                  "to that step (call loss.backward() before the next step)")
+
+
+class CascadeStepFn(torch.autograd.Function):
+    """The node of CascadeTrainHotPath.step_autograd that takes every map: apply(path, *cls_outs, *reg_outs, *feats) ->
+    a 1-element token.  The RPN gather and each stage's RoIAlign (_CascadeOutFn) consume the token and only store their
+    upstream gradients on the path, so the engine runs this backward after all of them: it issues the scatter and one
+    b2d_roi_align_bwd_multi over the stored gradients (stages whose outputs the loss did not reach are left out)."""
+
+    @staticmethod
+    def forward(ctx, path, *maps):
+        ctx.path, ctx.step_id = path, path._autograd_steps
+        return maps[0].new_zeros(1)
+
+    @staticmethod
+    def backward(ctx, g_token):
+        path = ctx.path
+        path._check_step(ctx.step_id)
+        g = path._pending
+        g_cls, g_reg = g["rpn"] if g["rpn"] is not None else (torch.zeros_like(path.tar_cls), torch.zeros_like(path.tar_reg))
+        dcls, dreg, dfeat = path.backward(g_cls, g_reg, g["roi"])
+        grads = list(dcls) + list(dreg) + list(dfeat)
+        grads += [None] * (len(ctx.needs_input_grad) - 1 - len(grads))
+        return (None,) + tuple(x if need else None for x, need in zip(grads, ctx.needs_input_grad[1:]))
+
+
+class _CascadeOutFn(torch.autograd.Function):
+    """An output of CascadeTrainHotPath.step_autograd (what = "rpn": the gathered head outputs, what = s: stage s's RoI
+    features) as a function of the token; its backward stores the upstream gradient on the path."""
+
+    @staticmethod
+    def forward(ctx, path, what, token, *bufs):
+        ctx.path, ctx.what, ctx.step_id = path, what, path._autograd_steps
+        ctx.set_materialize_grads(False)
+        outs = tuple(b.detach() for b in bufs)
+        return outs if len(outs) > 1 else outs[0]
+
+    @staticmethod
+    def backward(ctx, *grads):
+        path = ctx.path
+        path._check_step(ctx.step_id)
+        if ctx.what == "rpn":
+            if grads[0] is not None or grads[1] is not None:
+                path._pending["rpn"] = tuple(torch.zeros_like(b) if g is None else g
+                                             for g, b in zip(grads, (path.tar_cls, path.tar_reg)))
+        else:
+            path._pending["roi"][ctx.what] = grads[0]
+        g_token = torch.zeros(1, device=path.device)
+        return (None, None, g_token) + (None,) * len(grads)
+
+
 class InferHotPath(object):
     """CascadeRCNN.forward_test (SURVEY 3.2, lib/detectors/cascade_rcnn.py:157-200) minus the backbone, neck and head
     layers, batched: RPN proposals at the test configuration (K3 + K4) -> per stage FPN RoIAlign of the current boxes (K5)
