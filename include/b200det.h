@@ -210,7 +210,8 @@ B2D_API int b2d_rpn_proposals_targets(float* props, float* scores, int* count, i
                               const b2d_roi_target_args* tg_host, void* stream);
 
 /* generic segmented top-k (descending, ties -> lowest index): values [S][ld] with
- * per-segment counts -> idx int32[S][k] (padded -1), out_count int32[S]. */
+ * per-segment counts (NULL: n each) -> idx int32[S][k] (padded -1), out_count int32[S].
+ * n > 16384 needs ld == n and k <= 16384. */
 B2D_API size_t b2d_topk_workspace_bytes(long long n_max, int S, int k);
 B2D_API int b2d_topk(int* idx, int* out_count, const float* values, long long ld, const int* counts, long long n,
              int S, int k, void* workspace, size_t ws_bytes, void* stream);
@@ -311,9 +312,21 @@ B2D_API int b2d_fcos_targets(int64_t* cls_tar, float* reg_tar, float* ctr_tar, c
  * cls_out [B][ld][C] logits, reg_out [B][ld][4 * reg_classes] (reg_classes = C, or 1 for
  * class-agnostic regression), img_hw float[B][2] or NULL (no clamp).  Outputs
  * out_box [B][4][max_per_img], out_score / out_label [B][max_per_img], out_count int32[B].
- * cap = candidate slots per image (<= 16384); *overflow is set to 1 if an image had more
- * candidates (they are then truncated in enumeration order). */
+ * cap = candidate slots per image, 1 <= cap <= B2D_DET_MAX_CAP; *overflow is set to 1 if an
+ * image had more candidates (they are then truncated in enumeration order).  max_per_img <=
+ * min(cap, 16384).  cap <= 16384: one b2d_nms over the cap slots.  cap > 16384: b2d_nms over
+ * the 16384 best candidates of every image, then, for an image with more candidates and fewer
+ * than max_per_img survivors, an exact continuation of the greedy NMS over the rest (one kernel,
+ * no host synchronisation) -- the same result as one greedy NMS over all candidates.
+ * Workspace: 48 B per slot (B * cap) for the candidate arrays, plus one scratch used in turn by the
+ * round-0 top-k, b2d_nms and the continuation lists: the larger of about 34 MB per image (b2d_nms
+ * over 16384 boxes) and 16 B per slot (b2d_rcnn_detect_workspace_bytes: 0.31 GB for cap = 80000,
+ * B = 8; 0.28 GB for cap = 16384). */
+#define B2D_DET_MAX_CAP (1 << 20)
 B2D_API size_t b2d_rcnn_detect_workspace_bytes(int cap, int B);
+/* continuation rounds per image of the last b2d_rcnn_detect / b2d_dense_detect call (cap > 16384) that used this
+ * workspace -> rounds int32[B] (device, stream-ordered copy; 0 = finished by the first 16384 candidates) */
+B2D_API int b2d_detect_continuation_rounds(int* rounds, const void* workspace, int cap, int B, void* stream);
 B2D_API int b2d_rcnn_detect(float* out_box, float* out_score, int64_t* out_label, int* out_count, const float* props,
                     long long ld, const int* counts, long long n, const float* cls_out, const float* reg_out, int C,
                     int reg_classes, const float* means_host, const float* stds_host, const float* img_hw,
@@ -340,7 +353,7 @@ B2D_API int b2d_rcnn_detect_records(float* out_box, float* out_score, int64_t* o
  * only the first maximal channel of a row, if it is an NMS channel.  Candidates are ordered row-major, channel minor;
  * the NMS offset is channel * max(candidate boxes); label_add is added to the written labels only (1 for a sigmoid head's
  * 1-based labels).  Outputs and records as b2d_rcnn_detect(_records); workspace b2d_rcnn_detect_workspace_bytes(cap, B);
- * cap <= 16384 candidates per image, *overflow = 1 if an image had more.  events_host: NULL, or two cudaEvent_t (either
+ * cap <= B2D_DET_MAX_CAP candidates per image (as b2d_rcnn_detect), *overflow = 1 if an image had more.  events_host: NULL, or two cudaEvent_t (either
  * may be NULL) recorded after the candidate stage and after the NMS. */
 typedef struct b2d_dense_levels {
     int num_levels, _pad;

@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "libb200det.so")
 
 MAX_LEVELS = 8
 MAX_ANCHORS = 16
+DET_MAX_CAP = 1 << 20           # B2D_DET_MAX_CAP: candidate slots per image of b2d_rcnn_detect / b2d_dense_detect
 
 c_void_p, c_int, c_ll, c_float, c_size_t, c_ull = (ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong,
                                                    ctypes.c_float, ctypes.c_size_t, ctypes.c_ulonglong)
@@ -89,6 +90,7 @@ _SIGS = {
                          c_int, c_int, c_int, _P, _P, c_size_t, _P, _P],
     "b2d_dense_detect_records": [_P, _P, _P, _P, _P, _P, c_ll, _P, _P, _P, c_int, c_int, _P, c_ll, _P, c_float, c_int, c_float,
                                  c_int, c_int, c_int, c_int, _P, _P, c_size_t, _P, _P],
+    "b2d_detect_continuation_rounds": [_P, _P, c_int, c_int, _P],
     "b2d_dense_select": [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, _P, c_size_t, _P],
     "b2d_gather_head_outputs": [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, _P],
     "b2d_scatter_head_grads": [_P, _P, _P, _P, _P, c_int, _P, _P, c_int, c_int, _P],

@@ -23,6 +23,7 @@ struct RpnLaunch {
     long long mask_off[kMaxLevels], mask_per_img;
     int pre_nms, post_nms, max_num, score_mode, cls_ch, do_nms, out_ld;
     int raw;                            // 1: plain segmented top-k (no anchors / deltas / decode)
+    const int* seg_n;                   // b2d_topk with counts: valid elements per segment, at most n[l] (NULL: n[l])
     int dbg;                            // development knob (B2D_DBG)
     float nms_thr, min_size, ms[8];
     float* rec;                         // optional packed proposal records [B][out_ld][5] (b2d_rpn_cfg::records)
@@ -48,6 +49,11 @@ __device__ __forceinline__ void dbg_stamp(const RpnLaunch& p, int b, int cta, in
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
         p.dbg_t[((long long)b * kDbgCtas + cta) * kDbgStamps + k] = t;
     }
+}
+
+// elements of segment seg (level l) that take part in the selection
+__device__ __forceinline__ int seg_valid(const RpnLaunch& p, int seg, int l) {
+    return p.seg_n ? min(max(p.seg_n[seg], 0), p.n[l]) : p.n[l];
 }
 
 // launch-local segment index s (b-major over the launch's levels) -> global segment, image, level

@@ -28,6 +28,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "nms_common.cuh"
 
 namespace b2d {
 
@@ -323,11 +324,246 @@ __global__ void __launch_bounds__(256) k_rcnn_gather(float* __restrict__ out_box
     }
 }
 
+// ---- candidate sets past 16384 (cap > kDetT) ------------------------------------------------------------------------
+// Round 0 runs b2d_nms on the kDetT best candidates of every image (b2d_topk); an image with at most kDetT candidates is
+// then finished.  k_det_continue completes greedy NMS for the others: a candidate is kept iff no KEPT higher-ranked
+// candidate suppresses it, so the kept set of a processed prefix is final, and every later candidate a kept one suppresses
+// can be dropped (non-kept candidates suppress nothing).  One CTA per image loops: filter the unprocessed candidates against
+// the newly kept ones, take the next block of at most kContBlock survivors in rank order, run greedy NMS on it, append its
+// survivors -- until max_keep are kept or nothing is left.
+constexpr int kDetT = 16384;                  // round-0 candidates per image (the b2d_nms limit)
+constexpr int kContThreads = 1024;
+constexpr int kContBlock = 1024;              // candidates per continuation round (also the kept-box chunk of the filter)
+
+// round 0: the selected candidates in rank order (b2d_topk output) -> boxes and scores for b2d_nms (presorted)
+__global__ void __launch_bounds__(256) k_det_round0(float4* __restrict__ r0_box, float* __restrict__ r0_score,
+                                                    const int* __restrict__ r0_idx, const int* __restrict__ r0_n,
+                                                    const float4* __restrict__ nms_box, const float* __restrict__ cand_score,
+                                                    int cap) {
+    const int b = blockIdx.y, r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= r0_n[b]) return;
+    const long long i = (long long)b * cap + r0_idx[(long long)b * kDetT + r];
+    r0_box[(long long)b * kDetT + r] = nms_box[i];
+    r0_score[(long long)b * kDetT + r] = cand_score[i];
+}
+
+struct ContArgs {
+    const float4* nms_box; const float* cand_score; const int* cand_count;   // [B][cap], [B][cap], [B]
+    const int* r0_idx; const int64_t* keep0; const int* keep0_count;          // round 0: [B][kDetT] rank -> candidate, survivors
+    int64_t* keep; int* keep_count;                                           // [B][cap] candidate indices, [B]
+    uint64_t* list;                                                           // [B][2][cap] unprocessed candidates (ping-pong)
+    int* rounds;                                                              // [B] continuation rounds taken
+    int cap, max_keep;
+    float thr, thr_lo, thr_hi;
+};
+
+__device__ __forceinline__ uint64_t cand_comp(const ContArgs& a, long long base, int i) {
+    return make_comp(f2key(a.cand_score[base + i]), (uint32_t)i);
+}
+
+// block-wide minimum (all threads return it)
+__device__ __forceinline__ int block_min(int v, int* s_red) {
+    v = __reduce_min_sync(0xffffffffu, v);
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int m = s_red[0];
+    for (int w = 1; w < kContThreads / 32; ++w) m = min(m, s_red[w]);
+    return m;
+}
+
+__global__ void __launch_bounds__(kContThreads) k_det_continue(ContArgs a) {
+    __shared__ float4 s_box[kContBlock];
+    __shared__ float s_area[kContBlock];
+    __shared__ uint64_t s_blk[kContBlock];
+    __shared__ uint8_t s_dead[kContBlock];
+    __shared__ uint32_t s_hist[256];
+    __shared__ int s_red[kContThreads / 32];
+    __shared__ int s_n, s_m, s_done;
+    __shared__ uint64_t s_prefix;
+    __shared__ uint32_t s_need;
+    const int b = blockIdx.x, tid = threadIdx.x;
+    const int count = a.cand_count[b], k0 = a.keep0_count[b];
+    const long long base = (long long)b * a.cap;
+    int64_t* keep = a.keep + base;
+    for (int t = tid; t < k0; t += kContThreads)
+        keep[t] = a.r0_idx[(long long)b * kDetT + (int)a.keep0[(long long)b * kDetT + t]];
+    if (count <= kDetT || k0 >= a.max_keep) {                        // finished by round 0 (every image, normally)
+        if (tid == 0) { a.keep_count[b] = k0; a.rounds[b] = 0; }
+        return;
+    }
+    __syncthreads();                                                 // keep[0, k0) is read back below
+    uint64_t* cur = a.list + 2 * base;
+    uint64_t* nxt = cur + a.cap;
+    // the unprocessed candidates: all below the last one of round 0 (any order: blocks are picked by composite key)
+    const uint64_t c_last = cand_comp(a, base, a.r0_idx[(long long)b * kDetT + kDetT - 1]);
+    if (tid == 0) s_n = 0;
+    __syncthreads();
+    for (int i0 = 0; i0 < count; i0 += kContThreads) {
+        const int i = i0 + tid;
+        const uint64_t c = i < count ? cand_comp(a, base, i) : 0ull;
+        const bool in = i < count && c < c_last;
+        const int pos = warp_alloc(in, &s_n);
+        if (in) cur[pos] = c;
+    }
+    __syncthreads();
+    int n = s_n, kc = k0, filt = 0, rounds = 0;                      // keep[filt, kc): kept, not yet applied to the list
+    uint64_t tau = ~0ull;                                            // candidates >= tau are processed
+    while (true) {
+        // ---- drop the processed candidates and those a kept candidate in keep[filt, kc) suppresses (chunks of kContBlock)
+        do {
+            __syncthreads();                                         // every thread has read s_m (n) of the previous pass
+            const int nk = min(kc - filt, kContBlock);
+            for (int t = tid; t < nk; t += kContThreads) {
+                const float4 kb = a.nms_box[base + keep[filt + t]];
+                s_box[t] = kb; s_area[t] = area_of(kb);
+            }
+            if (tid == 0) s_m = 0;
+            __syncthreads();
+            for (int i0 = 0; i0 < n; i0 += kContThreads) {
+                const int i = i0 + tid;
+                bool live = false;
+                uint64_t c = 0ull;
+                if (i < n) {
+                    c = cur[i];
+                    live = c < tau;
+                    if (live && nk > 0) {
+                        const float4 bx = a.nms_box[base + comp_idx(c)];
+                        const float ar = area_of(bx);
+                        for (int j = 0; j < nk && live; ++j) live = !suppresses(s_box[j], s_area[j], bx, ar, a.thr, a.thr_lo, a.thr_hi);
+                    }
+                }
+                const int pos = warp_alloc(live, &s_m);
+                if (live) nxt[pos] = c;
+            }
+            __syncthreads();
+            n = s_m;
+            uint64_t* t = cur; cur = nxt; nxt = t;
+            filt += nk;
+        } while (filt < kc);
+        if (n == 0 || kc >= a.max_keep) break;
+        ++rounds;
+        // ---- tau = composite of the min(n, kContBlock)-th best remaining candidate (radix select, 8 bits per pass; stops
+        // as soon as the remaining count of the current bin is the number still needed)
+        const int m = min(n, kContBlock);
+        if (tid == 0) { s_prefix = 0ull; s_need = (uint32_t)m; }
+        int fixed = 0;                                               // leading bits of tau decided
+        while (fixed < 64) {
+            const int shift = 56 - fixed;
+            for (int t = tid; t < 256; t += kContThreads) s_hist[t] = 0u;
+            __syncthreads();
+            const uint64_t prefix = s_prefix;
+            const uint64_t himask = fixed == 0 ? 0ull : (~0ull << (64 - fixed));
+            for (int i0 = 0; i0 < n; i0 += kContThreads) {
+                const int i = i0 + tid;
+                const uint64_t c = i < n ? cur[i] : 0ull;
+                // warp-aggregated: the candidates of a round share their leading bits, so most fall in one bin
+                const bool in = i < n && (c & himask) == prefix;
+                const uint32_t bin = in ? ((uint32_t)(c >> shift) & 255u) : 256u;
+                const unsigned peers = __match_any_sync(0xffffffffu, bin);
+                if (in && (tid & 31) == __ffs(peers) - 1) atomicAdd(&s_hist[bin], (uint32_t)__popc(peers));
+            }
+            __syncthreads();
+            if (tid == 0) {
+                uint32_t run = 0, need = s_need;
+                int d = 255;
+                for (; d > 0 && run + s_hist[d] < need; --d) run += s_hist[d];
+                s_prefix = prefix | ((uint64_t)d << shift);
+                s_need = need - run;
+                s_done = (run + s_hist[d] == need) ? 1 : 0;          // the whole bin is taken: tau found
+            }
+            __syncthreads();
+            fixed += 8;
+            if (s_done) break;
+        }
+        tau = s_prefix;                                              // exactly m candidates have composite >= tau
+        // ---- the block, in rank order
+        if (tid == 0) s_m = 0;
+        __syncthreads();
+        for (int i0 = 0; i0 < n; i0 += kContThreads) {
+            const int i = i0 + tid;
+            const bool in = i < n && cur[i] >= tau;
+            const int pos = warp_alloc(in, &s_m);
+            if (in) s_blk[pos] = cur[i];
+        }
+        __syncthreads();
+        for (int t = m + tid; t < kContBlock; t += kContThreads) s_blk[t] = 0ull;
+        bitonic_sort_desc(s_blk, kContBlock);
+        for (int t = tid; t < m; t += kContThreads) {
+            const float4 bx = a.nms_box[base + comp_idx(s_blk[t])];
+            s_box[t] = bx; s_area[t] = area_of(bx); s_dead[t] = 0;
+        }
+        __syncthreads();
+        // ---- greedy NMS on the block; its first candidate survives (no kept candidate suppresses a listed one)
+        const int kc0 = kc;
+        int r = 0;
+        while (r < m && kc < a.max_keep) {
+            if (tid == 0) keep[kc] = comp_idx(s_blk[r]);
+            ++kc;
+            int next = 0x7fffffff;
+            for (int t = r + 1 + tid; t < m; t += kContThreads) {
+                if (s_dead[t]) continue;
+                if (suppresses(s_box[r], s_area[r], s_box[t], s_area[t], a.thr, a.thr_lo, a.thr_hi)) s_dead[t] = 1;
+                else next = min(next, t);
+            }
+            r = block_min(next, s_red);
+        }
+        filt = kc0;                                                  // the block's survivors filter the rest
+        if (kc >= a.max_keep) break;
+        __syncthreads();
+    }
+    if (tid == 0) { a.keep_count[b] = kc; a.rounds[b] = rounds; }
+}
+
 }  // namespace b2d
 
 using namespace b2d;
 
 static size_t det_al(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// The workspace of b2d_rcnn_detect / b2d_dense_detect: one carve-up for the launcher, the size query and
+// b2d_detect_continuation_rounds (base NULL: sizes only).
+struct DetWs {
+    float4* cand_box; float4* nms_box; float* cand_score; int* cand_label; int64_t* keep;   // [B][cap]: 48 B per slot
+    int* cand_count; uint32_t* maxkey; int* chunk_cnt;
+    // cap > kDetT only: round 0 ([B][kDetT]) and the continuation's round counts
+    int* r0_idx; int* r0_n; float4* r0_box; float* r0_score; int64_t* keep0; int* keep0_count; int* rounds;
+    char* scratch;                // cap <= kDetT: b2d_nms; cap > kDetT: top-k, then b2d_nms, then the continuation lists
+    size_t scratch_bytes, total;
+};
+
+static DetWs det_layout(char* base, int cap, int B) {
+    DetWs d;
+    memset(&d, 0, sizeof(d));
+    size_t o = 0;
+    auto carve = [&](size_t sz) { char* r = base ? base + o : nullptr; o += det_al(sz); return r; };
+    const size_t nb = (size_t)B * cap;
+    d.cand_box = (float4*)carve(nb * 16);
+    d.nms_box = (float4*)carve(nb * 16);
+    d.cand_score = (float*)carve(nb * 4);
+    d.cand_label = (int*)carve(nb * 4);
+    d.keep = (int64_t*)carve(nb * 8);
+    d.cand_count = (int*)carve((size_t)B * 4);
+    d.maxkey = (uint32_t*)carve((size_t)B * 4);
+    d.chunk_cnt = (int*)carve((size_t)B * kDetMaxChunks * 4);
+    if (cap <= kDetT) {
+        d.scratch_bytes = b2d_nms_workspace_bytes(cap, B);
+    } else {
+        const size_t nt = (size_t)B * kDetT;
+        d.r0_idx = (int*)carve(nt * 4);
+        d.r0_n = (int*)carve((size_t)B * 4);
+        d.r0_box = (float4*)carve(nt * 16);
+        d.r0_score = (float*)carve(nt * 4);
+        d.keep0 = (int64_t*)carve(nt * 8);
+        d.keep0_count = (int*)carve((size_t)B * 4);
+        d.rounds = (int*)carve((size_t)B * 4);
+        d.scratch_bytes = std::max(std::max(b2d_topk_workspace_bytes(cap, B, kDetT), b2d_nms_workspace_bytes(kDetT, B)),
+                                   nb * 16);                          // lists: 2 x 8 B per slot
+    }
+    d.scratch = carve(d.scratch_bytes);
+    d.total = o;
+    return d;
+}
 
 // The four stages on a filled DetArgs (everything but the workspace carve-up and the chunking): candidate count,
 // candidate write, class-offset boxes, b2d_nms, gather.  events_host (optional, dense form): cudaEvent_t recorded after
@@ -337,16 +573,15 @@ static int detect_run(DetArgs& p, float* out_box, float* out_score, int64_t* out
                       float nms_thr_f, int max_per_img, int label_add, int B, int* overflow, void* workspace, size_t ws_bytes,
                       void* const* events_host, cudaStream_t st, const char* what) {
     const int cap = p.cap;
-    char* w = (char*)workspace;
-    const size_t nb = (size_t)B * cap;
-    float4* cand_box = (float4*)w; w += det_al(nb * 16);
-    float4* nms_box = (float4*)w; w += det_al(nb * 16);
-    float* cand_score = (float*)w; w += det_al(nb * 4);
-    int* cand_label = (int*)w; w += det_al(nb * 4);
-    int64_t* keep = (int64_t*)w; w += det_al(nb * 8);
-    int* cand_count = (int*)w; w += det_al((size_t)B * 4);
-    uint32_t* maxkey = (uint32_t*)w; w += det_al((size_t)B * 4);
-    int* chunk_cnt = (int*)w; w += det_al((size_t)B * kDetMaxChunks * 4);
+    const DetWs d = det_layout((char*)workspace, cap, B);
+    float4* cand_box = d.cand_box;
+    float4* nms_box = d.nms_box;
+    float* cand_score = d.cand_score;
+    int* cand_label = d.cand_label;
+    int64_t* keep = d.keep;
+    int* cand_count = d.cand_count;
+    uint32_t* maxkey = d.maxkey;
+    int* chunk_cnt = d.chunk_cnt;
     // chunks of at least 32 rows, at most kDetMaxChunks CTAs per image (8 x 32 CTAs at 1000 proposals, B = 8)
     const long long nmax = p.counts ? p.ld : p.n;
     p.nchunk = (int)std::max(1ll, std::min((long long)kDetMaxChunks, (nmax + 31) / 32));
@@ -356,13 +591,33 @@ static int detect_run(DetArgs& p, float* out_box, float* out_score, int64_t* out
     dim3 gc(p.nchunk, B);
     k_rcnn_candidates<false, kDense><<<gc, kDetThreads, 0, st>>>(p, cand_box, cand_score, cand_label, cand_count, overflow);
     k_rcnn_candidates<true, kDense><<<gc, kDetThreads, 0, st>>>(p, cand_box, cand_score, cand_label, cand_count, overflow);
-    k_rcnn_offset_boxes<<<dim3(std::max(1, std::min(16, cdiv(cap, 256))), B), 256, 0, st>>>(nms_box, cand_box, cand_label,
-                                                                                             cand_count, maxkey, cap);
+    const int ob = cap <= kDetT ? std::max(1, std::min(16, cdiv(cap, 256))) : std::min(128, cdiv(cap, 256));
+    k_rcnn_offset_boxes<<<dim3(ob, B), 256, 0, st>>>(nms_box, cand_box, cand_label, cand_count, maxkey, cap);
     if (int rc = check_launch(what)) return rc;
     if (events_host && events_host[0]) cudaEventRecord((cudaEvent_t)events_host[0], st);
-    const int rc = b2d_nms(keep, out_count, (const float*)nms_box, cand_score, cap, cand_count, cap, B, nms_thr_f, max_per_img,
-                           0, w, ws_bytes - (size_t)(w - (char*)workspace), st);
-    if (rc != B2D_OK) return rc;
+    if (cap <= kDetT) {
+        const int rc = b2d_nms(keep, out_count, (const float*)nms_box, cand_score, cap, cand_count, cap, B, nms_thr_f,
+                               max_per_img, 0, d.scratch, ws_bytes - (size_t)(d.scratch - (char*)workspace), st);
+        if (rc != B2D_OK) return rc;
+    } else {
+        // round 0 on the kDetT best candidates of every image, then the continuation (see k_det_continue)
+        const size_t scratch = ws_bytes - (size_t)(d.scratch - (char*)workspace);
+        int rc = b2d_topk(d.r0_idx, d.r0_n, cand_score, cap, cand_count, cap, B, kDetT, d.scratch, scratch, st);
+        if (rc != B2D_OK) return rc;
+        k_det_round0<<<dim3(kDetT / 256, B), 256, 0, st>>>(d.r0_box, d.r0_score, d.r0_idx, d.r0_n, nms_box, cand_score, cap);
+        if ((rc = check_launch(what))) return rc;
+        rc = b2d_nms(d.keep0, d.keep0_count, (const float*)d.r0_box, d.r0_score, kDetT, d.r0_n, kDetT, B, nms_thr_f,
+                     max_per_img, 1, d.scratch, scratch, st);
+        if (rc != B2D_OK) return rc;
+        ContArgs a;
+        a.nms_box = nms_box; a.cand_score = cand_score; a.cand_count = cand_count;
+        a.r0_idx = d.r0_idx; a.keep0 = d.keep0; a.keep0_count = d.keep0_count;
+        a.keep = keep; a.keep_count = out_count; a.list = (uint64_t*)d.scratch; a.rounds = d.rounds;
+        a.cap = cap; a.max_keep = max_per_img;
+        nms_thr_bounds(nms_thr_f, a.thr, a.thr_lo, a.thr_hi);
+        k_det_continue<<<B, kContThreads, 0, st>>>(a);
+        if ((rc = check_launch(what))) return rc;
+    }
     if (events_host && events_host[1]) cudaEventRecord((cudaEvent_t)events_host[1], st);
     dim3 g(cdiv(max_per_img, 256), B);
     k_rcnn_gather<<<g, 256, 0, st>>>(out_box, out_score, out_label, records, keep, out_count, cand_box, cand_score,
@@ -373,10 +628,16 @@ static int detect_run(DetArgs& p, float* out_box, float* out_score, int64_t* out
 extern "C" {
 
 size_t b2d_rcnn_detect_workspace_bytes(int cap, int B) {
-    if (cap < 1 || B < 1) return 0;
-    const size_t n = (size_t)B * cap;
-    return det_al(n * 16) * 2 + det_al(n * 4) * 2 + det_al(n * 8) + det_al((size_t)B * 4) * 2 +
-           det_al((size_t)B * kDetMaxChunks * 4) + b2d_nms_workspace_bytes(cap, B);
+    if (cap < 1 || B < 1 || cap > B2D_DET_MAX_CAP) return 0;
+    return det_layout(nullptr, cap, B).total;
+}
+
+int b2d_detect_continuation_rounds(int* rounds, const void* workspace, int cap, int B, void* stream) {
+    B2D_REQUIRE(rounds && workspace && B >= 1 && cap > kDetT && cap <= B2D_DET_MAX_CAP,
+                "detect_continuation_rounds: need a workspace of a call with cap > 16384");
+    const DetWs d = det_layout((char*)workspace, cap, B);
+    cudaMemcpyAsync(rounds, d.rounds, sizeof(int) * B, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    return check_launch("detect_continuation_rounds");
 }
 
 static int rcnn_detect_impl(float* out_box, float* out_score, int64_t* out_label, int* out_count, float* records,
@@ -388,7 +649,8 @@ static int rcnn_detect_impl(float* out_box, float* out_score, int64_t* out_label
                 "rcnn_detect: null pointer");
     B2D_REQUIRE(B >= 1 && n >= 0 && ld >= n && C >= 2 && C <= kDetMaxC && (reg_classes == C || reg_classes == 1),
                 "rcnn_detect: need 2 <= C <= 128 and reg_classes in {1, C}");
-    B2D_REQUIRE(cap >= 1 && cap <= 16384 && max_per_img >= 1 && max_per_img <= cap, "rcnn_detect: need max_per_img <= cap <= 16384");
+    B2D_REQUIRE(cap >= 1 && cap <= B2D_DET_MAX_CAP && max_per_img >= 1 && max_per_img <= std::min(cap, kDetT),
+                "rcnn_detect: need 1 <= cap <= 1048576 and max_per_img <= min(cap, 16384)");
     B2D_REQUIRE(workspace && ws_bytes >= b2d_rcnn_detect_workspace_bytes(cap, B), "rcnn_detect: workspace too small");
     DetArgs p;
     memset(&p, 0, sizeof(p));
@@ -411,7 +673,8 @@ static int dense_detect_impl(float* out_box, float* out_score, int64_t* out_labe
                 "dense_detect: null pointer");
     B2D_REQUIRE(B >= 1 && ld >= 1 && C >= 1 && C <= kDetMaxC && transform >= 0 && transform <= 2,
                 "dense_detect: need 1 <= C <= 128 and transform in {0, 1, 2}");
-    B2D_REQUIRE(cap >= 1 && cap <= 16384 && max_per_img >= 1 && max_per_img <= cap, "dense_detect: need max_per_img <= cap <= 16384");
+    B2D_REQUIRE(cap >= 1 && cap <= B2D_DET_MAX_CAP && max_per_img >= 1 && max_per_img <= std::min(cap, kDetT),
+                "dense_detect: need 1 <= cap <= 1048576 and max_per_img <= min(cap, 16384)");
     B2D_REQUIRE(workspace && ws_bytes >= b2d_rcnn_detect_workspace_bytes(cap, B), "dense_detect: workspace too small");
     const int L = lv_host->num_levels;
     B2D_REQUIRE(L >= 1 && L <= kMaxLevels && lv_host->offset[0] == 0, "dense_detect: need 1..8 levels, the first at offset 0");

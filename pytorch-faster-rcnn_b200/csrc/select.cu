@@ -31,14 +31,14 @@ __global__ void __launch_bounds__(kHcThreads) k_hist(RpnLaunch p) {
     __shared__ uint32_t s_h[kHistBins];
     int seg, b, l;
     seg_of(p.lv0, p.lvn, p.L, blockIdx.y, seg, b, l);
-    const int n = p.n[l], k = p.kcap[l];
-    if (k >= n) return;                                  // no selection on this level
+    const int n = p.n[l], k = p.kcap[l], nv = seg_valid(p, seg, l);
+    if (k >= nv) return;                                 // no selection on this level
     const int start = blockIdx.x * kChunk;
-    if (start >= n) return;
+    if (start >= nv) return;
     for (int t = threadIdx.x; t < kHistBins; t += blockDim.x) s_h[t] = 0;
     __syncthreads();
     const float* cls = seg_cls(p, b, l);
-    const int end = min(start + kChunk, n);
+    const int end = min(start + kChunk, nv);
     {
         constexpr int kPer = kChunk / kHcThreads;         // 16 independent loads in flight per thread
         float v[kPer];
@@ -103,13 +103,13 @@ __global__ void __launch_bounds__(kHcThreads) k_compact(RpnLaunch p) {
     __shared__ int s_n, s_n2, s_base, s_base2;
     int seg, b, l;
     seg_of(p.lv0, p.lvn, p.L, blockIdx.y, seg, b, l);
-    const int n = p.n[l], k = p.kcap[l];
-    if (k >= n) return;
+    const int n = p.n[l], k = p.kcap[l], nv = seg_valid(p, seg, l);
+    if (k >= nv) return;
     const int start = blockIdx.x * kChunk;
-    if (start >= n) return;
+    if (start >= nv) return;
     if (threadIdx.x == 0) { s_n = 0; s_n2 = 0; }
     const float* cls = seg_cls(p, b, l);
-    const int end = min(start + kChunk, n);
+    const int end = min(start + kChunk, nv);
     // the whole chunk (16 values per thread) is requested before the threshold search, whose latency it hides
     constexpr int kPer = kChunk / kHcThreads;
     float v[kPer];
@@ -157,18 +157,18 @@ __global__ void __launch_bounds__(kSelThreads) k_select(RpnLaunch p) {
     int seg, b, l;
     seg_of(p.lv0, p.lvn, p.L, blockIdx.x, seg, b, l);
     const b2d_level& lv = p.pyr.lv[l];
-    const int n = p.n[l], k = p.kcap[l];
+    const int n = p.n[l], k = p.kcap[l], nv = seg_valid(p, seg, l);
     const float* cls = seg_cls(p, b, l);
     const bool identity = (k >= n) && !p.do_nms;          // AnchorHead path without top-k: keep index order
     int total = 0;
     bool presorted = false;                               // s_buf holds two sorted runs: [0, split_at) and [split_off, ...)
     int split_at = 1 << 30, split_off = 0;
-    if (k >= n) {
-        for (int i = threadIdx.x; i < n; i += blockDim.x)
+    if (k >= nv) {
+        for (int i = threadIdx.x; i < nv; i += blockDim.x)
             s_buf[i] = identity ? make_comp(0xffffffffu, (uint32_t)i)
                                 : make_comp(f2key(load_logit(cls, n, i, p.score_mode, p.cls_ch)), (uint32_t)i);
-        total = n;
-        if (!identity && n <= kBucketCap) {
+        total = nv;
+        if (!identity && nv <= kBucketCap) {
             __syncthreads();
             presorted = bucket_sort_desc(s_buf, s_buf + kBucketCap, total, s_off, s_cur, s_wsum, p.dbg);
         }
@@ -913,7 +913,7 @@ int b2d_topk(int* idx, int* out_count, const float* values, long long ld, const 
         return check_launch("topk");
     }
     // pyramid-sized inputs: radix histogram + compaction + exact narrowing (the K3 machinery)
-    B2D_REQUIRE(!counts && ld == n, "topk: n > 16384 needs dense equal-length segments");
+    B2D_REQUIRE(ld == n, "topk: n > 16384 needs ld == n");
     B2D_REQUIRE(k <= kSortCap, "topk: k must be <= 16384");
     b2d_pyramid pyr; b2d_rpn_cfg cfg;
     topk_cfg(n, k, pyr, cfg);
@@ -921,7 +921,7 @@ int b2d_topk(int* idx, int* out_count, const float* values, long long ld, const 
     size_t need = 0;
     B2D_REQUIRE(rpn_plan(p, &pyr, S, &cfg, (char*)workspace, &need), "topk: unsupported size");
     B2D_REQUIRE(workspace && ws_bytes >= need, "topk: workspace too small");
-    p.cls[0] = values; p.reg[0] = nullptr; p.img_hw = nullptr; p.raw = 1;
+    p.cls[0] = values; p.reg[0] = nullptr; p.img_hw = nullptr; p.raw = 1; p.seg_n = counts;
     B2D_SMEM(k_select, kSortCap * 8, "k_select");   // per device
     cudaMemsetAsync(workspace, 0, p.zero_bytes, st);
     dim3 grid(cdiv(n, kChunk), S);

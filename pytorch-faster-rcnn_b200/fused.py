@@ -946,6 +946,15 @@ class _CascadeOutFn(torch.autograd.Function):
         return (None, None, g_token) + (None,) * len(grads)
 
 
+def _detect_cap(max_candidates, bound, who):
+    """Candidate slots per image of b2d_rcnn_detect / b2d_dense_detect: max_candidates, at most the exact bound (no
+    image can have more candidates); checked here so that a bad value fails before any kernel runs."""
+    if (isinstance(max_candidates, bool) or not isinstance(max_candidates, (int, np.integer))
+            or not 1 <= max_candidates <= _C.DET_MAX_CAP):
+        raise _C.B200DetError("%s: max_candidates must be an integer in 1..%d, got %r" % (who, _C.DET_MAX_CAP, max_candidates))
+    return max(1, min(int(max_candidates), bound))
+
+
 class InferHotPath(object):
     """CascadeRCNN.forward_test (SURVEY 3.2, lib/detectors/cascade_rcnn.py:157-200) minus the backbone, neck and head
     layers, batched: RPN proposals at the test configuration (K3 + K4) -> per stage FPN RoIAlign of the current boxes (K5)
@@ -953,12 +962,17 @@ class InferHotPath(object):
     (b2d_refine_bboxes_argmax) -> after the last stage BBoxHead.predict_bboxes_single_image on that stage's input boxes
     (b2d_rcnn_detect: softmax, per-class decode + clamp, class-offset NMS, top max_per_img).  num_stages = 1 is
     faster_rcnn_r50_fpn, 3 the cascade.  Everything is allocated here; step() reads nothing back to the host, so a step
-    (head modules included) can be captured in one CUDA graph after a first eager call."""
+    (head modules included) can be captured in one CUDA graph after a first eager call.
+    max_candidates: (box, class) candidate slots per image of the detection stage (at most the exact bound P * (C - 1),
+    P in strict mode).  An image with more candidates sets a device flag that check() raises.  Above 16384 the NMS runs on
+    the 16384 best candidates and continues exactly over the rest when that leaves fewer than max_per_img detections;
+    at the bound no image can overflow.  Workspace: 48 B per slot and image, plus a scratch of the larger of ~34 MB per
+    image and 16 B per slot."""
 
     def __init__(self, B, grids, device, strides=(4, 8, 16, 32, 64), feat_channels=256, num_classes=21, num_stages=1,
                  rpn_test=None, rcnn_test=None,
                  stage_stds=((0.1, 0.1, 0.2, 0.2), (0.05, 0.05, 0.1, 0.1), (0.033, 0.033, 0.067, 0.067)),
-                 reg_class_agnostic=False, layout=1):
+                 reg_class_agnostic=False, layout=1, max_candidates=16384):
         rpn_test = rpn_test or dict(pre_nms=1000, post_nms=1000, max_num=1000, nms_iou=0.7, min_bbox_size=0)
         rcnn_test = rcnn_test or dict(min_score=0.05, nms_iou=0.5, max_per_img=100, nms_type='official')
         if not 1 <= num_stages <= len(stage_stds):
@@ -967,6 +981,7 @@ class InferHotPath(object):
             # b2d_rcnn_detect holds a row's classes in one warp; without this check the first step would only fail at
             # the detection call, after the proposals, RoIAlign and the caller's head (or in the middle of a graph capture)
             raise _C.B200DetError("InferHotPath: 2..128 classes (background included) supported, got %d" % int(num_classes))
+        _detect_cap(max_candidates, _C.DET_MAX_CAP, "InferHotPath")
         z4 = (0.0, 0.0, 0.0, 0.0)
         self.B, self.device, self.S = B, device, int(num_stages)
         self.NC, self.reg_c = int(num_classes), 1 if reg_class_agnostic else int(num_classes)
@@ -983,9 +998,9 @@ class InferHotPath(object):
         mode = get('nms_type', 'official')
         self.min_score, self.nms_thr = float(np.float32(get('min_score'))), _C.floor_f32(float(get('nms_iou')))
         self.strict = int(mode == 'strict')
-        self.cap = max(1, min(16384, P * ((self.NC - 1) if not self.strict else 1)))
+        self.cap = _detect_cap(max_candidates, P * ((self.NC - 1) if not self.strict else 1), "InferHotPath")
         mpi = get('max_per_img')
-        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap))
+        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap, 16384))
         self.det_box = torch.zeros((B, 4, M), dtype=torch.float32, device=device)
         self.det_score = torch.zeros((B, M), dtype=torch.float32, device=device)
         self.det_label = torch.zeros((B, M), dtype=torch.int64, device=device)
@@ -1041,11 +1056,12 @@ class InferHotPath(object):
                     records=records, stages=stages)
 
     def check(self):
-        """Synchronise and raise if the last step had an image with more than 16384 (box, class) candidates (its
+        """Synchronise and raise if the last step had an image with more than cap (box, class) candidates (its
         candidates past the cap were dropped in enumeration order)."""
         torch.cuda.synchronize(self.device)
         if int(self.overflow[0]):
-            raise _C.B200DetError("rcnn_detect: more than 16384 (box, class) candidates; raise min_score")
+            raise _C.B200DetError("rcnn_detect: more than %d (box, class) candidates; raise min_score or max_candidates"
+                                  % self.cap)
 
 
 class DenseInferHotPath(object):
@@ -1061,14 +1077,17 @@ class DenseInferHotPath(object):
     num_classes counts the background as the reference heads do: a sigmoid head (RetinaNet with use_sigmoid, FCOS) has
     num_classes - 1 class channels and 1-based labels, a softmax head num_classes channels with channel 0 the background.
     Everything is allocated here; step() reads nothing back to the host, so a step can be captured in one CUDA graph after
-    a first eager call.  More than 16384 (box, class) candidates in an image set a device flag that check() raises."""
+    a first eager call.  More than max_candidates (box, class) candidates in an image set a device flag that check()
+    raises; max_candidates (default 16384, at most the exact bound P * |class channels|, P in strict mode) works as in
+    InferHotPath."""
 
     def __init__(self, B, grids, device, head="retina", num_classes=21, test_cfg=None, strides=(8, 16, 32, 64, 128),
                  use_sigmoid=True, anchor_scales=tuple(4 * 2 ** (i / 3) for i in range(3)), anchor_ratios=(0.5, 1.0, 2.0),
                  center_lt=False, target_means=(0.0, 0.0, 0.0, 0.0), target_stds=(1.0, 1.0, 1.0, 1.0), reg_mean=0.0,
-                 reg_std=300.0, use_centerness=True, scale_factor=1.0):
+                 reg_std=300.0, use_centerness=True, scale_factor=1.0, max_candidates=16384):
         if head not in ("retina", "fcos"):
             raise _C.B200DetError("DenseInferHotPath: head must be 'retina' or 'fcos', got %r" % (head,))
+        _detect_cap(max_candidates, _C.DET_MAX_CAP, "DenseInferHotPath")
         test_cfg = test_cfg or dict(pre_nms=1000, min_bbox_size=0, min_score=0.05, nms_iou=0.5, max_per_img=100,
                                     nms_type="strict")
         get = (lambda k, d=None: test_cfg.get(k, d)) if hasattr(test_cfg, "get") else (lambda k, d=None: getattr(test_cfg, k, d))
@@ -1129,9 +1148,9 @@ class DenseInferHotPath(object):
             self.lv.num_levels = 1                                    # score [B][C][total] as one level
             self.lv.offset[0], self.lv.img_stride[0], self.lv.class_stride[0] = 0, C * T, T
             self.lv.base[0] = self.score.data_ptr()
-        self.cap = max(1, min(16384, self.P * (len(chans) if not self.strict else 1)))
+        self.cap = _detect_cap(max_candidates, self.P * (len(chans) if not self.strict else 1), "DenseInferHotPath")
         mpi = get("max_per_img")
-        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap))
+        self.M = M = max(1, min(int(mpi) if mpi is not None else self.cap, self.cap, 16384))
         self.det_box = torch.zeros((B, 4, M), dtype=torch.float32, device=device)
         self.det_score = torch.zeros((B, M), dtype=torch.float32, device=device)
         self.det_label = torch.zeros((B, M), dtype=torch.int64, device=device)
@@ -1202,8 +1221,9 @@ class DenseInferHotPath(object):
                     records=records, sel_boxes=boxes, sel_count=count, sel_rows=rows)
 
     def check(self):
-        """Synchronise and raise if the last step had an image with more than 16384 (box, class) candidates (its
+        """Synchronise and raise if the last step had an image with more than cap (box, class) candidates (its
         candidates past the cap were dropped in enumeration order)."""
         torch.cuda.synchronize(self.device)
         if int(self.overflow[0]):
-            raise _C.B200DetError("dense_detect: more than 16384 (box, class) candidates in an image; raise min_score")
+            raise _C.B200DetError("dense_detect: more than %d (box, class) candidates in an image; raise min_score or "
+                                  "max_candidates" % self.cap)
